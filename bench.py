@@ -6,7 +6,7 @@ dense stride-1 patches.  One step = one pass of the whole path over the batch.  
 collective on the data path (weak scaling: every rank owns its own batch); the barrier and the max-over-ranks
 reduction are the only torch.distributed calls.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--faces F]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--faces F] [--dump-outputs DIR]
 
 `value`  : whole-job faces/s with the crops already resident in HBM (crf_analyze_crops_device), CUDA events on
            the library's stream, max over ranks.
@@ -176,8 +176,8 @@ def ref_forest():
     try:
         from oracle import ref as R
         hp, ffd = ROOT / "staged" / "trees_headpose", ROOT / "staged" / "trees_ffd"
-        if not hp.exists():
-            hp, ffd = Path("/root/reference/data/trees_headpose"), Path("/root/reference/data/trees_ffd")
+        if not hp.exists() and R.REF_DATA is not None:
+            hp, ffd = R.REF_DATA / "trees_headpose", R.REF_DATA / "trees_ffd"
         if R.available() and hp.exists() and ffd.exists():
             _REF_FF = R.FaceForest(str(hp), str(ffd))
     except Exception as e:  # noqa: BLE001
@@ -287,6 +287,25 @@ def run_reference(args, rank: int, world: int):
 # orientations x (re, im) with separately rounded multiply and add.
 GABOR_BAND = 32
 GABOR_EXECUTED_FLOP_PER_PIXEL = sum(2 * (15 * K * (GABOR_BAND - 1 + K) / GABOR_BAND + 29 * K) for K in (9, 13, 19, 25)) + 2 * 49 * 7 * 2
+
+
+DUMP_BYTES = 60_000_000   # keeps a dump, .npy headers included, under 64 MB
+
+
+def dump_outputs(out_dir: str, rec: np.ndarray) -> None:
+    """--dump-outputs: the records the last timed step returned, one float64 array per crf_face_t field (DIR/<field>.npy,
+    first axis = face, in batch order), so that two builds can be compared output for output on the same seeded inputs.
+    Above DUMP_BYTES in all, a fixed seeded sample of the faces is written instead and DIR/face_index.npy lists them."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    per_face = 8 * sum(int(np.prod(rec.dtype[n].shape)) for n in rec.dtype.names)
+    idx = np.arange(len(rec))
+    if per_face * len(rec) > DUMP_BYTES:
+        keep = DUMP_BYTES // (per_face + 8)
+        idx = np.sort(np.random.default_rng(0).choice(len(rec), keep, replace=False))
+        np.save(d / "face_index.npy", idx.astype(np.float64))
+    for name in rec.dtype.names:
+        np.save(d / f"{name}.npy", rec[name][idx].astype(np.float64))
 
 
 def other_workloads(crf, wl, torch, gm, om, local_rank, dev, crops, args):
@@ -453,6 +472,8 @@ def run_b200(args, rank: int, world: int, local_rank: int):
     e1.record(stream)
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out.cpu().numpy().view(crf.FACE_DTYPE))
     stage_ms, stage_launches = ctx.stage_ms()
     launches = ctx.counters()["kernel_launches"]
     clocks = sampler.stop() if rank == 0 else None
@@ -627,7 +648,12 @@ def main():
     ap.add_argument("--strong-faces", type=int, default=32768, help="total crops of the strong-scaling pass (0 = skip)")
     ap.add_argument("--c3-frames", type=int, default=64)
     ap.add_argument("--c5-images", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the last timed step (rank 0's batch) as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the records of the b200 path; the reference arm times bounded CPU samples and returns none")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     # stdout carries exactly one JSON line: library banners written to fd 1 meanwhile (NCCL prints its version there) go to stderr
     sys.stdout.flush()

@@ -56,6 +56,21 @@ def _procedural_face(rng: np.random.Generator, size: int = 130) -> np.ndarray:
     return np.clip(img, 0, 255).astype(np.uint8)
 
 
+def procedural_lfw(n: int = 20, seed: int = 2016):
+    """Stand-ins for the LFW fixtures in load_lfw's format: a procedural face pasted into a 250x250 frame, its box, a pose class and
+    no landmark annotation (parts are zeros).  The tests run on these when the fixtures are not staged."""
+    import cv2
+    rng = np.random.default_rng(seed)
+    out = []
+    for k in range(n):
+        frame = cv2.GaussianBlur(rng.integers(0, 256, (250, 250, 3), dtype=np.uint8), (0, 0), 3)
+        s = int(rng.integers(100, 161))
+        x, y = (int(v) for v in rng.integers(0, 250 - s, 2))
+        frame[y:y + s, x:x + s] = _procedural_face(rng, s)
+        out.append(dict(name=f"procedural_{k:02d}", img=frame, box=(x, y, s, s), pose=int(rng.integers(-2, 3)), parts=np.zeros((10, 2), np.int32)))
+    return out
+
+
 def _bases(rng: np.random.Generator):
     faces = load_lfw()
     if faces:

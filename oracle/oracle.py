@@ -6,7 +6,6 @@ cpu_baseline / --impl reference legs.  The product package never imports this mo
 from __future__ import annotations
 
 import ctypes as C
-import os
 import subprocess
 from pathlib import Path
 
@@ -298,6 +297,3 @@ def area_under_curve(x1, x2, mean, std) -> np.float32:
 
 def hardware_concurrency() -> int:
     return int(lib().orc_hardware_concurrency())
-
-
-REF_DATA = Path(os.environ.get("CRF_REFERENCE_DATA", "/root/reference/data"))

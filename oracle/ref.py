@@ -1,13 +1,14 @@
-"""ctypes binding of oracle/_ref/libcrf_ref.so: the REAL reference sources (unmodified, compiled where they lie under
-/root/reference by oracle/Makefile `ref`) behind the C entry points of oracle/ref_driver.cc.
+"""ctypes binding of oracle/_ref/libcrf_ref.so: the REAL reference sources (unmodified, compiled where they lie in a
+checkout of the reference project by oracle/Makefile `ref`) behind the C entry points of oracle/ref_driver.cc.
 
-TEST INFRASTRUCTURE ONLY.  The library can only be BUILT where /root/reference exists (this container); the built .so
-travels to the GPU box, but the 282 MB of text archives it loads do not, so on the GPU box the tests use the golden
-vectors this module produced here (tests/golden/make_ref_golden.py -> tests/golden/ref_*.npz).
+TEST INFRASTRUCTURE ONLY.  The reference project is not part of this repository: the library is built only when
+CRF_REFERENCE names a checkout of it (src/, include/, data/).  Without it the tests use the golden vectors this module
+produced (tests/golden/make_ref_golden.py -> tests/golden/ref_*.npz).
 """
 from __future__ import annotations
 
 import ctypes as C
+import os
 import subprocess
 from pathlib import Path
 
@@ -15,11 +16,12 @@ import numpy as np
 
 _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "_ref" / "libcrf_ref.so"
-REFERENCE = Path("/root/reference")
+REFERENCE = Path(os.environ["CRF_REFERENCE"]) if os.environ.get("CRF_REFERENCE") else None
+REF_DATA = REFERENCE / "data" if REFERENCE else None   # the shipped forests (trees_*), LFW fixtures (imgs/) and config files
 
 
 def can_build() -> bool:
-    return (REFERENCE / "src" / "FaceForest.cpp").exists()
+    return REFERENCE is not None and (REFERENCE / "src" / "FaceForest.cpp").exists()
 
 
 def available() -> bool:

@@ -9,8 +9,9 @@ ROOT = Path(__file__).resolve().parents[1]
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
 
+from oracle.ref import REF_DATA  # noqa: E402  the reference project's data/, None unless CRF_REFERENCE names a checkout
+
 GOLDEN = Path(__file__).resolve().parent / "golden"
-REF_DATA = Path("/root/reference/data")
 
 
 def pytest_configure(config):
@@ -55,11 +56,20 @@ def synth_models(crf, O, synth_dirs):
 
 
 @pytest.fixture(scope="session")
-def staged_models(crf, O):
+def shipped():
+    """True when the shipped forests and the LFW fixtures are staged (tools/stage_data.py, from a checkout of the reference
+    project).  Otherwise the tests that use them run on the synthetic forests and workloads.procedural_lfw(), against golden
+    vectors made for exactly those inputs (tests/golden/make_synth_golden.py)."""
+    from face_alignment_cvpr_2012_b200 import workloads as wl
+    return wl.staged_model_path() is not None and bool(wl.load_lfw())
+
+
+@pytest.fixture(scope="session")
+def staged_models(crf, O, shipped, synth_models):
+    if not shipped:
+        return synth_models
     from face_alignment_cvpr_2012_b200 import workloads as wl
     p = wl.staged_model_path()
-    if p is None:
-        pytest.skip("staged/model.crfb200 not present (run tools/stage_data.py where /root/reference exists)")
     return crf.Model(packed=str(p)), O.Model(packed=str(p))
 
 
@@ -69,14 +79,22 @@ def cv2_golden():
 
 
 @pytest.fixture(scope="session")
-def lfw_golden():
-    return np.load(GOLDEN / "lfw_e2e.npz")
+def lfw_golden(shipped):
+    return np.load(GOLDEN / ("lfw_e2e.npz" if shipped else "synth_lfw.npz"))
 
 
 @pytest.fixture(scope="session")
-def lfw_faces():
+def faces(shipped):
+    """The 20 LFW fixtures when staged, else their procedural stand-ins (same format, no landmark annotation)."""
     from face_alignment_cvpr_2012_b200 import workloads as wl
-    f = wl.load_lfw()
-    if not f:
-        pytest.skip("staged/imgs not present")
-    return f
+    return wl.load_lfw() if shipped else wl.procedural_lfw()
+
+
+@pytest.fixture(scope="session")
+def lfw_faces(shipped):
+    """The real LFW fixtures, for the tests that need real faces with annotated landmarks (a face detector, accuracy against the
+    annotation).  Only together with the shipped forests, which lfw_golden and staged_models pair with them."""
+    from face_alignment_cvpr_2012_b200 import workloads as wl
+    if not shipped:
+        pytest.skip("staged/imgs and staged/model.crfb200 not present (tools/stage_data.py writes them from a checkout of the reference project)")
+    return wl.load_lfw()

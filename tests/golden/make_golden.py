@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Generates the committed golden fixtures (run in the build container, where cv2 4.13 and /root/reference exist).
+"""Generates the committed golden fixtures (needs cv2 4.13 and CRF_REFERENCE naming a checkout of the reference project).
 
   cv2_stages.npz   inputs + cv2 4.13 outputs of the OpenCV-defined stages of the path (SURVEY Appendix A):
                    cvtColor(BGR2GRAY), resize(INTER_LINEAR), integral, Sobel(8U), erode/dilate 3x3, equalizeHist, Canny(-1, 5),
@@ -21,8 +21,7 @@ HERE = Path(__file__).resolve().parent
 ROOT = HERE.parents[1]
 sys.path.insert(0, str(ROOT))
 from oracle import oracle as O  # noqa: E402
-
-REF = Path("/root/reference/data")
+from oracle.ref import REF_DATA as REF  # noqa: E402  (CRF_REFERENCE: a checkout of the reference project)
 
 
 def gabor_planes_cv2(gray):

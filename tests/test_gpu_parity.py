@@ -463,10 +463,10 @@ def test_lfw_golden_end_to_end(rctx, lfw_faces, lfw_golden):
     assert abs(float(np.mean(errs)) - 0.0747) < 0.01  # SURVEY §4 / Appendix D
 
 
-def test_lfw_leaf_id_checksums(O, rctx, staged_models, lfw_faces, lfw_golden):
+def test_lfw_leaf_id_checksums(O, rctx, staged_models, faces, lfw_golden):
     _, om = staged_models
     names = lfw_golden["names"].tolist()
-    for f in lfw_faces[:6]:
+    for f in faces[:6]:
         k = names.index(f["name"])
         sc = rctx.stage_gray_resize(f["img"], f["box"])
         planes, _ = rctx.stage_channels(sc)
@@ -514,11 +514,11 @@ def test_full_size_properties(crf, staged_models, gpu):
     assert d_out.cpu().numpy().tobytes() == got.tobytes()
 
 
-def test_face_forest_class_mirror(crf, staged_models, lfw_faces, lfw_golden, gpu):
+def test_face_forest_class_mirror(crf, staged_models, faces, lfw_golden, gpu):
     gm, _ = staged_models
     ff = crf.FaceForest(model=gm)
     assert ff.is_inizialized
-    f = lfw_faces[0]
+    f = faces[0]
     face = ff.analyzeFace(f["img"], f["box"])
     k = lfw_golden["names"].tolist().index(f["name"])
     assert np.array_equal(face.ffd_cordinates, lfw_golden["recs"][k]["ffd"]) and face.bbox == tuple(f["box"])

@@ -4,7 +4,10 @@ and (b) the oracle run live on the same inputs (all record fields).  Shapes foll
 stride-1 crops through the shared-memory window kernel (config 2), default-stride crops incl. noise, 1080p frames with
 ragged boxes (config 3), head pose only (config 4), mixed resolutions up to 4K with a > 1000 px box (config 5).
 Bit-exact: head pose / variance bits, forest composition, vote counts, MeanShift iterations (exact mode), final integer
-landmarks; pre-rounding MeanShift means within TOL_PX."""
+landmarks; pre-rounding MeanShift means within TOL_PX.
+Without the shipped forests and LFW fixtures staged, the same checks run on the synthetic forests and procedural faces
+against tests/golden/synth_campaign.npz (tests/golden/make_synth_golden.py: the reference library's results on those inputs
+where it is available, else the CPU oracle's; its `source` entry says which)."""
 import importlib.util
 from pathlib import Path
 
@@ -16,11 +19,11 @@ TOL_PX = 0.5
 GOLDEN = Path(__file__).resolve().parent / "golden"
 
 
-def _load_sets():
+def _load_sets(faces):
     spec = importlib.util.spec_from_file_location("make_ref_golden", GOLDEN / "make_ref_golden.py")
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)
-    return m.campaign_sets()
+    return m.campaign_sets(faces)
 
 
 @pytest.fixture(scope="module")
@@ -31,13 +34,14 @@ def gpu(crf):
 
 
 @pytest.fixture(scope="module")
-def sets(lfw_faces):
-    return _load_sets()
+def sets(faces):
+    return _load_sets(faces)
 
 
 @pytest.fixture(scope="module")
-def ref_golden():
-    return np.load(GOLDEN / "ref_campaign.npz")
+def ref_golden(shipped):
+    """The reference's own results on the shipped forests; on the synthetic forests, synth_campaign.npz (see its `source`)."""
+    return np.load(GOLDEN / ("ref_campaign.npz" if shipped else "synth_campaign.npz"))
 
 
 def _list_from_record(rec, ntrees=20):
@@ -190,7 +194,7 @@ def test_compose_knife_edges(crf, O, gpu, staged_models):
     assert bad == 0, f"{bad} of {len(hp)} compositions differ"
 
 
-def test_cv2_gabor_planes_downstream(crf, O, gpu, staged_models, lfw_faces):
+def test_cv2_gabor_planes_downstream(crf, O, gpu, staged_models, faces):
     """The canonical (separable) Gabor arithmetic against cv2's own filter2D (DFT path for kernels >= 9x9) on the 20 LFW faces
     + 64 synthetic crops: the 8-bit planes differ by +-1 LSB at a rate <= 2e-4, and pushing BOTH sets of planes through the
     shipped forests on the GPU moves no landmark by more than 0.5 px."""
@@ -200,7 +204,7 @@ def test_cv2_gabor_planes_downstream(crf, O, gpu, staged_models, lfw_faces):
     ctx = crf.Context(gm, 0)
     bank = O.gabor_bank()
     crops, _ = wl.make_crops(64, seed=4806)
-    items = [(f["img"], f["box"]) for f in lfw_faces] + [(c, (0, 0, 100, 100)) for c in crops]
+    items = [(f["img"], f["box"]) for f in faces] + [(c, (0, 0, 100, 100)) for c in crops]
     n_px = n_diff = n_leaf = n_leaf_diff = 0
     worst = 0.0
     for img, box in items:

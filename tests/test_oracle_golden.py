@@ -130,20 +130,17 @@ def test_area_under_curve_sums_to_one(O):
     assert abs(tot - 1.0) < 0.06
 
 
-def test_cv2_gabor_planes_downstream(O, lfw_faces):
+def test_cv2_gabor_planes_downstream(O, staged_models, faces):
     """What the +-1-LSB distance between the canonical Gabor arithmetic and cv2's filter2D (DFT path for kernels >= 9x9) does
     downstream: cv2-made planes and the oracle's planes through the shipped forests on LFW faces + synthetic crops.  Observed on
     the full set (20 faces + 64 crops, tests/test_gpu_reference_campaign.py runs it on the GPU): 2.8e-5 of the u8 samples differ,
     1e-5 of the leaf ids, landmarks move by <= 0.02 px."""
     import cv2
     from face_alignment_cvpr_2012_b200 import workloads as wl
-    p = wl.staged_model_path()
-    if p is None:
-        pytest.skip("staged/model.crfb200 not present")
-    om = O.Model(packed=str(p))
+    _, om = staged_models
     bank = O.gabor_bank()
     crops, _ = wl.make_crops(6, seed=4806)
-    items = [(f["img"], f["box"]) for f in lfw_faces[:6]] + [(c, (0, 0, 100, 100)) for c in crops]
+    items = [(f["img"], f["box"]) for f in faces[:6]] + [(c, (0, 0, 100, 100)) for c in crops]
     n_px = n_diff = n_leaf = n_leaf_diff = 0
     worst = 0.0
     for img, box in items:

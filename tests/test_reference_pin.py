@@ -7,33 +7,41 @@ trees through the reference's serialize() methods, Forest/Tree::evaluateMT + Tre
 FaceForest::analyzeFace, getFacialFeaturesVotesMT (vote lists, in order) and MeanShift::shift.  The OpenCV arithmetic
 under the reference comes from the stand-in, i.e. from the oracle's cv2-pinned stages (tests/test_oracle_golden.py).
 
-Needs /root/reference (text archives + sources), so these run in the build container; the GPU box gets the golden
-vectors made from the same library (tests/golden/make_ref_golden.py, tests/golden/ref_*.npz)."""
+Needs the reference's library: built from a checkout of the reference project named by CRF_REFERENCE, or a prebuilt
+oracle/_ref/libcrf_ref.so.  The forests are the shipped text archives of that checkout when present, else the synthetic
+ones (synthetic_model.py writes the reference's own archive format); the faces are the LFW fixtures of that checkout,
+else workloads.procedural_lfw().  Without the library the GPU tests use the golden vectors made from it
+(tests/golden/make_ref_golden.py, tests/golden/ref_*.npz)."""
 import numpy as np
 import pytest
 
 from conftest import REF_DATA
 
-HP_DIR, FFD_DIR = REF_DATA / "trees_headpose", REF_DATA / "trees_ffd"
+HP_DIR, FFD_DIR = (REF_DATA / "trees_headpose", REF_DATA / "trees_ffd") if REF_DATA else (None, None)
 
 
 @pytest.fixture(scope="module")
 def R():
     from oracle import ref
-    if not ref.can_build() or not HP_DIR.exists():
-        pytest.skip("/root/reference not present: the real-reference build and its text archives live in the build container")
+    if not ref.available():
+        pytest.skip("no reference library: oracle/_ref/libcrf_ref.so is absent and CRF_REFERENCE names no checkout to build it from")
     ref.build()
     return ref
 
 
 @pytest.fixture(scope="module")
-def ff(R):
-    return R.FaceForest(str(HP_DIR), str(FFD_DIR))
+def archives(synth_dirs):
+    return (str(HP_DIR), str(FFD_DIR)) if HP_DIR is not None and HP_DIR.exists() else synth_dirs
 
 
 @pytest.fixture(scope="module")
-def om(O, R):
-    return O.Model(str(HP_DIR), str(FFD_DIR))
+def ff(R, archives):
+    return R.FaceForest(*archives)
+
+
+@pytest.fixture(scope="module")
+def om(O, R, archives):
+    return O.Model(*archives)
 
 
 def _planes(rng, C=38, H=125, W=125):
@@ -45,6 +53,9 @@ def _planes(rng, C=38, H=125, W=125):
 
 def _lfw():
     import cv2
+    if REF_DATA is None or not (REF_DATA / "imgs" / "index_random_subset.txt").exists():
+        from face_alignment_cvpr_2012_b200 import workloads as wl
+        return [(f["img"], f["box"]) for f in wl.procedural_lfw()]
     out = []
     for line in (REF_DATA / "imgs" / "index_random_subset.txt").read_text().split("\n"):
         t = line.split()
@@ -81,7 +92,7 @@ def test_leaf_ids_and_headpose_match_reference(O, R, ff, om, stride, H, W):
     rs.close(); os_.close()
 
 
-def test_eval_test_matches_reference(O, R, om):
+def test_eval_test_matches_reference(O, R):
     """ImageSample::evalTest on random rectangles (the integer mean-difference of SURVEY A.6) against the stage the oracle's
     leaf ids are built on — checked indirectly above; here directly against the integer formula."""
     rng = np.random.default_rng(7)

@@ -1,5 +1,6 @@
 import sys, time
-sys.path.insert(0, '/root/repo')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 import numpy as np
 import face_alignment_cvpr_2012_b200 as crf
 from face_alignment_cvpr_2012_b200 import workloads as wl

@@ -1,12 +1,13 @@
 #!/usr/bin/env python
-"""Stage what the GPU box needs from /root/reference/data into staged/ (git-ignored; travels with gpurun):
+"""Stage what the tests and the benchmark use from the reference project's data/ (checkout named by CRF_REFERENCE) into
+staged/ (git-ignored):
 
   staged/model.crfb200   packed binary image of data/trees_headpose + data/trees_ffd (crf_model_save_packed)
   staged/imgs/           the 20 LFW jpgs + index_random_subset.txt (fixtures for C1 and the synthetic generators)
   staged/trees_headpose, staged/trees_ffd   the 115 Boost text archives themselves (282 MB): what the REAL reference code
                          (oracle/_ref/libcrf_ref.so, bench.py's cpu_baseline kind "reference") loads on the GPU box
 
-/root/reference does not exist on the GPU box; nothing at run time reads it.
+Nothing at run time reads the reference checkout itself.
 """
 import shutil
 import sys
@@ -15,10 +16,12 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
-REF = Path("/root/reference/data")
+from oracle.ref import REF_DATA as REF  # noqa: E402
 
 
 def main() -> int:
+    if REF is None:
+        raise SystemExit("set CRF_REFERENCE to a checkout of the reference project")
     import face_alignment_cvpr_2012_b200 as crf
     crf.build()
     out = ROOT / "staged"
