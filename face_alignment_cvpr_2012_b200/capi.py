@@ -20,6 +20,7 @@ NUM_POSE_FORESTS = 5
 NUM_STAGES = 8
 STAGE_NAMES = ["resize", "plain_channels", "gabor", "hp_traverse", "hp_reduce", "ffd_traverse", "votes", "meanshift"]
 MAX_SCALED_H = 521
+FACE_NOT_ANALYSED = 8   # crf_face_t::flags of a detected box the analysis path cannot take (crf_analyze_images)
 
 
 class CrfError(RuntimeError):
@@ -66,7 +67,7 @@ EXPORTS = [
     "crf_stage_compose", "crf_stage_compose_batch", "crf_stage_votes_meanshift", "crf_stage_meanshift",
     "crf_model_load_forest", "crf_model_set_features", "crf_model_get_features", "crf_model_leaf_dump", "crf_stage_feature_channels",
     "crf_stage_eval_patches", "crf_stage_eval_tests", "crf_stage_eval_tests_sum", "crf_model_load_tree", "crf_stage_meanshift_opt", "crf_stage_area_under_curve",
-    "crf_cascade_load", "crf_cascade_free", "crf_cascade_info", "crf_detect_faces",
+    "crf_cascade_load", "crf_cascade_free", "crf_cascade_info", "crf_detect_faces", "crf_detect_faces_batch", "crf_analyze_images",
     "crf_multi_create", "crf_multi_destroy", "crf_multi_device_count", "crf_multi_ctx", "crf_multi_analyze_batch", "crf_multi_analyze_crops",
 ]
 
@@ -148,6 +149,10 @@ def lib() -> C.CDLL:
     L.crf_cascade_free.restype = None
     L.crf_cascade_info.argtypes = [vp, i32p, i32p, i32p, i32p]
     L.crf_detect_faces.argtypes = [vp, vp, u8p, C.c_int, C.c_int, C.c_size_t, C.c_double, C.c_int, C.c_int, C.POINTER(Rect), C.c_int]
+    L.crf_detect_faces_batch.argtypes = [vp, vp, C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_double, C.c_int, C.c_int,
+                                         C.POINTER(Rect), i32p, C.c_int]
+    L.crf_analyze_images.argtypes = [vp, vp, C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_double, C.c_int, C.c_int,
+                                     C.POINTER(Rect), i32p, vp, C.c_int]
     L.crf_multi_create.argtypes = [vp, i32p, C.c_int, C.POINTER(Options), C.POINTER(vp)]
     L.crf_multi_destroy.argtypes = [vp]
     L.crf_multi_destroy.restype = None

@@ -196,9 +196,11 @@ struct crf_ctx {
   int ms_variant = 3;   // resident MeanShift CTAs per SM the kernel is compiled for (register cap); CRF_MS_VARIANT overrides
   size_t work_budget = (size_t)64 << 30;  // bytes of work buffers a launch may use (min(64 GB, half of the free memory at creation))
   StageTimer timer;
-  // face-box source (haar.cuh): device image of the last cascade used + pyramid-level buffers
+  // face-box source (haar.cuh): device image of the last cascade used + the buffers of a group of frames
   const struct crf_cascade* haar_cached = nullptr;
-  Buf d_haar_stages, d_haar_weak, d_haar_feats, d_haar_level, d_haar_S, d_haar_Q, d_haar_flags;
+  Buf d_haar_stages, d_haar_weak, d_haar_feats, d_haar_frames, d_haar_S, d_haar_Q, d_haar_flags, d_haar_list[2], d_haar_rows, d_haar_levels, d_haar_counts, d_haar_cand;
+  // first stage of each cascade stage group after the first (CRF_HAAR_SPLIT="a,b,..."; measured, DESIGN §4.5)
+  std::vector<int> haar_split{3, 8};
 };
 
 namespace crf {
@@ -293,15 +295,22 @@ static bool is_pinned_host(const void* p) {
   return a.type == cudaMemoryTypeHost;
 }
 
-// src/FaceForest.cpp:199-204 (scale, scaled size) + the argument checks of the path.
-static int make_desc(const crf_ctx* c, int rows, int cols, size_t step, size_t img_off, const crf_rect_t& b, FaceDesc& d) {
-  if (b.x < 0 || b.y < 0 || b.width <= 0 || b.height <= 0 || (long long)b.x + b.width > cols || (long long)b.y + b.height > rows)
-    return fail(CRF_ERR_ARG, "bbox outside image");
+// The box checks of the analysis path: nullptr if the box can be analysed, else the reason.
+static const char* box_error(int rows, int cols, const crf_rect_t& b) {
+  if (b.x < 0 || b.y < 0 || b.width <= 0 || b.height <= 0 || (long long)b.x + b.width > cols || (long long)b.y + b.height > rows) return "bbox outside image";
   const float scale = static_cast<float>(125) / static_cast<float>(b.width);
   const int sw = (int)(b.width * scale), sh = (int)(b.height * scale);
-  if (sw <= kPatch || sh <= kPatch) return fail(CRF_ERR_ARG, "scaled face smaller than a patch");
-  if (sw > 125) return fail(CRF_ERR_ARG, "scaled face wider than face_size");
-  if (sh > CRF_MAX_SCALED_H) return fail(CRF_ERR_ARG, "scaled face taller than CRF_MAX_SCALED_H (f32 integral exactness limit)");
+  if (sw <= kPatch || sh <= kPatch) return "scaled face smaller than a patch";
+  if (sw > 125) return "scaled face wider than face_size";
+  if (sh > CRF_MAX_SCALED_H) return "scaled face taller than CRF_MAX_SCALED_H (f32 integral exactness limit)";
+  return nullptr;
+}
+
+// src/FaceForest.cpp:199-204 (scale, scaled size) + the argument checks of the path.
+static int make_desc(const crf_ctx* c, int rows, int cols, size_t step, size_t img_off, const crf_rect_t& b, FaceDesc& d) {
+  if (const char* e = box_error(rows, cols, b)) return fail(CRF_ERR_ARG, e);
+  const float scale = static_cast<float>(125) / static_cast<float>(b.width);
+  const int sw = (int)(b.width * scale), sh = (int)(b.height * scale);
   d.img_off = img_off; d.img_step = step;
   d.bx = b.x; d.by = b.y; d.bw = b.width; d.bh = b.height;
   d.W = sw; d.H = sh; d.scale = scale; d.pad = 0;
@@ -792,6 +801,236 @@ static int analyze_host(crf_ctx* c, const uint8_t* const* images, int n_images, 
 
 #include "haar.cuh"
 
+namespace crf {
+// Faces whose descriptors point into frames already in device memory (d_imgs): descriptors up, records into d_out (n x crf_face_t),
+// chunked like the host path; faces flagged for the worst-case capacities are re-run wide.  Returns when d_out is complete.
+static int analyze_resident(crf_ctx* c, const std::vector<FaceDesc>& descs, int Hmax, const uint8_t* d_imgs, crf_face_t* d_out, bool headpose_only) {
+  const int n = (int)descs.size();
+  int rc;
+  c->w = &c->ws[0];
+  cudaStream_t s0 = c->ws[0].stream;
+  if ((rc = c->d_fd.reserve((size_t)n * sizeof(FaceDesc)))) return rc;
+  CU(cudaMemcpyAsync(c->d_fd.p, descs.data(), (size_t)n * sizeof(FaceDesc), cudaMemcpyHostToDevice, s0));
+  CU(cudaMemsetAsync(d_out, 0, (size_t)n * sizeof(crf_face_t), s0));
+  const int chunk = pick_chunk(c, Hmax, headpose_only);
+  Plan p; p.n = std::min(n, chunk); p.Hmax = Hmax; p.nplanes = c->layout.nplanes; p.need_gabor = c->layout.gabor_first >= 0; p.hp_stride = c->opt.hp_stride; p.ffd_stride = c->opt.ffd_stride; p.tree_cap = c->mp_ntrees_cfg;
+  p.need_ffd = !headpose_only;
+  const int nsets = n > chunk ? c->nstreams : 1;
+  for (int k = 0; k < nsets; k++) { c->w = &c->ws[k]; if ((rc = ensure(c, p))) return rc; }
+  CU(cudaStreamSynchronize(s0));
+  // consecutive chunks alternate between the two streams / work sets
+  int k = 0;
+  for (int f0 = 0; f0 < n; f0 += chunk, k++) {
+    const int m = std::min(chunk, n - f0);
+    c->w = &c->ws[k % nsets];
+    if ((rc = run_faces(c, c->d_fd.as<FaceDesc>() + f0, m, Hmax, d_imgs, d_out + f0, headpose_only, c->mp_ntrees_cfg, nullptr))) return rc;
+  }
+  for (int q = 0; q < nsets; q++) CU(cudaStreamSynchronize(c->ws[q].stream));
+  c->w = &c->ws[0];
+  if (!headpose_only) {
+    // faces whose composition or vote count exceeded the batched capacities: fetch the flags, re-run those faces wide
+    // (4 bytes come back, not the records: the flag is counted on the device)
+    int n_wide = 0;
+    CU(cudaMemsetAsync(c->d_misc.p, 0, 4, s0));
+    k_count_wide<<<(n + 255) / 256, 256, 0, s0>>>(d_out, n, c->d_misc.as<int>());
+    KCHECK(); count_launch(c, CRF_STAGE_MEANSHIFT);
+    CU(cudaMemcpyAsync(&n_wide, c->d_misc.p, 4, cudaMemcpyDeviceToHost, s0));
+    CU(cudaStreamSynchronize(s0));
+    if (n_wide > 0) {
+      std::vector<crf_face_t> tmp((size_t)n);
+      CU(cudaMemcpyAsync(tmp.data(), d_out, (size_t)n * sizeof(crf_face_t), cudaMemcpyDeviceToHost, s0));
+      CU(cudaStreamSynchronize(s0));
+      std::vector<int> wide;
+      for (int i = 0; i < n; i++) if (tmp[(size_t)i].flags & 6) wide.push_back(i);
+      if (!wide.empty() && (rc = rerun_wide(c, c->d_fd.as<FaceDesc>(), descs, d_imgs, d_out, wide))) return rc;
+      CU(cudaStreamSynchronize(s0));
+    }
+  }
+  c->cnt.faces += n;
+  c->timer.collect();
+  return pull_counters(c);
+}
+
+// ---- detectMultiScale on groups of frames (haar.cuh) ------------------------------------------------------------------------
+// Frames resident at once: at most this many, and no more than half the work budget holds (the analysis of a group's faces needs
+// the rest), so that a long video or a batch of 4K frames is not uploaded in one piece.
+constexpr int kDetectGroupFrames = 64;
+
+struct DetectPlan {
+  std::vector<HaarLevel> levels;
+  int rows_pf = 0;                 // window rows of one frame over all levels
+  size_t int_pf = 0, win_pf = 0;   // integral elements / windows of one frame over all levels
+};
+
+// the scales of CascadeClassifierImpl::detectMultiScale (flags 0, no maxSize); levels below min_size are not built
+static DetectPlan detect_plan(const Cascade& K, int rows, int cols, double scale_factor, int min_size) {
+  DetectPlan p;
+  for (double factor = 1;; factor *= scale_factor) {
+    HaarLevel L{};
+    L.factor = factor;
+    L.win_w = (int)std::lrint(K.win_w * factor); L.win_h = (int)std::lrint(K.win_h * factor);
+    L.sw = (int)std::lrint(cols / factor); L.sh = (int)std::lrint(rows / factor);
+    if (L.win_w > cols || L.win_h > rows || L.sw < K.win_w || L.sh < K.win_h) break;
+    if (L.win_w < min_size || L.win_h < min_size) continue;
+    L.scale_x = 1. / ((double)L.sw / cols); L.scale_y = 1. / ((double)L.sh / rows);
+    L.ystep = factor > 2. ? 1 : 2;
+    L.nx = (L.sw - K.win_w + 1 + L.ystep - 1) / L.ystep; L.ny = (L.sh - K.win_h + 1 + L.ystep - 1) / L.ystep;
+    L.row_off = p.rows_pf;
+    L.int_fs = (size_t)(L.sw + 1) * (L.sh + 1);
+    p.rows_pf += L.ny;
+    p.int_pf += L.int_fs;
+    p.win_pf += (size_t)L.nx * L.ny;
+    p.levels.push_back(L);
+  }
+  return p;
+}
+
+// Frames [f0, f0 + nf) into d_haar_frames, frame k at k * rows * step.  Pinned frames are copied straight (frames adjacent in host memory
+// in one copy); pageable ones are packed into the two pinned staging buffers by a few threads and copied from there.
+static int upload_frames(crf_ctx* c, const uint8_t* const* images, int f0, int nf, int rows, size_t step, cudaStream_t s) {
+  const size_t fb = (size_t)rows * step;
+  uint8_t* d = c->d_haar_frames.as<uint8_t>();
+  std::vector<int> pageable;
+  for (int k = 0; k < nf;) {
+    if (!is_pinned_host(images[f0 + k])) { pageable.push_back(k++); continue; }
+    int j = k + 1;
+    while (j < nf && images[f0 + j] == images[f0 + j - 1] + fb && is_pinned_host(images[f0 + j])) j++;
+    CU(cudaMemcpyAsync(d + (size_t)k * fb, images[f0 + k], (size_t)(j - k) * fb, cudaMemcpyHostToDevice, s));
+    k = j;
+  }
+  const size_t per = std::max<size_t>(1, ((size_t)64 << 20) / fb);   // frames per staging buffer: ~64 MB
+  for (size_t p0 = 0, b = 0; p0 < pageable.size(); p0 += per, b ^= 1) {
+    const size_t m = std::min(per, pageable.size() - p0);
+    CU(cudaEventSynchronize(c->ev_copied[b]));   // the buffer's previous copy has left the host
+    if (c->h_stage_bytes[b] < per * fb) {
+      if (c->h_stage[b]) cudaFreeHost(c->h_stage[b]);
+      c->h_stage[b] = nullptr; c->h_stage_bytes[b] = 0;
+      CU(cudaHostAlloc((void**)&c->h_stage[b], per * fb, cudaHostAllocDefault));
+      c->h_stage_bytes[b] = per * fb;
+    }
+    uint8_t* st = c->h_stage[b];
+    parallel_for((int)m, m * fb, [&](int i) { std::memcpy(st + (size_t)i * fb, images[f0 + pageable[p0 + i]], fb); });
+    for (size_t i = 0; i < m;) {   // runs of consecutive frame slots in one copy
+      size_t j = i + 1;
+      while (j < m && pageable[p0 + j] == pageable[p0 + j - 1] + 1) j++;
+      CU(cudaMemcpyAsync(d + (size_t)pageable[p0 + i] * fb, st + i * fb, (j - i) * fb, cudaMemcpyHostToDevice, s));
+      i = j;
+    }
+    CU(cudaEventRecord(c->ev_copied[b], s));
+  }
+  c->cnt.h2d_bytes += (size_t)nf * fb;
+  return CRF_OK;
+}
+
+// detectMultiScale on n_images equal-size frames, a group of frames at a time.  After a group's boxes are grouped, per_group(f0, nf, boxes)
+// runs while the group's frames are still in d_haar_frames (frame f0 + k at k * rows * step); boxes[k] are frame f0 + k's.
+template <class F>
+static int detect_frames(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step,
+                         double scale_factor, int min_neighbors, int min_size, F&& per_group) {
+  CU(cudaSetDevice(c->device));
+  c->w = &c->ws[0];
+  cudaStream_t s = c->w->stream;
+  int rc;
+  const Cascade& K = cas->c;
+  if (c->haar_cached != cas) {
+    if ((rc = upload(c->d_haar_stages, K.stages, s)) || (rc = upload(c->d_haar_weak, K.weak, s)) || (rc = upload(c->d_haar_feats, K.features, s))) return rc;
+    c->haar_cached = cas;
+  }
+  const HaarDev dev{c->d_haar_stages.as<HaarStage>(), c->d_haar_weak.as<HaarWeak>(), c->d_haar_feats.as<HaarFeature>(), (int)K.stages.size(), K.win_w, K.win_h};
+  // stage groups: [0, split[0]), [split[0], split[1]), ..., up to the last stage
+  std::vector<int> bounds;
+  for (int b : c->haar_split) if (b > (bounds.empty() ? 0 : bounds.back()) && b < dev.nstages) bounds.push_back(b);
+  bounds.push_back(dev.nstages);
+  DetectPlan plan = detect_plan(K, rows, cols, scale_factor, min_size);
+  const size_t fb = (size_t)rows * step;
+  // work lists hold 32-bit flag indices
+  if (plan.win_pf >= ((size_t)1 << 31)) return fail(CRF_ERR_ARG, "frame too large for the detector (2^31 windows)");
+  const size_t per_frame = fb + plan.int_pf * 8 + plan.win_pf * (1 + 2 * sizeof(uint2)) + (size_t)plan.rows_pf * 4;
+  int group = (int)std::min<size_t>(kDetectGroupFrames, std::max<size_t>(1, c->work_budget / 2 / per_frame));
+  if (!plan.win_pf) group = kDetectGroupFrames;
+  else group = (int)std::min<size_t>((size_t)group, (((size_t)1 << 32) - 1) / plan.win_pf);
+  const int nl = (int)plan.levels.size();
+  std::vector<std::vector<crf_rect_t>> boxes;
+  std::vector<int> frame_count;
+  for (int f0 = 0; f0 < n_images; f0 += group) {
+    const int nf = std::min(group, n_images - f0);
+    boxes.assign((size_t)nf, {});
+    if (nl > 0) {
+      size_t io = 0, fo = 0;
+      for (HaarLevel& L : plan.levels) { L.int_off = io; io += (size_t)nf * L.int_fs; L.flag_off = fo; fo += (size_t)nf * L.nx * L.ny; }
+      const int nrows = nf * plan.rows_pf;
+      if ((rc = c->d_haar_frames.reserve((size_t)nf * fb)) || (rc = c->d_haar_S.reserve(io * 4)) || (rc = c->d_haar_Q.reserve(io * 4)) ||
+          (rc = c->d_haar_flags.reserve(fo)) || (rc = c->d_haar_list[0].reserve(fo * sizeof(uint2))) || (rc = c->d_haar_list[1].reserve(fo * sizeof(uint2))) ||
+          (rc = c->d_haar_rows.reserve((size_t)nrows * 4)) || (rc = c->d_haar_counts.reserve((size_t)(kDetectGroupFrames + 4) * 4)))
+        return rc;
+      if ((rc = upload_frames(c, images, f0, nf, rows, step, s))) return rc;
+      if ((rc = upload(c->d_haar_levels, plan.levels, s))) return rc;
+      unsigned* lists_n = c->d_haar_counts.as<unsigned>();   // [0], [1]: lengths of the two work lists; [4...]: candidates per frame
+      int* fcount = c->d_haar_counts.as<int>() + 4;
+      CU(cudaMemsetAsync(lists_n, 0, 4 * sizeof(unsigned), s));
+      uint32_t* S = c->d_haar_S.as<uint32_t>();
+      uint32_t* Q = c->d_haar_Q.as<uint32_t>();
+      uint8_t* flags = c->d_haar_flags.as<uint8_t>();
+      uint2* list[2] = {c->d_haar_list[0].as<uint2>(), c->d_haar_list[1].as<uint2>()};
+      for (const HaarLevel& L : plan.levels) {
+        k_haar_rows<<<dim3((L.sh + 7) / 8, nf), 256, 0, s>>>(c->d_haar_frames.as<uint8_t>(), fb, rows, cols, step, L, S, Q);
+        k_haar_cols<<<dim3((L.sw + 1 + 31) / 32, nf), dim3(32, 32), 0, s>>>(L, S, Q);
+        k_haar_eval_first<<<dim3((L.nx + 127) / 128, L.ny, nf), 128, 0, s>>>(L, S, Q, dev, bounds[0], flags, list[0], lists_n);
+        KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 3);
+      }
+      const HaarLevel* d_levels = c->d_haar_levels.as<HaarLevel>();
+      for (size_t g = 1; g < bounds.size(); g++) {
+        const int in = (int)((g - 1) & 1), out = (int)(g & 1);
+        if (g >= 2) CU(cudaMemsetAsync(lists_n + out, 0, sizeof(unsigned), s));
+        k_haar_eval_list<<<c->sm_count * 8, 128, 0, s>>>(d_levels, nl, S, dev, bounds[g - 1], bounds[g], list[in], lists_n + in, flags, list[out], lists_n + out);
+        KCHECK(); count_launch(c, CRF_STAGE_RESIZE);
+      }
+      int* d_rows = c->d_haar_rows.as<int>();
+      k_haar_scan<true><<<(nrows + 7) / 8, 256, 0, s>>>(d_levels, nl, nrows, plan.rows_pf, flags, d_rows, nullptr, nullptr);
+      k_haar_row_offsets<<<nf, 1024, 0, s>>>(plan.rows_pf, d_rows, fcount);
+      KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 2);
+      frame_count.assign((size_t)nf, 0);
+      CU(cudaMemcpyAsync(frame_count.data(), fcount, (size_t)nf * 4, cudaMemcpyDeviceToHost, s));
+      CU(cudaStreamSynchronize(s));
+      size_t total = 0;
+      for (int v : frame_count) total += (size_t)v;
+      if ((rc = c->d_haar_cand.reserve(std::max<size_t>(total, 1) * sizeof(crf_rect_t)))) return rc;
+      k_haar_scan<false><<<(nrows + 7) / 8, 256, 0, s>>>(d_levels, nl, nrows, plan.rows_pf, flags, d_rows, fcount, c->d_haar_cand.as<crf_rect_t>());
+      KCHECK(); count_launch(c, CRF_STAGE_RESIZE);
+      std::vector<crf_rect_t> cand(total);
+      if (total) CU(cudaMemcpyAsync(cand.data(), c->d_haar_cand.p, total * sizeof(crf_rect_t), cudaMemcpyDeviceToHost, s));
+      CU(cudaStreamSynchronize(s));
+      c->cnt.d2h_bytes += (size_t)nf * 4 + total * sizeof(crf_rect_t);
+      for (int k = 0, o = 0; k < nf; o += frame_count[(size_t)k], k++) boxes[(size_t)k].assign(cand.begin() + o, cand.begin() + o + frame_count[(size_t)k]);
+      // cv::groupRectangles per frame; quadratic in a frame's candidates, so the work estimate is their square
+      size_t work = 0;
+      for (int v : frame_count) work += (size_t)v * v;
+      parallel_for(nf, work * 64, [&](int k) { group_rectangles(boxes[(size_t)k], min_neighbors, 0.2); });
+    }
+    if ((rc = per_group(f0, nf, boxes))) return rc;
+  }
+  return CRF_OK;
+}
+
+// FaceForest::detectFace's enlargement (src/FaceForest.cpp:147-157): 5 % of the width left and right, 15 % of the WIDTH added to the height
+// twice, intersected with the frame (intersect() of src/face_utils.cpp:325-347 returns (0, 0, 0, 0) when they do not overlap).
+static crf_rect_t enlarge_detection(const crf_rect_t& r, int rows, int cols) {
+  const int ox = (int)(r.width * 0.05), oy = (int)(r.width * 0.15);
+  const int x0 = std::max(r.x - ox, 0), y0 = std::max(r.y, 0), x1 = std::min(r.x - ox + r.width + 2 * ox, cols), y1 = std::min(r.y + r.height + 2 * oy, rows);
+  return x1 > x0 && y1 > y0 ? crf_rect_t{x0, y0, x1 - x0, y1 - y0} : crf_rect_t{0, 0, 0, 0};
+}
+
+static int detect_args(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, double scale_factor, int cap,
+                       const void* out) {
+  if (!c) return fail(CRF_ERR_STATE, "context is not initialised");
+  if (!cas || n_images < 0 || (n_images > 0 && !images) || rows < 1 || cols < 1 || step < (size_t)cols * 3 || !(scale_factor > 1.0) || cap < 0 || (cap > 0 && !out))
+    return fail(CRF_ERR_ARG, "bad argument");
+  for (int i = 0; i < n_images; i++) if (!images[i]) return fail(CRF_ERR_ARG, "null frame");
+  return CRF_OK;
+}
+}  // namespace crf
+
+
 // =============================================================================================
 // C ABI
 // =============================================================================================
@@ -821,71 +1060,72 @@ int crf_cascade_info(const crf_cascade* c, int* win_w, int* win_h, int* nstages,
 
 int crf_detect_faces(crf_ctx* c, const crf_cascade* cas, const uint8_t* bgr, int rows, int cols, size_t step, double scale_factor, int min_neighbors, int min_size,
                      crf_rect_t* out, int cap) {
-  if (!c) return fail(CRF_ERR_STATE, "context is not initialised");
-  if (!cas || !bgr || rows < 1 || cols < 1 || step < (size_t)cols * 3 || !(scale_factor > 1.0) || cap < 0 || (cap > 0 && !out)) return fail(CRF_ERR_ARG, "bad argument");
-  CU(cudaSetDevice(c->device));
-  cudaStream_t s = c->w->stream;
-  int rc;
-  const Cascade& K = cas->c;
-  if (c->haar_cached != cas) {
-    if ((rc = upload(c->d_haar_stages, K.stages, s)) || (rc = upload(c->d_haar_weak, K.weak, s)) || (rc = upload(c->d_haar_feats, K.features, s))) return rc;
-    c->haar_cached = cas;
-  }
-  if ((rc = c->d_imgs[0].reserve((size_t)rows * step))) return rc;
-  CU(cudaMemcpyAsync(c->d_imgs[0].p, bgr, (size_t)rows * step, cudaMemcpyHostToDevice, s));
-  c->cnt.h2d_bytes += (size_t)rows * step;
-  // the scales of CascadeClassifierImpl::detectMultiScale (flags 0, no maxSize)
-  struct Level { double factor; int win_w, win_h, sw, sh, ystep, nx, ny; size_t flag_off; };
-  std::vector<Level> levels;
-  size_t flag_bytes = 0;
-  for (double factor = 1;; factor *= scale_factor) {
-    Level L;
-    L.factor = factor;
-    L.win_w = (int)std::lrint(K.win_w * factor); L.win_h = (int)std::lrint(K.win_h * factor);
-    L.sw = (int)std::lrint(cols / factor); L.sh = (int)std::lrint(rows / factor);
-    if (L.win_w > cols || L.win_h > rows || L.sw < K.win_w || L.sh < K.win_h) break;
-    if (L.win_w < min_size || L.win_h < min_size) continue;
-    L.ystep = factor > 2. ? 1 : 2;
-    L.nx = (L.sw - K.win_w + 1 + L.ystep - 1) / L.ystep; L.ny = (L.sh - K.win_h + 1 + L.ystep - 1) / L.ystep;
-    L.flag_off = flag_bytes;
-    flag_bytes += (size_t)L.nx * L.ny;
-    levels.push_back(L);
-  }
-  std::vector<crf_rect_t> cand;
-  if (!levels.empty()) {
-    const Level& L0 = levels[0];
-    const size_t npx = (size_t)(L0.sw + 1) * (L0.sh + 1);
-    if ((rc = c->d_haar_level.reserve((size_t)L0.sw * L0.sh)) || (rc = c->d_haar_S.reserve(npx * 4)) || (rc = c->d_haar_Q.reserve(npx * 4)) || (rc = c->d_haar_flags.reserve(flag_bytes))) return rc;
-    for (const Level& L : levels) {
-      k_haar_level<<<dim3((L.sw + 127) / 128, L.sh), 128, 0, s>>>(c->d_imgs[0].as<uint8_t>(), rows, cols, step, c->d_haar_level.as<uint8_t>(), L.sh, L.sw,
-                                                                   1. / ((double)L.sw / cols), 1. / ((double)L.sh / rows));
-      k_haar_rowscan<<<(L.sh + 7) / 8, 256, 0, s>>>(c->d_haar_level.as<uint8_t>(), L.sh, L.sw, c->d_haar_S.as<uint32_t>(), c->d_haar_Q.as<uint32_t>());
-      k_haar_colscan<<<(L.sw + 1 + 127) / 128, 128, 0, s>>>(L.sh, L.sw, c->d_haar_S.as<uint32_t>(), c->d_haar_Q.as<uint32_t>());
-      k_haar_eval<<<dim3((L.nx + 127) / 128, L.ny), 128, 0, s>>>(c->d_haar_S.as<uint32_t>(), c->d_haar_Q.as<uint32_t>(), L.sw, L.sh, K.win_w, K.win_h, L.ystep, L.nx, L.ny,
-                                                                 c->d_haar_stages.as<HaarStage>(), (int)K.stages.size(), c->d_haar_weak.as<HaarWeak>(), c->d_haar_feats.as<HaarFeature>(),
-                                                                 c->d_haar_flags.as<uint8_t>() + L.flag_off);
-      KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 4);
-    }
-    std::vector<uint8_t> flags(flag_bytes);
-    CU(cudaMemcpyAsync(flags.data(), c->d_haar_flags.p, flag_bytes, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    c->cnt.d2h_bytes += flag_bytes;
-    // CascadeClassifierInvoker's scan: windows in raster order, one extra step after a window the first stage rejected
-    for (const Level& L : levels) {
-      const uint8_t* f = flags.data() + L.flag_off;
-      for (int iy = 0; iy < L.ny; iy++)
-        for (int ix = 0; ix < L.nx; ix++) {
-          const uint8_t v = f[(size_t)iy * L.nx + ix];
-          if (v & 1) cand.push_back(crf_rect_t{(int)std::lrint(ix * L.ystep * L.factor), (int)std::lrint(iy * L.ystep * L.factor), L.win_w, L.win_h});
-          if (v & 2) ix++;
+  if (int rc = detect_args(c, cas, &bgr, 1, rows, cols, step, scale_factor, cap, out)) return rc;
+  int total = 0;
+  const int rc = detect_frames(c, cas, &bgr, 1, rows, cols, step, scale_factor, min_neighbors, min_size, [&](int, int, std::vector<std::vector<crf_rect_t>>& boxes) -> int {
+    for (const crf_rect_t& r : boxes[0]) { if (total < cap) out[total] = r; total++; }
+    return CRF_OK;
+  });
+  return rc ? rc : total;
+}
+
+int crf_detect_faces_batch(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, double scale_factor,
+                           int min_neighbors, int min_size, crf_rect_t* out, int* image_of_box, int cap) {
+  if (int rc = detect_args(c, cas, images, n_images, rows, cols, step, scale_factor, cap, out)) return rc;
+  if (cap > 0 && !image_of_box) return fail(CRF_ERR_ARG, "bad argument");
+  int total = 0;
+  const int rc = detect_frames(c, cas, images, n_images, rows, cols, step, scale_factor, min_neighbors, min_size, [&](int f0, int nf, std::vector<std::vector<crf_rect_t>>& boxes) -> int {
+    for (int k = 0; k < nf; k++)
+      for (const crf_rect_t& r : boxes[(size_t)k]) {
+        if (total < cap) { out[total] = r; image_of_box[total] = f0 + k; }
+        total++;
+      }
+    return CRF_OK;
+  });
+  return rc ? rc : total;
+}
+
+int crf_analyze_images(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, double scale_factor,
+                       int min_neighbors, int min_size, crf_rect_t* boxes, int* image_of_box, crf_face_t* out, int cap) {
+  if (int rc = detect_args(c, cas, images, n_images, rows, cols, step, scale_factor, cap, boxes)) return rc;
+  if (cap > 0 && (!image_of_box || !out)) return fail(CRF_ERR_ARG, "bad argument");
+  if (!c->full_model) return fail(CRF_ERR_STATE, "analyzeFace needs the head-pose forest and the 5 pose forests; this context holds a single forest");
+  const size_t fb = (size_t)rows * step;
+  int total = 0;
+  const int rc = detect_frames(c, cas, images, n_images, rows, cols, step, scale_factor, min_neighbors, min_size, [&](int f0, int nf, std::vector<std::vector<crf_rect_t>>& det) -> int {
+    // FaceDescs point into the group's device frames: the analysis reads the copy made for detection
+    std::vector<FaceDesc> descs;
+    std::vector<int> slot;   // output index of descs[i]
+    int Hmax = 0;
+    for (int k = 0; k < nf; k++)
+      for (const crf_rect_t& r : det[(size_t)k]) {
+        if (total < cap) {
+          const crf_rect_t e = enlarge_detection(r, rows, cols);
+          boxes[total] = e; image_of_box[total] = f0 + k; out[total] = crf_face_t{};
+          if (box_error(rows, cols, e)) {
+            out[total].flags = CRF_FACE_NOT_ANALYSED;
+          } else {
+            FaceDesc d;
+            if (int rc2 = make_desc(c, rows, cols, step, (size_t)k * fb, e, d)) return rc2;
+            descs.push_back(d); slot.push_back(total);
+            Hmax = std::max(Hmax, d.H);
+          }
         }
-    }
-  } else {
-    CU(cudaStreamSynchronize(s));
-  }
-  group_rectangles(cand, min_neighbors, 0.2);
-  for (int i = 0; i < (int)cand.size() && i < cap; i++) out[i] = cand[(size_t)i];
-  return (int)cand.size();
+        total++;
+      }
+    if (descs.empty()) return CRF_OK;
+    int rc2;
+    if ((rc2 = c->d_faces.reserve(descs.size() * sizeof(crf_face_t)))) return rc2;
+    if ((rc2 = analyze_resident(c, descs, Hmax, c->d_haar_frames.as<uint8_t>(), c->d_faces.as<crf_face_t>(), false))) return rc2;
+    c->cnt.h2d_bytes += descs.size() * sizeof(FaceDesc);
+    std::vector<crf_face_t> rec(descs.size());
+    CU(cudaMemcpyAsync(rec.data(), c->d_faces.p, rec.size() * sizeof(crf_face_t), cudaMemcpyDeviceToHost, c->ws[0].stream));
+    CU(cudaStreamSynchronize(c->ws[0].stream));
+    c->cnt.d2h_bytes += rec.size() * sizeof(crf_face_t);
+    for (size_t i = 0; i < rec.size(); i++) out[slot[i]] = rec[i];
+    return CRF_OK;
+  });
+  return rc ? rc : total;
 }
 
 const char* crf_last_error(void) { return g_last_error.c_str(); }
@@ -1132,7 +1372,8 @@ void crf_ctx_destroy(crf_ctx* c) {
   if (c->tex_mp_wide) cudaDestroyTextureObject(c->tex_mp_wide);
   Buf* all[] = {&c->d_hp_slotsn, &c->d_mp_slotsn, &c->d_hp_nroot, &c->d_mp_nroot, &c->d_hp_slotsw, &c->d_mp_slotsw, &c->d_hp_slots16, &c->d_mp_slots16, &c->d_hp_slots, &c->d_hp_roots, &c->d_hp_m, &c->d_mp_slots, &c->d_mp_roots, &c->d_mp_mask, &c->d_mp_leaf, &c->d_xs, &c->d_coef[0], &c->d_coef[1],
                 &c->d_coef[2], &c->d_coef[3], &c->d_coef[4], &c->d_coef_sep[1], &c->d_coef_sep[2], &c->d_coef_sep[3], &c->d_coef_sep[4], &c->d_imgs[0], &c->d_imgs[1], &c->d_fd, &c->d_faces, &c->d_counters, &c->d_misc,
-                &c->d_haar_stages, &c->d_haar_weak, &c->d_haar_feats, &c->d_haar_level, &c->d_haar_S, &c->d_haar_Q, &c->d_haar_flags};
+                &c->d_haar_stages, &c->d_haar_weak, &c->d_haar_feats, &c->d_haar_frames, &c->d_haar_S, &c->d_haar_Q, &c->d_haar_flags, &c->d_haar_list[0],
+                &c->d_haar_list[1], &c->d_haar_rows, &c->d_haar_levels, &c->d_haar_counts, &c->d_haar_cand};
   for (Buf* b : all) b->release();
   for (auto& w : c->ws) {
     for (Buf* b : w.all) b->release();
@@ -1180,6 +1421,15 @@ int crf_ctx_create(const crf_model* m, int device, const crf_options_t* opt, crf
     if (const char* v = std::getenv("CRF_MS_MODE")) c->ms_mode = std::strcmp(v, "exact") == 0 ? CRF_MS_EXACT : CRF_MS_FAST;
   if (c->opt.ms_mode < CRF_MS_DEFAULT || c->opt.ms_mode > CRF_MS_FAST) return fail(CRF_ERR_ARG, "ms_mode must be CRF_MS_DEFAULT, CRF_MS_EXACT or CRF_MS_FAST");
   if (const char* v = std::getenv("CRF_STREAMS")) c->nstreams = std::strtol(v, nullptr, 0) == 2 ? 2 : 1;
+  if (const char* v = std::getenv("CRF_HAAR_SPLIT")) {
+    c->haar_split.clear();
+    for (char* e = nullptr;; v = e + 1) {
+      const long k = std::strtol(v, &e, 0);
+      if (e == v) break;
+      c->haar_split.push_back((int)k);
+      if (*e != ',') break;
+    }
+  }
   for (auto& w : c->ws) CU(cudaStreamCreateWithFlags(&w.stream, cudaStreamNonBlocking));
   CU(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   for (int i = 0; i < 2; i++) {
@@ -1388,49 +1638,7 @@ int crf_analyze_crops_device(crf_ctx* c, const uint8_t* d_bgr_batch, int n, int 
     if (rc) return rc;
     Hmax = std::max(Hmax, descs[i].H);
   }
-  int rc;
-  c->w = &c->ws[0];
-  cudaStream_t s0 = c->ws[0].stream;
-  if ((rc = c->d_fd.reserve((size_t)n * sizeof(FaceDesc)))) return rc;
-  CU(cudaMemcpyAsync(c->d_fd.p, descs.data(), (size_t)n * sizeof(FaceDesc), cudaMemcpyHostToDevice, s0));
-  CU(cudaMemsetAsync(d_out, 0, (size_t)n * sizeof(crf_face_t), s0));
-  const int chunk = pick_chunk(c, Hmax, headpose_only != 0);
-  Plan p; p.n = std::min(n, chunk); p.Hmax = Hmax; p.nplanes = c->layout.nplanes; p.need_gabor = c->layout.gabor_first >= 0; p.hp_stride = c->opt.hp_stride; p.ffd_stride = c->opt.ffd_stride; p.tree_cap = c->mp_ntrees_cfg;
-  p.need_ffd = !headpose_only;
-  const int nsets = n > chunk ? c->nstreams : 1;
-  for (int k = 0; k < nsets; k++) { c->w = &c->ws[k]; if ((rc = ensure(c, p))) return rc; }
-  CU(cudaStreamSynchronize(s0));
-  // consecutive chunks alternate between the two streams / work sets
-  int k = 0;
-  for (int f0 = 0; f0 < n; f0 += chunk, k++) {
-    const int m = std::min(chunk, n - f0);
-    c->w = &c->ws[k % nsets];
-    if ((rc = run_faces(c, c->d_fd.as<FaceDesc>() + f0, m, Hmax, d_bgr_batch, d_out + f0, headpose_only != 0, c->mp_ntrees_cfg, nullptr))) return rc;
-  }
-  for (int q = 0; q < nsets; q++) CU(cudaStreamSynchronize(c->ws[q].stream));
-  c->w = &c->ws[0];
-  if (!headpose_only) {
-    // faces whose composition or vote count exceeded the batched capacities: fetch the flags, re-run those faces wide
-    // (4 bytes come back, not the records: the flag is counted on the device)
-    int n_wide = 0;
-    CU(cudaMemsetAsync(c->d_misc.p, 0, 4, s0));
-    k_count_wide<<<(n + 255) / 256, 256, 0, s0>>>(d_out, n, c->d_misc.as<int>());
-    KCHECK(); count_launch(c, CRF_STAGE_MEANSHIFT);
-    CU(cudaMemcpyAsync(&n_wide, c->d_misc.p, 4, cudaMemcpyDeviceToHost, s0));
-    CU(cudaStreamSynchronize(s0));
-    if (n_wide > 0) {
-      std::vector<crf_face_t> tmp((size_t)n);
-      CU(cudaMemcpyAsync(tmp.data(), d_out, (size_t)n * sizeof(crf_face_t), cudaMemcpyDeviceToHost, s0));
-      CU(cudaStreamSynchronize(s0));
-      std::vector<int> wide;
-      for (int i = 0; i < n; i++) if (tmp[(size_t)i].flags & 6) wide.push_back(i);
-      if (!wide.empty() && (rc = rerun_wide(c, c->d_fd.as<FaceDesc>(), descs, d_bgr_batch, d_out, wide))) return rc;
-      CU(cudaStreamSynchronize(s0));
-    }
-  }
-  c->cnt.faces += n;
-  c->timer.collect();
-  return pull_counters(c);
+  return analyze_resident(c, descs, Hmax, d_bgr_batch, d_out, headpose_only != 0);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -5,10 +5,11 @@
 // The algorithm is OpenCV's (objdetect/cascadedetect.cpp; not under /root/reference): per scale factor = 1.3^k a bilinear
 // pyramid level of the gray frame, integral images of values and squares, then every window position of the level's
 // ystep grid walks the 22 stages / 2135 stumps until a stage sum falls below its threshold; surviving windows are grouped
-// by cv::groupRectangles.  Here: one thread per window position (adjacent threads = adjacent windows, so the corner
-// loads of a stump coalesce; the cascade tables are broadcast loads), early exit per thread, results as two byte maps
-// (passed all stages / rejected by stage 0 — the latter drives OpenCV's "skip one more step" scan rule, which is a
-// sequential dependence along x and is applied on the host together with the grouping, as OpenCV does it serially too).
+// by cv::groupRectangles.  Here a group of frames goes through each step in one launch: pyramid level + row scan, column
+// scan, the first stage group over every window (one thread per window position, adjacent threads = adjacent windows, so
+// the corner loads of a stump coalesce; the cascade tables are broadcast loads), later stage groups on compacted work lists
+// of the survivors, then OpenCV's "skip one more step after a stage-0 reject" scan rule and the candidate compaction on the
+// device.  Only the candidate rectangles come back; grouping (cv::groupRectangles) runs on the host, a frame per thread.
 // Arithmetic follows oracle/haar.py, which is pinned against cv2 4.13 on the shipped images (IoU of the boxes >= 0.9:
 // cv2 builds its pyramid with INTER_LINEAR_EXACT, this path with the INTER_LINEAR arithmetic of k_gray_resize).
 #pragma once
@@ -108,105 +109,275 @@ static int load_cascade(const std::string& path, Cascade& c, std::string& err) {
 }
 
 // ---- kernels ---------------------------------------------------------------------------------------------------------------
-// pyramid level: BGR2GRAY of the source pixels, then INTER_LINEAR (k_gray_resize's arithmetic) to sw x sh; u8 [sh][sw]
-__global__ void k_haar_level(const uint8_t* __restrict__ bgr, int rows, int cols, size_t step, uint8_t* __restrict__ out, int sh, int sw, double scale_x, double scale_y) {
-  const int dx = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y;
-  if (dx >= sw || dy >= sh) return;
-  int v;
-  if (sw == cols && sh == rows) {
-    v = gray_at(bgr, step, dy, dx);
-  } else {
-    float fx = (float)((dx + 0.5) * scale_x - 0.5);
-    int sx = (int)floorf(fx);
-    fx -= sx;
-    if (sx < 0) { fx = 0; sx = 0; }
-    if (sx >= cols - 1) { fx = 0; sx = cols - 1; }
-    const int a0 = __float2int_rn((1.f - fx) * 2048.f), a1 = __float2int_rn(fx * 2048.f);
-    float fy = (float)((dy + 0.5) * scale_y - 0.5);
-    int sy = (int)floorf(fy);
-    fy -= sy;
-    const int b0 = __float2int_rn((1.f - fy) * 2048.f), b1 = __float2int_rn(fy * 2048.f);
-    const int sy0 = min(max(sy, 0), rows - 1), sy1 = min(max(sy + 1, 0), rows - 1), sx1 = min(sx + 1, cols - 1);
-    const int row0 = gray_at(bgr, step, sy0, sx) * a0 + gray_at(bgr, step, sy0, sx1) * a1;
-    const int row1 = gray_at(bgr, step, sy1, sx) * a0 + gray_at(bgr, step, sy1, sx1) * a1;
-    v = (((b0 * (row0 >> 4)) >> 16) + ((b1 * (row1 >> 4)) >> 16) + 2) >> 2;
-    v = min(max(v, 0), 255);
-  }
-  out[(size_t)dy * sw + dx] = (uint8_t)v;
+// The frames of a group (equal size) are detected together; every buffer holds all frames of the group, level by level:
+//   S, Q   [level][frame][(sh + 1) x (sw + 1)] u32 integrals of values and squares (pitch sw + 1)
+//   flags  [level][frame][ny][nx] u8 per window of the level's ystep grid: bit 0 = passed every stage, bit 1 = rejected by stage 0
+//   rows   [frame][level][iy] candidates per window row, then their offsets within the frame
+// Launches per group: 3 per pyramid level, 1 per later stage group, 3 for the scan rule and the candidate compaction, whatever
+// the number of frames.
+struct HaarLevel {
+  double factor, scale_x, scale_y;
+  int sw, sh, nx, ny, ystep, win_w, win_h;
+  int row_off;                // first window row of the level among a frame's rows
+  size_t int_off, int_fs;     // S / Q of frame f at int_off + f * int_fs
+  size_t flag_off;            // flags of frame f at flag_off + f * nx * ny
+};
+
+struct HaarDev { const HaarStage* stages; const HaarWeak* weak; const HaarFeature* feats; int nstages, win_w, win_h; };
+
+// pyramid pixel: BGR2GRAY of the source pixels, then INTER_LINEAR (k_gray_resize's arithmetic) to sw x sh
+__device__ __forceinline__ int haar_level_px(const uint8_t* __restrict__ bgr, int rows, int cols, size_t step, const HaarLevel& L, int dx, int dy) {
+  if (L.sw == cols && L.sh == rows) return gray_at(bgr, step, dy, dx);
+  float fx = (float)((dx + 0.5) * L.scale_x - 0.5);
+  int sx = (int)floorf(fx);
+  fx -= sx;
+  if (sx < 0) { fx = 0; sx = 0; }
+  if (sx >= cols - 1) { fx = 0; sx = cols - 1; }
+  const int a0 = __float2int_rn((1.f - fx) * 2048.f), a1 = __float2int_rn(fx * 2048.f);
+  float fy = (float)((dy + 0.5) * L.scale_y - 0.5);
+  int sy = (int)floorf(fy);
+  fy -= sy;
+  const int b0 = __float2int_rn((1.f - fy) * 2048.f), b1 = __float2int_rn(fy * 2048.f);
+  const int sy0 = min(max(sy, 0), rows - 1), sy1 = min(max(sy + 1, 0), rows - 1), sx1 = min(sx + 1, cols - 1);
+  const int row0 = gray_at(bgr, step, sy0, sx) * a0 + gray_at(bgr, step, sy0, sx1) * a1;
+  const int row1 = gray_at(bgr, step, sy1, sx) * a0 + gray_at(bgr, step, sy1, sx1) * a1;
+  const int v = (((b0 * (row0 >> 4)) >> 16) + ((b1 * (row1 >> 4)) >> 16) + 2) >> 2;
+  return min(max(v, 0), 255);
 }
 
-// integral images of values (S) and squares (Q, modulo 2^32 as OpenCV keeps them), (sh + 1) x (sw + 1), pitch P = sw + 1.
-// Pass 1: one warp per row, inclusive scan along x.  Pass 2: one thread per column, running sum down the rows.
-__global__ void k_haar_rowscan(const uint8_t* __restrict__ img, int sh, int sw, uint32_t* __restrict__ S, uint32_t* __restrict__ Q) {
-  const int y = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (y >= sh) return;
-  const int P = sw + 1;
+// Pyramid level fused with the row pass of its integrals: one warp per level row builds the row's pixels and scans them along x.
+// grid (ceil(sh / 8), frames), 256 threads.
+__global__ void __launch_bounds__(256) k_haar_rows(const uint8_t* __restrict__ frames, size_t frame_bytes, int rows, int cols, size_t step, HaarLevel L,
+                                                   uint32_t* __restrict__ S, uint32_t* __restrict__ Q) {
+  const int y = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31, f = blockIdx.y;
+  if (y >= L.sh) return;
+  const uint8_t* __restrict__ bgr = frames + (size_t)f * frame_bytes;
+  const size_t P = (size_t)L.sw + 1;
+  uint32_t* __restrict__ s = S + L.int_off + (size_t)f * L.int_fs;
+  uint32_t* __restrict__ q = Q + L.int_off + (size_t)f * L.int_fs;
+  if (y == 0) for (size_t x = lane; x < P; x += 32) { s[x] = 0; q[x] = 0; }
+  if (lane == 0) { s[(size_t)(y + 1) * P] = 0; q[(size_t)(y + 1) * P] = 0; }
   uint32_t cs = 0, cq = 0;
-  if (lane == 0) { S[(size_t)(y + 1) * P] = 0; Q[(size_t)(y + 1) * P] = 0; }
-  for (int x0 = 0; x0 < sw; x0 += 32) {
+  for (int x0 = 0; x0 < L.sw; x0 += 32) {
     const int x = x0 + lane;
-    uint32_t v = x < sw ? img[(size_t)y * sw + x] : 0u, q = v * v;
+    uint32_t v = x < L.sw ? (uint32_t)haar_level_px(bgr, rows, cols, step, L, x, y) : 0u, sq = v * v;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t nv = __shfl_up_sync(0xffffffffu, v, o), nq = __shfl_up_sync(0xffffffffu, q, o);
-      if (lane >= o) { v += nv; q += nq; }
+      const uint32_t nv = __shfl_up_sync(0xffffffffu, v, o), nq = __shfl_up_sync(0xffffffffu, sq, o);
+      if (lane >= o) { v += nv; sq += nq; }
     }
-    if (x < sw) { S[(size_t)(y + 1) * P + x + 1] = cs + v; Q[(size_t)(y + 1) * P + x + 1] = cq + q; }
+    if (x < L.sw) { s[(size_t)(y + 1) * P + x + 1] = cs + v; q[(size_t)(y + 1) * P + x + 1] = cq + sq; }
     cs += __shfl_sync(0xffffffffu, v, 31);
-    cq += __shfl_sync(0xffffffffu, q, 31);
-  }
-}
-__global__ void k_haar_colscan(int sh, int sw, uint32_t* __restrict__ S, uint32_t* __restrict__ Q) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, P = sw + 1;
-  if (x > sw) return;
-  uint32_t s = 0, q = 0;
-  S[x] = 0; Q[x] = 0;
-  for (int y = 1; y <= sh; y++) {
-    s += S[(size_t)y * P + x]; q += Q[(size_t)y * P + x];
-    S[(size_t)y * P + x] = s; Q[(size_t)y * P + x] = q;
+    cq += __shfl_sync(0xffffffffu, sq, 31);
   }
 }
 
-// One thread per window of the level's ystep grid.  flags[iy][ix]: bit 0 = passed every stage, bit 1 = rejected by stage 0.
-__global__ void __launch_bounds__(128) k_haar_eval(const uint32_t* __restrict__ S, const uint32_t* __restrict__ Q, int sw, int sh, int win_w, int win_h, int ystep,
-                                                   int nx, int ny, const HaarStage* __restrict__ stages, int nstages, const HaarWeak* __restrict__ weak,
-                                                   const HaarFeature* __restrict__ feats, uint8_t* __restrict__ flags) {
-  const int ix = blockIdx.x * blockDim.x + threadIdx.x, iy = blockIdx.y;
-  if (ix >= nx || iy >= ny) return;
-  const int x = ix * ystep, y = iy * ystep, P = sw + 1;
-  const uint32_t* __restrict__ s0 = S + (size_t)y * P + x;
-  const uint32_t* __restrict__ q0 = Q + (size_t)y * P + x;
-  auto rs = [&](const uint32_t* __restrict__ p, int rx, int ry, int rw, int rh) -> uint32_t {
-    return p[(size_t)(ry + rh) * P + rx + rw] - p[(size_t)ry * P + rx + rw] - p[(size_t)(ry + rh) * P + rx] + p[(size_t)ry * P + rx];
-  };
-  // HaarEvaluator::setWindow: variance normalisation over the inner (w - 2) x (h - 2) rect
-  const double area = (double)((win_w - 2) * (win_h - 2));
-  const double vs = (double)rs(s0, 1, 1, win_w - 2, win_h - 2), vq = (double)rs(q0, 1, 1, win_w - 2, win_h - 2);
-  const double nf = area * vq - vs * vs;
-  uint8_t out = 0;
-  if (nf > 0.) {
-    const float inv = (float)(1.0 / sqrt(nf));
-    if ((float)area * inv < 0.1f) {
-      out = 1;
-      for (int si = 0; si < nstages; si++) {
-        const HaarStage st = stages[si];
-        float sum = 0.f;
-        for (int k = st.first; k < st.first + st.count; k++) {
-          const HaarWeak wk = weak[k];
-          const HaarFeature& f = feats[wk.feature];
-          float v = 0.f;
+// Column pass: a CTA owns 32 columns, its 32 warps 32 consecutive chunks of rows.  Each thread sums its chunk of one column, the chunk
+// totals of a column are scanned in shared memory, then every chunk is walked again with its carry.  S and Q are u32 sums modulo 2^32
+// (OpenCV keeps the square sums in 32 bits too) and integer addition is associative, so any summation order gives the bits of a serial
+// walk down the column.  grid (ceil((sw + 1) / 32), frames), block (32, 32).
+__global__ void __launch_bounds__(1024) k_haar_cols(HaarLevel L, uint32_t* __restrict__ S, uint32_t* __restrict__ Q) {
+  __shared__ uint32_t ts[32][32], tq[32][32];
+  const int tx = threadIdx.x, ty = threadIdx.y, x = blockIdx.x * 32 + tx, f = blockIdx.y;
+  const size_t P = (size_t)L.sw + 1;
+  const int R = (L.sh + 31) / 32, y0 = 1 + ty * R, y1 = min(L.sh + 1, y0 + R);
+  const bool col = x < (int)P;
+  uint32_t* __restrict__ s = S + L.int_off + (size_t)f * L.int_fs + x;
+  uint32_t* __restrict__ q = Q + L.int_off + (size_t)f * L.int_fs + x;
+  uint32_t as = 0, aq = 0;
+  if (col)
+    for (int y = y0; y < y1; y++) { as += s[(size_t)y * P]; aq += q[(size_t)y * P]; }
+  ts[ty][tx] = as; tq[ty][tx] = aq;
+  __syncthreads();
+  uint32_t cs = 0, cq = 0;
+  for (int k = 0; k < ty; k++) { cs += ts[k][tx]; cq += tq[k][tx]; }
+  if (col)
+    for (int y = y0; y < y1; y++) {
+      cs += s[(size_t)y * P]; cq += q[(size_t)y * P];
+      s[(size_t)y * P] = cs; q[(size_t)y * P] = cq;
+    }
+}
+
+__device__ __forceinline__ uint32_t haar_rectsum(const uint32_t* __restrict__ p, size_t P, int rx, int ry, int rw, int rh) {
+  return p[(size_t)(ry + rh) * P + rx + rw] - p[(size_t)ry * P + rx + rw] - p[(size_t)(ry + rh) * P + rx] + p[(size_t)ry * P + rx];
+}
+
+// Stages [s_begin, s_end) of the window at s0, one thread per window, in the cascade's order: v = v + weight * rectsum over the feature's
+// rects, sum = sum + leaf over the stumps (f32, unfused under -fmad=false).  A window's sums are never split across lanes: a reordered
+// f32 sum could flip a stump or a stage near its threshold.  Returns the first stage whose sum falls below its threshold, or -1.
+__device__ __forceinline__ int haar_stages(const uint32_t* __restrict__ s0, size_t P, float inv, const HaarDev& K, int s_begin, int s_end) {
+  for (int si = s_begin; si < s_end; si++) {
+    const HaarStage st = K.stages[si];
+    float sum = 0.f;
+    for (int k = st.first; k < st.first + st.count; k++) {
+      const HaarWeak wk = K.weak[k];
+      const HaarFeature& f = K.feats[wk.feature];
+      float v = 0.f;
 #pragma unroll
-          for (int r = 0; r < 3; r++) {
-            const HaarRect hr = f.r[r];
-            if (hr.weight != 0.f) v = v + hr.weight * (float)rs(s0, hr.x, hr.y, hr.w, hr.h);
-          }
-          sum = sum + ((v * inv < wk.threshold) ? wk.left : wk.right);
-        }
-        if (!(sum >= st.threshold)) { out = si == 0 ? 2 : 0; break; }
+      for (int r = 0; r < 3; r++) {
+        const HaarRect hr = f.r[r];
+        if (hr.weight != 0.f) v = v + hr.weight * (float)haar_rectsum(s0, P, hr.x, hr.y, hr.w, hr.h);
+      }
+      sum = sum + ((v * inv < wk.threshold) ? wk.left : wk.right);
+    }
+    if (!(sum >= st.threshold)) return si;
+  }
+  return -1;
+}
+
+// warp-aggregated append of the lanes' items to a work list (every lane of the warp calls it)
+__device__ __forceinline__ void haar_append(bool keep, uint2 item, uint2* __restrict__ list, unsigned* __restrict__ count) {
+  const unsigned m = __ballot_sync(0xffffffffu, keep);
+  if (!m) return;
+  const int lane = threadIdx.x & 31, leader = __ffs(m) - 1;
+  unsigned base = 0;
+  if (lane == leader) base = atomicAdd(count, (unsigned)__popc(m));
+  base = __shfl_sync(0xffffffffu, base, leader);
+  if (keep) list[base + __popc(m & ((1u << lane) - 1u))] = item;
+}
+
+// First stage group, every window of one level of every frame of the group: HaarEvaluator::setWindow's variance normalisation over the
+// inner (w - 2) x (h - 2) rect, stages [0, s_end); writes the window's flag byte and appends the survivors (flag index, 1 / nf) to the
+// work list of the next stage group.  grid (ceil(nx / 128), ny, frames), 128 threads.
+__global__ void __launch_bounds__(128) k_haar_eval_first(HaarLevel L, const uint32_t* __restrict__ S, const uint32_t* __restrict__ Q, HaarDev K, int s_end,
+                                                         uint8_t* __restrict__ flags, uint2* __restrict__ list, unsigned* __restrict__ count) {
+  const int ix = blockIdx.x * blockDim.x + threadIdx.x, iy = blockIdx.y, f = blockIdx.z;
+  bool keep = false;
+  uint2 item = make_uint2(0u, 0u);
+  if (ix < L.nx) {
+    const size_t P = (size_t)L.sw + 1;
+    const size_t o = L.int_off + (size_t)f * L.int_fs + (size_t)(iy * L.ystep) * P + (size_t)ix * L.ystep;
+    const uint32_t* __restrict__ s0 = S + o;
+    const uint32_t* __restrict__ q0 = Q + o;
+    const double area = (double)((K.win_w - 2) * (K.win_h - 2));
+    const double vs = (double)haar_rectsum(s0, P, 1, 1, K.win_w - 2, K.win_h - 2), vq = (double)haar_rectsum(q0, P, 1, 1, K.win_w - 2, K.win_h - 2);
+    const double nf = area * vq - vs * vs;
+    uint8_t out = 0;
+    float inv = 0.f;
+    if (nf > 0.) {
+      inv = (float)(1.0 / sqrt(nf));
+      if ((float)area * inv < 0.1f) {
+        const int r = haar_stages(s0, P, inv, K, 0, s_end);
+        if (r < 0) { if (s_end >= K.nstages) out = 1; else keep = true; }
+        else if (r == 0) out = 2;
       }
     }
+    const size_t idx = L.flag_off + (size_t)f * L.nx * L.ny + (size_t)iy * L.nx + ix;
+    flags[idx] = out;
+    item = make_uint2((unsigned)idx, __float_as_uint(inv));
   }
-  flags[(size_t)iy * nx + ix] = out;
+  haar_append(keep, item, list, count);
+}
+
+// index of the last level whose field is <= v (the level tables are sorted by every offset)
+template <class T, class G>
+__device__ __forceinline__ int haar_level_of(const HaarLevel* __restrict__ levels, int nlevels, T v, G field) {
+  int lo = 0, hi = nlevels - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (field(levels[mid]) <= v) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// A later stage group [s_begin, s_end) on the previous group's survivors, grid-stride over the list (its length is on the device, so the
+// launch does not wait for the host).  Compaction changes which thread handles a window, never the order of its arithmetic.  Survivors of
+// the last group get bit 0 of their flag; the others are appended to the next list.
+__global__ void __launch_bounds__(128) k_haar_eval_list(const HaarLevel* __restrict__ levels, int nlevels, const uint32_t* __restrict__ S, HaarDev K,
+                                                        int s_begin, int s_end, const uint2* __restrict__ list_in, const unsigned* __restrict__ count_in,
+                                                        uint8_t* __restrict__ flags, uint2* __restrict__ list_out, unsigned* __restrict__ count_out) {
+  const unsigned n = *count_in;
+  const bool last = s_end >= K.nstages;
+  for (unsigned base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
+    const unsigned i = base + threadIdx.x;
+    bool keep = false;
+    uint2 it = make_uint2(0u, 0u);
+    if (i < n) {
+      it = list_in[i];
+      const HaarLevel& L = levels[haar_level_of(levels, nlevels, (size_t)it.x, [](const HaarLevel& l) { return l.flag_off; })];
+      const size_t r = it.x - L.flag_off, nxy = (size_t)L.nx * L.ny, f = r / nxy, w = r - f * nxy;
+      const int iy = (int)(w / L.nx), ix = (int)(w - (size_t)iy * L.nx);
+      const size_t P = (size_t)L.sw + 1;
+      const uint32_t* __restrict__ s0 = S + L.int_off + f * L.int_fs + (size_t)(iy * L.ystep) * P + (size_t)ix * L.ystep;
+      if (haar_stages(s0, P, __uint_as_float(it.y), K, s_begin, s_end) < 0) {
+        if (last) flags[it.x] = 1; else keep = true;
+      }
+    }
+    if (!last) haar_append(keep, it, list_out, count_out);
+  }
+}
+
+// OpenCV's scan (CascadeClassifierInvoker) visits the windows of a row in x order and takes one extra step after a window rejected by
+// stage 0: visited(0) = 1, visited(ix) = !(visited(ix - 1) && rej0(ix - 1)).  32 windows at a time from the ballot of their rej0 bits.
+__device__ __forceinline__ unsigned haar_visited(unsigned rej0, bool& carry) {
+  unsigned vis = 0;
+  bool v = carry;
+#pragma unroll
+  for (int b = 0; b < 32; b++) {
+    if (v) vis |= 1u << b;
+    v = !(v && ((rej0 >> b) & 1u));
+  }
+  carry = v;
+  return vis;
+}
+
+// One warp per window row (frame-major, then level, then iy): candidates = visited windows that passed every stage.  COUNT: the row's
+// candidate count into rows[].  Otherwise: the candidate rectangles, in (level, iy, ix) order per frame and frame after frame, at the
+// row's offset (rows[] after k_haar_row_offsets) plus the counts of the frames before.  grid ceil(frames * rows_pf / 8), 256 threads.
+template <bool COUNT>
+__global__ void __launch_bounds__(256) k_haar_scan(const HaarLevel* __restrict__ levels, int nlevels, int nrows, int rows_pf, const uint8_t* __restrict__ flags,
+                                                   int* __restrict__ rows, const int* __restrict__ frame_count, crf_rect_t* __restrict__ cand) {
+  const int rid = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (rid >= nrows) return;
+  const int f = rid / rows_pf, rr = rid - f * rows_pf;
+  const HaarLevel& L = levels[haar_level_of(levels, nlevels, rr, [](const HaarLevel& l) { return l.row_off; })];
+  const int iy = rr - L.row_off;
+  const uint8_t* __restrict__ fl = flags + L.flag_off + (size_t)f * L.nx * L.ny + (size_t)iy * L.nx;
+  int base = 0;
+  if (!COUNT) {
+    base = rows[rid];
+    for (int k = 0; k < f; k++) base += frame_count[k];
+  }
+  bool carry = true;
+  int n = 0;
+  for (int x0 = 0; x0 < L.nx; x0 += 32) {
+    const int ix = x0 + lane;
+    const uint8_t v = ix < L.nx ? fl[ix] : 0;
+    const unsigned rej0 = __ballot_sync(0xffffffffu, v & 2), pass = __ballot_sync(0xffffffffu, v & 1);
+    const unsigned c = haar_visited(rej0, carry) & pass;
+    if (!COUNT && ((c >> lane) & 1u))
+      cand[base + n + __popc(c & ((1u << lane) - 1u))] = crf_rect_t{(int)rint(ix * L.ystep * L.factor), (int)rint(iy * L.ystep * L.factor), L.win_w, L.win_h};
+    n += __popc(c);
+  }
+  if (COUNT && lane == 0) rows[rid] = n;
+}
+
+// Exclusive scan of one frame's row counts in place (row offsets within the frame) and the frame's candidate count.  grid frames, 1024 threads.
+__global__ void __launch_bounds__(1024) k_haar_row_offsets(int rows_pf, int* __restrict__ rows, int* __restrict__ frame_count) {
+  __shared__ int wsum[32];
+  int* __restrict__ r = rows + (size_t)blockIdx.x * rows_pf;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int carry = 0;
+  for (int b = 0; b < rows_pf; b += 1024) {
+    const int i = b + threadIdx.x;
+    const int v = i < rows_pf ? r[i] : 0;
+    int x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
+    if (lane == 31) wsum[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+      int t = wsum[lane];
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, t, o); if (lane >= o) t += y; }
+      wsum[lane] = t;
+    }
+    __syncthreads();
+    if (i < rows_pf) r[i] = carry + (warp ? wsum[warp - 1] : 0) + x - v;
+    carry += wsum[31];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) frame_count[blockIdx.x] = carry;
 }
 
 // ---- host: scales, scan rule, cv::groupRectangles ----------------------------------------------------------------------------

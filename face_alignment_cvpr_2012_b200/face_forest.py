@@ -468,6 +468,35 @@ class CascadeClassifier:
             capi.check(n)
         return [(r.x, r.y, r.width, r.height) for r in out[: min(n, cap)]]
 
+    def _frames(self, frames):
+        frames = [np.ascontiguousarray(f, np.uint8) for f in frames]
+        if frames and any(f.shape != frames[0].shape for f in frames):
+            raise ValueError("frames of one call must have equal sizes")
+        return frames, (C.c_void_p * max(len(frames), 1))(*[f.ctypes.data for f in frames])
+
+    def detectMultiScaleBatch(self, ctx: "Context", frames, scaleFactor: float = 1.1, minNeighbors: int = 3, minSize=(0, 0)) -> list:
+        """detectMultiScale on every frame of `frames` (equal-size BGR frames: a list or an [n, rows, cols, 3] array) in one call
+        (crf_detect_faces_batch): one list of (x, y, w, h) per frame, each equal to detectMultiScale on that frame."""
+        frames, ptrs = self._frames(frames)
+        if not frames:
+            return []
+        rows, cols = frames[0].shape[:2]
+        L = capi.lib()
+        args = (ctx.h, self.h, ptrs, len(frames), rows, cols, cols * 3, float(scaleFactor), int(minNeighbors), int(max(minSize)))
+        cap = 64 * len(frames)
+        while True:
+            out, iob = (Rect * cap)(), np.zeros(cap, np.int32)
+            n = L.crf_detect_faces_batch(*args, out, capi.ptr(iob, C.c_int32), cap)
+            if n < 0:
+                capi.check(n)
+            if n <= cap:
+                break
+            cap = n
+        per = [[] for _ in frames]
+        for r, i in zip(out[:n], iob[:n]):
+            per[i].append((r.x, r.y, r.width, r.height))
+        return per
+
 
 class MultiContext:
     """Several GPUs behind one caller (crf_multi_*): one context and one host thread per GPU inside the library, contiguous
@@ -580,6 +609,38 @@ class FaceForest:
         if faces is not None:
             faces.clear(); faces.extend(out)
         return out
+
+    def analyzeImages(self, frames) -> list:
+        """analyzeImage(img) with the Haar cascade of fd_option for every frame of `frames` (equal-size BGR frames) in one call
+        (crf_analyze_images): the frames cross PCIe once, for detection and analysis.  One list of Face per frame, in
+        detectMultiScale's order.  A detection whose enlarged box the analysis path cannot take (a face cut by the bottom border) comes
+        back with a zero record whose flags carry capi.FACE_NOT_ANALYSED, where analyzeImage would raise."""
+        if not self.is_inizialized:
+            raise AssertionError("CV_Assert(is_inizialized)")
+        if self.m_face_cascade is None:
+            raise AssertionError("no face cascade loaded: set fd_option.path_face_cascade")
+        fd = self.option.fd_option
+        frames, ptrs = self.m_face_cascade._frames(frames)
+        if not frames:
+            return []
+        rows, cols = frames[0].shape[:2]
+        L = capi.lib()
+        args = (self.ctx.h, self.m_face_cascade.h, ptrs, len(frames), rows, cols, cols * 3, float(fd.search_scale_factor), int(fd.min_neighbors),
+                int(fd.min_feature_size))
+        cap = 64 * len(frames)
+        while True:   # a second call only when the frames hold more than 64 faces each on average
+            boxes, iob, recs = (Rect * cap)(), np.zeros(cap, np.int32), np.zeros(cap, FACE_DTYPE)
+            n = L.crf_analyze_images(*args, boxes, capi.ptr(iob, C.c_int32), recs.ctypes.data, cap)
+            if n < 0:
+                capi.check(n)
+            if n <= cap:
+                break
+            cap = n
+        per = [[] for _ in frames]
+        for k in range(n):
+            b = boxes[k]
+            per[iob[k]].extend(self._to_faces(recs[k:k + 1], [(b.x, b.y, b.width, b.height)]))
+        return per
 
 
 class MeanShift:

@@ -86,8 +86,12 @@ typedef struct {
   int   ms_iters[CRF_NUM_PARTS];     /* MeanShift iterations executed */
   int   n_votes[CRF_NUM_PARTS];      /* votes per part (src/face_utils.cpp:289-298) */
   int   flags;                       /* bit0: composition clamped (reference would index out of bounds); bits 1-2 are internal
-                                        (face re-run with worst-case capacities) and never set in returned records */
+                                        (face re-run with worst-case capacities) and never set in returned records;
+                                        bit3: CRF_FACE_NOT_ANALYSED (crf_analyze_images only) */
 } crf_face_t;
+
+/* crf_face_t::flags of a detected box that the analysis path cannot take (record otherwise zero) */
+#define CRF_FACE_NOT_ANALYSED 8
 
 typedef struct {
   int hp_trees, hp_nodes, hp_leaves, hp_max_depth;
@@ -191,6 +195,25 @@ void crf_cascade_free(crf_cascade* c);
 int crf_cascade_info(const crf_cascade* c, int* win_w, int* win_h, int* nstages, int* nweak);
 int crf_detect_faces(crf_ctx* ctx, const crf_cascade* c, const uint8_t* bgr, int rows, int cols, size_t step, double scale_factor,
                      int min_neighbors, int min_size, crf_rect_t* out, int cap);
+/* detectMultiScale on n_images equal-size frames in one call.  Boxes are grouped by frame in frame order; within a frame they are
+ * exactly what crf_detect_faces returns for that frame, in the same order.  image_of_box[i] = frame of box i.
+ * Each frame crosses PCIe once.  Frames are processed in groups of at most 64 (fewer when half the context's work budget, min(64 GB,
+ * half the free memory), cannot hold 64); each pyramid level, cascade stage group and scan step of a group is one launch.
+ * cap smaller than the box count: every frame is still searched, the true count is returned and the first `cap` boxes are written
+ * (cap = 0 sizes a buffer).  Returns the total box count or a negative status. */
+int crf_detect_faces_batch(crf_ctx* ctx, const crf_cascade* c, const uint8_t* const* images, int n_images, int rows, int cols,
+                           size_t step, double scale_factor, int min_neighbors, int min_size,
+                           crf_rect_t* out, int* image_of_box, int cap);
+/* FaceForest::analyzeImage(img, faces) for n_images frames: detection as above, detectFace's enlargement + clipping
+ * (src/FaceForest.cpp:147-157), then analyzeFace for every box, reading the frames from the device copy made for detection (no second
+ * upload).  boxes (the enlarged boxes) / image_of_box / out: cap entries, in the order of crf_detect_faces_batch.
+ * Unlike crf_analyze_faces, a box the analysis path rejects (typically a detection at the bottom border whose clipped box scales to a face
+ * shorter than a 31-px patch) does not fail the call: its record is zero except flags = CRF_FACE_NOT_ANALYSED, and every other face is
+ * analysed normally.  cap smaller than the face count: everything is detected, the true count is returned, and only the first `cap`
+ * boxes are written and analysed.  Returns the face count or a negative status. */
+int crf_analyze_images(crf_ctx* ctx, const crf_cascade* c, const uint8_t* const* images, int n_images, int rows, int cols,
+                       size_t step, double scale_factor, int min_neighbors, int min_size,
+                       crf_rect_t* boxes, int* image_of_box, crf_face_t* out, int cap);
 
 /* ---- several GPUs behind one caller (SURVEY 8e): one context + one host thread per GPU, contiguous shards of the faces (cut at frame
  * boundaries when the boxes are grouped by frame), a forest replica per GPU, records written straight into `out`.  No collective:
