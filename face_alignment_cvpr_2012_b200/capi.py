@@ -33,6 +33,16 @@ class Rect(C.Structure):
     _fields_ = [("x", C.c_int), ("y", C.c_int), ("width", C.c_int), ("height", C.c_int)]
 
 
+class Image(C.Structure):
+    """crf_image_t: one BGR frame of any size (rows x cols pixels, step bytes per row)."""
+    _fields_ = [("bgr", C.c_void_p), ("rows", C.c_int), ("cols", C.c_int), ("step", C.c_size_t)]
+
+
+def images(frames) -> "C.Array":
+    """crf_image_t descriptors of C-contiguous [rows, cols, 3] u8 frames (at least one element, so an empty list still passes a pointer)."""
+    return (Image * max(len(frames), 1))(*[Image(f.ctypes.data, f.shape[0], f.shape[1], f.strides[0]) for f in frames])
+
+
 class Options(C.Structure):
     _fields_ = [("hp_stride", C.c_int), ("hp_min_foreground", C.c_float), ("ffd_stride", C.c_int), ("ffd_min_samples", C.c_int),
                 ("ffd_min_foreground", C.c_float), ("ffd_min_pf", C.c_float), ("ffd_max_variance", C.c_float),
@@ -69,6 +79,7 @@ EXPORTS = [
     "crf_stage_eval_patches", "crf_stage_eval_tests", "crf_stage_eval_tests_sum", "crf_model_load_tree", "crf_stage_meanshift_opt", "crf_stage_area_under_curve",
     "crf_cascade_load", "crf_cascade_free", "crf_cascade_info", "crf_detect_faces", "crf_detect_faces_batch", "crf_analyze_images",
     "crf_multi_create", "crf_multi_destroy", "crf_multi_device_count", "crf_multi_ctx", "crf_multi_analyze_batch", "crf_multi_analyze_crops",
+    "crf_analyze_batch_mixed", "crf_detect_faces_batch_mixed", "crf_analyze_images_mixed", "crf_multi_analyze_batch_mixed",
 ]
 
 _lib = None
@@ -119,6 +130,7 @@ def lib() -> C.CDLL:
     L.crf_host_free.restype = None
     L.crf_analyze_faces.argtypes = [vp, vp, C.c_int, C.c_int, C.c_size_t, C.POINTER(Rect), C.c_int, vp]
     L.crf_analyze_batch.argtypes = [vp, C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_size_t, C.POINTER(Rect), i32p, C.c_int, vp]
+    L.crf_analyze_batch_mixed.argtypes = [vp, C.POINTER(Image), C.c_int, C.POINTER(Rect), i32p, C.c_int, vp]
     L.crf_analyze_crops.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, vp]
     L.crf_headpose_crops.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, vp]
     L.crf_analyze_crops_device.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, vp, C.c_int]
@@ -153,6 +165,8 @@ def lib() -> C.CDLL:
                                          C.POINTER(Rect), i32p, C.c_int]
     L.crf_analyze_images.argtypes = [vp, vp, C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_double, C.c_int, C.c_int,
                                      C.POINTER(Rect), i32p, vp, C.c_int]
+    L.crf_detect_faces_batch_mixed.argtypes = [vp, vp, C.POINTER(Image), C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(Rect), i32p, C.c_int]
+    L.crf_analyze_images_mixed.argtypes = [vp, vp, C.POINTER(Image), C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(Rect), i32p, vp, C.c_int]
     L.crf_multi_create.argtypes = [vp, i32p, C.c_int, C.POINTER(Options), C.POINTER(vp)]
     L.crf_multi_destroy.argtypes = [vp]
     L.crf_multi_destroy.restype = None
@@ -160,6 +174,7 @@ def lib() -> C.CDLL:
     L.crf_multi_ctx.argtypes = [vp, C.c_int]
     L.crf_multi_ctx.restype = vp
     L.crf_multi_analyze_batch.argtypes = [vp, C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_size_t, C.POINTER(Rect), i32p, C.c_int, vp]
+    L.crf_multi_analyze_batch_mixed.argtypes = [vp, C.POINTER(Image), C.c_int, C.POINTER(Rect), i32p, C.c_int, vp]
     L.crf_multi_analyze_crops.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, vp, C.c_int]
     _lib = L
     return L

@@ -2,6 +2,7 @@
 // Orchestrates what FaceForest::analyzeFace does for one face (reference src/FaceForest.cpp:183-258),
 // for whole batches of faces at a time.  There is no CPU fallback: every stage is a CUDA kernel.
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -197,7 +198,7 @@ struct crf_ctx {
   size_t work_budget = (size_t)64 << 30;  // bytes of work buffers a launch may use (min(64 GB, half of the free memory at creation))
   StageTimer timer;
   // face-box source (haar.cuh): device image of the last cascade used + the buffers of a group of frames
-  const struct crf_cascade* haar_cached = nullptr;
+  unsigned long long haar_cached = 0;   // crf_cascade::id of the cascade in d_haar_stages / weak / feats (0 = none)
   Buf d_haar_stages, d_haar_weak, d_haar_feats, d_haar_frames, d_haar_S, d_haar_Q, d_haar_flags, d_haar_list[2], d_haar_rows, d_haar_levels, d_haar_counts, d_haar_cand;
   // first stage of each cascade stage group after the first (CRF_HAAR_SPLIT="a,b,..."; measured, DESIGN §4.5)
   std::vector<int> haar_split{3, 8};
@@ -621,21 +622,56 @@ static int rerun_wide(crf_ctx* c, const FaceDesc* d_fd_all, const std::vector<Fa
   return CRF_OK;
 }
 
-// Host-resident inputs.  image(i) = pointer to frame i; faces are processed in chunks, frames of a chunk
-// are copied on a second stream into one of two device buffers so the copy of chunk k+1 overlaps chunk k.
-static int analyze_host(crf_ctx* c, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, const crf_rect_t* boxes,
-                        const int* image_of_box, int n, crf_face_t* out, bool headpose_only) {
+static size_t image_bytes(const crf_image_t& im) { return (size_t)im.rows * im.step; }
+
+static bool bad_geometry(const crf_image_t& im) { return im.rows < 1 || im.cols < 1 || im.step < (size_t)im.cols * 3; }
+
+// The descriptor rule of the _mixed calls: every frame has pixels, rows, cols >= 1 and step >= cols * 3.
+static int image_args(const crf_image_t* images, int n_images) {
+  for (int i = 0; i < n_images; i++) {
+    if (!images[i].bgr) return fail(CRF_ERR_ARG, "null frame");
+    if (bad_geometry(images[i])) return fail(CRF_ERR_ARG, "bad frame descriptor (rows, cols >= 1, step >= cols * 3)");
+  }
+  return CRF_OK;
+}
+
+// The checks a boxes-given call makes before any work: each box names a frame in range with pixels and fits that frame's analysis path.
+// (A null frame that no box names is accepted here: the equal-size calls always did.)
+static int box_args(const crf_image_t* images, int n_images, const crf_rect_t* boxes, const int* image_of_box, int n) {
+  for (int k = 0; k < n_images; k++)
+    if (bad_geometry(images[k])) return fail(CRF_ERR_ARG, "bad frame descriptor (rows, cols >= 1, step >= cols * 3)");
+  for (int i = 0; i < n; i++) {
+    const int im = image_of_box ? image_of_box[i] : i;
+    if (im < 0 || im >= n_images || !images[im].bgr) return fail(CRF_ERR_ARG, "image index out of range");
+    if (const char* e = box_error(images[im].rows, images[im].cols, boxes[i])) return fail(CRF_ERR_ARG, e);
+  }
+  return CRF_OK;
+}
+
+// n_images descriptors of equal-size frames: what the calls that take one (rows, cols, step) pass to the generalised core.  NULL when
+// images is (the core reports it).
+static const crf_image_t* same_size(const uint8_t* const* images, int n_images, int rows, int cols, size_t step, std::vector<crf_image_t>& v) {
+  if (!images) return nullptr;
+  v.resize((size_t)std::max(n_images, 0));
+  for (int i = 0; i < n_images; i++) v[(size_t)i] = crf_image_t{images[i], rows, cols, step};
+  return v.data();
+}
+
+// Host-resident inputs.  images[k] describes frame k; faces are processed in chunks, frames of a chunk are copied on a second stream
+// into one of two device buffers so the copy of chunk k+1 overlaps chunk k.
+static int analyze_host(crf_ctx* c, const crf_image_t* images, int n_images, const crf_rect_t* boxes, const int* image_of_box, int n,
+                        crf_face_t* out, bool headpose_only) {
   if (!c) return fail(CRF_ERR_STATE, "context is not initialised");
   if (!c->full_model) return fail(CRF_ERR_STATE, "analyzeFace needs the head-pose forest and the 5 pose forests; this context holds a single forest");
   if (n < 0 || (n > 0 && (!images || !boxes || !out))) return fail(CRF_ERR_ARG, "null argument");
   if (n == 0) return CRF_OK;
-  if (step < (size_t)cols * 3) return fail(CRF_ERR_ARG, "step smaller than a row");
+  if (int rc = box_args(images, n_images, boxes, image_of_box, n)) return rc;
   CU(cudaSetDevice(c->device));
-  const size_t img_bytes = (size_t)rows * step;
   std::vector<FaceDesc> descs((size_t)n);
   int Hmax_first = 0;
   for (int i = 0; i < n; i++) {
-    int rc = make_desc(c, rows, cols, step, 0, boxes[i], descs[i]);
+    const crf_image_t& im = images[image_of_box ? image_of_box[i] : i];
+    int rc = make_desc(c, im.rows, im.cols, im.step, 0, boxes[i], descs[i]);
     if (rc) return rc;
     Hmax_first = std::max(Hmax_first, descs[i].H);
   }
@@ -653,20 +689,16 @@ static int analyze_host(crf_ctx* c, const uint8_t* const* images, int n_images, 
   // when the boxes cover well under the frames' area (a few faces in a 1080p / 4K frame), only the box pixels travel — packed
   // row by row into a pinned staging buffer on the host while the GPU works on the previous chunk, then one H2D copy.
   // Pageable sources always go through the staging buffer (a threaded pack + pinned H2D beats the driver's pageable copy).
-  for (int i = 0; i < n; i++) {
-    const int im = image_of_box ? image_of_box[i] : i;
-    if (im < 0 || im >= n_images || !images[im]) return fail(CRF_ERR_ARG, "image index out of range");
-  }
   // a batch is treated as pinned only if every frame it names is (one pageable frame sends the whole batch through the packed path)
   bool src_pinned = true;
   {
     int last = -1;
     for (int i = 0; i < n && src_pinned; i++) {
       const int im = image_of_box ? image_of_box[i] : i;
-      if (im != last) { src_pinned = is_pinned_host(images[im]); last = im; }
+      if (im != last) { src_pinned = is_pinned_host(images[im].bgr); last = im; }
     }
   }
-  struct Chunk { int f0, f1, Hmax; bool roi; size_t bytes; std::vector<int> frames; };
+  struct Chunk { int f0, f1, Hmax; bool roi; size_t bytes; std::vector<int> frames; std::vector<size_t> slot_off; };
   std::vector<Chunk> chunks;
   std::vector<crf_rect_t> src_box((size_t)n);   // where the pixels are in the caller's frame (ROI mode rewrites the descriptor)
   for (int f0 = 0; f0 < n; f0 += chunk) {
@@ -675,17 +707,17 @@ static int analyze_host(crf_ctx* c, const uint8_t* const* images, int n_images, 
     size_t roi_bytes = 0;
     for (int i = f0; i < ch.f1; i++) {
       const int im = image_of_box ? image_of_box[i] : i;
-      if (im < 0 || im >= n_images) return fail(CRF_ERR_ARG, "image index out of range");
       auto it = slot_of.find(im);
       int slot;
-      if (it == slot_of.end()) { slot = (int)ch.frames.size(); ch.frames.push_back(im); slot_of.emplace(im, slot); }
-      else slot = it->second;
-      descs[i].img_off = (size_t)slot * img_bytes;
+      if (it == slot_of.end()) {   // frame-mode slots: the chunk's distinct frames back to back
+        slot = (int)ch.frames.size(); ch.frames.push_back(im); slot_of.emplace(im, slot);
+        ch.slot_off.push_back(ch.bytes); ch.bytes += image_bytes(images[im]);
+      } else slot = it->second;
+      descs[i].img_off = ch.slot_off[(size_t)slot];
       src_box[i] = boxes[i];
       roi_bytes += ((size_t)boxes[i].width * boxes[i].height * 3 + 15) & ~(size_t)15;
       ch.Hmax = std::max(ch.Hmax, descs[i].H);
     }
-    ch.bytes = ch.frames.size() * img_bytes;
     if (roi_bytes * 10 < ch.bytes * 6 || (!src_pinned && roi_bytes <= ch.bytes + ch.bytes / 4)) {
       ch.roi = true; ch.bytes = roi_bytes;
       size_t off = 0;
@@ -732,7 +764,9 @@ static int analyze_host(crf_ctx* c, const uint8_t* const* images, int n_images, 
       parallel_for(ch.f1 - ch.f0, ch.bytes, [&](int k2) {
         const int i = ch.f0 + k2;
         const crf_rect_t& bx = src_box[i];
-        const uint8_t* src = images[image_of_box ? image_of_box[i] : i] + (size_t)bx.y * step + (size_t)bx.x * 3;
+        const crf_image_t& im = images[image_of_box ? image_of_box[i] : i];
+        const size_t step = im.step;
+        const uint8_t* src = im.bgr + (size_t)bx.y * step + (size_t)bx.x * 3;
         uint8_t* dst = st + descs[i].img_off;
         const size_t rowb = (size_t)bx.width * 3;
         if (rowb == step) std::memcpy(dst, src, rowb * bx.height);
@@ -747,11 +781,12 @@ static int analyze_host(crf_ctx* c, const uint8_t* const* images, int n_images, 
     size_t i = 0;
     while (i < ch.frames.size()) {
       size_t j = i + 1;
-      while (j < ch.frames.size() && images[ch.frames[j]] == images[ch.frames[j - 1]] + img_bytes) j++;
-      CU(cudaMemcpyAsync(c->d_imgs[b].as<uint8_t>() + i * img_bytes, images[ch.frames[i]], (j - i) * img_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+      while (j < ch.frames.size() && images[ch.frames[j]].bgr == images[ch.frames[j - 1]].bgr + image_bytes(images[ch.frames[j - 1]])) j++;
+      const size_t end = j < ch.frames.size() ? ch.slot_off[j] : ch.bytes;
+      CU(cudaMemcpyAsync(c->d_imgs[b].as<uint8_t>() + ch.slot_off[i], images[ch.frames[i]].bgr, end - ch.slot_off[i], cudaMemcpyHostToDevice, c->copy_stream));
       i = j;
     }
-    c->cnt.h2d_bytes += ch.frames.size() * img_bytes;
+    c->cnt.h2d_bytes += ch.bytes;
     CU(cudaEventRecord(c->ev_copied[b], c->copy_stream));
     return CRF_OK;
   };
@@ -856,17 +891,19 @@ static int analyze_resident(crf_ctx* c, const std::vector<FaceDesc>& descs, int 
 // the rest), so that a long video or a batch of 4K frames is not uploaded in one piece.
 constexpr int kDetectGroupFrames = 64;
 
-struct DetectPlan {
-  std::vector<HaarLevel> levels;
-  int rows_pf = 0;                 // window rows of one frame over all levels
-  size_t int_pf = 0, win_pf = 0;   // integral elements / windows of one frame over all levels
+// The pyramid levels of one frame: instances without their group offsets.
+struct FramePlan {
+  std::vector<HaarInst> levels;
+  int nrows = 0;                   // window rows over all levels
+  size_t nint = 0, nwin = 0;       // integral elements / windows over all levels
 };
 
 // the scales of CascadeClassifierImpl::detectMultiScale (flags 0, no maxSize); levels below min_size are not built
-static DetectPlan detect_plan(const Cascade& K, int rows, int cols, double scale_factor, int min_size) {
-  DetectPlan p;
+static FramePlan detect_plan(const Cascade& K, const crf_image_t& im, double scale_factor, int min_size) {
+  FramePlan p;
+  const int rows = im.rows, cols = im.cols;
   for (double factor = 1;; factor *= scale_factor) {
-    HaarLevel L{};
+    HaarInst L{};
     L.factor = factor;
     L.win_w = (int)std::lrint(K.win_w * factor); L.win_h = (int)std::lrint(K.win_h * factor);
     L.sw = (int)std::lrint(cols / factor); L.sh = (int)std::lrint(rows / factor);
@@ -875,96 +912,136 @@ static DetectPlan detect_plan(const Cascade& K, int rows, int cols, double scale
     L.scale_x = 1. / ((double)L.sw / cols); L.scale_y = 1. / ((double)L.sh / rows);
     L.ystep = factor > 2. ? 1 : 2;
     L.nx = (L.sw - K.win_w + 1 + L.ystep - 1) / L.ystep; L.ny = (L.sh - K.win_h + 1 + L.ystep - 1) / L.ystep;
-    L.row_off = p.rows_pf;
-    L.int_fs = (size_t)(L.sw + 1) * (L.sh + 1);
-    p.rows_pf += L.ny;
-    p.int_pf += L.int_fs;
-    p.win_pf += (size_t)L.nx * L.ny;
+    L.rows = rows; L.cols = cols; L.step = im.step;
+    p.nrows += L.ny;
+    p.nint += (size_t)(L.sw + 1) * (L.sh + 1);
+    p.nwin += (size_t)L.nx * L.ny;
     p.levels.push_back(L);
   }
   return p;
 }
 
-// Frames [f0, f0 + nf) into d_haar_frames, frame k at k * rows * step.  Pinned frames are copied straight (frames adjacent in host memory
-// in one copy); pageable ones are packed into the two pinned staging buffers by a few threads and copied from there.
-static int upload_frames(crf_ctx* c, const uint8_t* const* images, int f0, int nf, int rows, size_t step, cudaStream_t s) {
-  const size_t fb = (size_t)rows * step;
+// Frames [f0, f0 + nf) into d_haar_frames at off[k] (prefix sums of rows x step).  Pinned frames are copied straight (frames adjacent in
+// host memory in one copy); pageable ones are packed into the two pinned staging buffers (~64 MB a batch) by a few threads and copied
+// from there.
+static int upload_frames(crf_ctx* c, const crf_image_t* images, int f0, int nf, const std::vector<size_t>& off, cudaStream_t s) {
+  auto fb = [&](int k) { return image_bytes(images[f0 + k]); };
   uint8_t* d = c->d_haar_frames.as<uint8_t>();
   std::vector<int> pageable;
   for (int k = 0; k < nf;) {
-    if (!is_pinned_host(images[f0 + k])) { pageable.push_back(k++); continue; }
+    if (!is_pinned_host(images[f0 + k].bgr)) { pageable.push_back(k++); continue; }
     int j = k + 1;
-    while (j < nf && images[f0 + j] == images[f0 + j - 1] + fb && is_pinned_host(images[f0 + j])) j++;
-    CU(cudaMemcpyAsync(d + (size_t)k * fb, images[f0 + k], (size_t)(j - k) * fb, cudaMemcpyHostToDevice, s));
+    while (j < nf && images[f0 + j].bgr == images[f0 + j - 1].bgr + fb(j - 1) && is_pinned_host(images[f0 + j].bgr)) j++;
+    CU(cudaMemcpyAsync(d + off[(size_t)k], images[f0 + k].bgr, off[(size_t)j] - off[(size_t)k], cudaMemcpyHostToDevice, s));
     k = j;
   }
-  const size_t per = std::max<size_t>(1, ((size_t)64 << 20) / fb);   // frames per staging buffer: ~64 MB
-  for (size_t p0 = 0, b = 0; p0 < pageable.size(); p0 += per, b ^= 1) {
-    const size_t m = std::min(per, pageable.size() - p0);
+  const size_t batch = (size_t)64 << 20;
+  for (size_t p0 = 0, b = 0; p0 < pageable.size(); b ^= 1) {
+    size_t p1 = p0 + 1, bytes = fb(pageable[p0]);
+    while (p1 < pageable.size() && bytes + fb(pageable[p1]) <= batch) bytes += fb(pageable[p1++]);
     CU(cudaEventSynchronize(c->ev_copied[b]));   // the buffer's previous copy has left the host
-    if (c->h_stage_bytes[b] < per * fb) {
+    if (c->h_stage_bytes[b] < bytes) {
       if (c->h_stage[b]) cudaFreeHost(c->h_stage[b]);
       c->h_stage[b] = nullptr; c->h_stage_bytes[b] = 0;
-      CU(cudaHostAlloc((void**)&c->h_stage[b], per * fb, cudaHostAllocDefault));
-      c->h_stage_bytes[b] = per * fb;
+      CU(cudaHostAlloc((void**)&c->h_stage[b], bytes, cudaHostAllocDefault));
+      c->h_stage_bytes[b] = bytes;
     }
     uint8_t* st = c->h_stage[b];
-    parallel_for((int)m, m * fb, [&](int i) { std::memcpy(st + (size_t)i * fb, images[f0 + pageable[p0 + i]], fb); });
-    for (size_t i = 0; i < m;) {   // runs of consecutive frame slots in one copy
+    std::vector<size_t> st_off(p1 - p0 + 1, 0);
+    for (size_t i = p0; i < p1; i++) st_off[i - p0 + 1] = st_off[i - p0] + fb(pageable[i]);
+    parallel_for((int)(p1 - p0), bytes, [&](int i) { std::memcpy(st + st_off[(size_t)i], images[f0 + pageable[p0 + i]].bgr, fb(pageable[p0 + i])); });
+    for (size_t i = p0; i < p1;) {   // runs of consecutive frame slots in one copy
       size_t j = i + 1;
-      while (j < m && pageable[p0 + j] == pageable[p0 + j - 1] + 1) j++;
-      CU(cudaMemcpyAsync(d + (size_t)pageable[p0 + i] * fb, st + i * fb, (j - i) * fb, cudaMemcpyHostToDevice, s));
+      while (j < p1 && pageable[j] == pageable[j - 1] + 1) j++;
+      CU(cudaMemcpyAsync(d + off[(size_t)pageable[i]], st + st_off[i - p0], st_off[j - p0] - st_off[i - p0], cudaMemcpyHostToDevice, s));
       i = j;
     }
     CU(cudaEventRecord(c->ev_copied[b], s));
+    p0 = p1;
   }
-  c->cnt.h2d_bytes += (size_t)nf * fb;
+  c->cnt.h2d_bytes += off[(size_t)nf];
   return CRF_OK;
 }
 
-// detectMultiScale on n_images equal-size frames, a group of frames at a time.  After a group's boxes are grouped, per_group(f0, nf, boxes)
-// runs while the group's frames are still in d_haar_frames (frame f0 + k at k * rows * step); boxes[k] are frame f0 + k's.
+// detectMultiScale on n_images frames of any sizes, a group of consecutive frames at a time.  After a group's boxes are grouped,
+// per_group(f0, nf, off, boxes) runs while the group's frames are still in d_haar_frames (frame f0 + k at off[k]); boxes[k] are frame
+// f0 + k's.
 template <class F>
-static int detect_frames(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step,
-                         double scale_factor, int min_neighbors, int min_size, F&& per_group) {
+static int detect_frames(crf_ctx* c, const crf_cascade* cas, const crf_image_t* images, int n_images, double scale_factor, int min_neighbors,
+                         int min_size, F&& per_group) {
+  const Cascade& K = cas->c;
+  std::vector<FramePlan> plans((size_t)n_images);
+  for (int i = 0; i < n_images; i++) {
+    plans[(size_t)i] = detect_plan(K, images[i], scale_factor, min_size);
+    // work lists hold 32-bit flag indices
+    if (plans[(size_t)i].nwin >= ((size_t)1 << 31)) return fail(CRF_ERR_ARG, "frame too large for the detector (2^31 windows)");
+  }
   CU(cudaSetDevice(c->device));
   c->w = &c->ws[0];
   cudaStream_t s = c->w->stream;
   int rc;
-  const Cascade& K = cas->c;
-  if (c->haar_cached != cas) {
+  if (c->haar_cached != cas->id) {
     if ((rc = upload(c->d_haar_stages, K.stages, s)) || (rc = upload(c->d_haar_weak, K.weak, s)) || (rc = upload(c->d_haar_feats, K.features, s))) return rc;
-    c->haar_cached = cas;
+    c->haar_cached = cas->id;
   }
   const HaarDev dev{c->d_haar_stages.as<HaarStage>(), c->d_haar_weak.as<HaarWeak>(), c->d_haar_feats.as<HaarFeature>(), (int)K.stages.size(), K.win_w, K.win_h};
   // stage groups: [0, split[0]), [split[0], split[1]), ..., up to the last stage
   std::vector<int> bounds;
   for (int b : c->haar_split) if (b > (bounds.empty() ? 0 : bounds.back()) && b < dev.nstages) bounds.push_back(b);
   bounds.push_back(dev.nstages);
-  DetectPlan plan = detect_plan(K, rows, cols, scale_factor, min_size);
-  const size_t fb = (size_t)rows * step;
-  // work lists hold 32-bit flag indices
-  if (plan.win_pf >= ((size_t)1 << 31)) return fail(CRF_ERR_ARG, "frame too large for the detector (2^31 windows)");
-  const size_t per_frame = fb + plan.int_pf * 8 + plan.win_pf * (1 + 2 * sizeof(uint2)) + (size_t)plan.rows_pf * 4;
-  int group = (int)std::min<size_t>(kDetectGroupFrames, std::max<size_t>(1, c->work_budget / 2 / per_frame));
-  if (!plan.win_pf) group = kDetectGroupFrames;
-  else group = (int)std::min<size_t>((size_t)group, (((size_t)1 << 32) - 1) / plan.win_pf);
-  const int nl = (int)plan.levels.size();
+  auto footprint = [&](int i) { const FramePlan& p = plans[(size_t)i]; return image_bytes(images[i]) + p.nint * 8 + p.nwin * (1 + 2 * sizeof(uint2)) + (size_t)p.nrows * 4; };
   std::vector<std::vector<crf_rect_t>> boxes;
   std::vector<int> frame_count;
-  for (int f0 = 0; f0 < n_images; f0 += group) {
-    const int nf = std::min(group, n_images - f0);
+  for (int f0 = 0, f1; f0 < n_images; f0 = f1) {
+    // a group: consecutive frames, at most kDetectGroupFrames, within half the work budget, fewer than 2^32 windows
+    size_t bytes = footprint(f0), wins = plans[(size_t)f0].nwin;
+    for (f1 = f0 + 1; f1 < n_images && f1 - f0 < kDetectGroupFrames; f1++) {
+      if (bytes + footprint(f1) > c->work_budget / 2 || wins + plans[(size_t)f1].nwin > ((size_t)1 << 32) - 1) break;
+      bytes += footprint(f1); wins += plans[(size_t)f1].nwin;
+    }
+    const int nf = f1 - f0;
     boxes.assign((size_t)nf, {});
-    if (nl > 0) {
-      size_t io = 0, fo = 0;
-      for (HaarLevel& L : plan.levels) { L.int_off = io; io += (size_t)nf * L.int_fs; L.flag_off = fo; fo += (size_t)nf * L.nx * L.ny; }
-      const int nrows = nf * plan.rows_pf;
-      if ((rc = c->d_haar_frames.reserve((size_t)nf * fb)) || (rc = c->d_haar_S.reserve(io * 4)) || (rc = c->d_haar_Q.reserve(io * 4)) ||
+    // the instance table (frame-major, then level), the frames' device offsets and their window-row ranges
+    std::vector<HaarInst> inst;
+    std::vector<size_t> off((size_t)nf + 1, 0);
+    std::vector<int> frame_rows((size_t)nf + 1, 0);
+    size_t io = 0, fo = 0;
+    int nrows = 0, brows = 0, bcols = 0, beval = 0;
+    for (int k = 0; k < nf; k++) {
+      off[(size_t)k + 1] = off[(size_t)k] + image_bytes(images[f0 + k]);
+      for (HaarInst L : plans[(size_t)(f0 + k)].levels) {
+        L.img_off = off[(size_t)k]; L.frame = k;
+        L.int_off = io; io += (size_t)(L.sw + 1) * (L.sh + 1);
+        L.flag_off = fo; fo += (size_t)L.nx * L.ny;
+        L.row_off = nrows; nrows += L.ny;
+        L.blk_rows = brows; brows += (L.sh + 7) / 8;
+        L.blk_cols = bcols; bcols += (L.sw + 1 + 31) / 32;
+        L.blk_eval = beval; beval += (L.nx + 127) / 128 * L.ny;
+        inst.push_back(L);
+      }
+      frame_rows[(size_t)k + 1] = nrows;
+    }
+    if (!inst.empty()) {
+      const int ninst = (int)inst.size();
+      // one upload: the instances, then the frames' row ranges, then the search keys (HaarKeys)
+      const size_t tab = ((size_t)ninst * sizeof(HaarInst) + 15) & ~(size_t)15;
+      std::vector<int> ints(frame_rows);
+      for (int k = 0; k < 5; k++)
+        for (const HaarInst& L : inst)
+          ints.push_back(k == 0 ? L.blk_rows : k == 1 ? L.blk_cols : k == 2 ? L.blk_eval : k == 3 ? L.row_off : (int)(unsigned)L.flag_off);
+      std::vector<uint8_t> table(tab + ints.size() * sizeof(int));
+      std::memcpy(table.data(), inst.data(), (size_t)ninst * sizeof(HaarInst));
+      std::memcpy(table.data() + tab, ints.data(), ints.size() * sizeof(int));
+      if ((rc = c->d_haar_frames.reserve(off[(size_t)nf])) || (rc = c->d_haar_S.reserve(io * 4)) || (rc = c->d_haar_Q.reserve(io * 4)) ||
           (rc = c->d_haar_flags.reserve(fo)) || (rc = c->d_haar_list[0].reserve(fo * sizeof(uint2))) || (rc = c->d_haar_list[1].reserve(fo * sizeof(uint2))) ||
           (rc = c->d_haar_rows.reserve((size_t)nrows * 4)) || (rc = c->d_haar_counts.reserve((size_t)(kDetectGroupFrames + 4) * 4)))
         return rc;
-      if ((rc = upload_frames(c, images, f0, nf, rows, step, s))) return rc;
-      if ((rc = upload(c->d_haar_levels, plan.levels, s))) return rc;
+      if ((rc = upload_frames(c, images, f0, nf, off, s))) return rc;
+      if ((rc = upload(c->d_haar_levels, table, s))) return rc;
+      const HaarInst* d_inst = c->d_haar_levels.as<HaarInst>();
+      const int* d_frame_rows = reinterpret_cast<const int*>(c->d_haar_levels.as<uint8_t>() + tab);
+      const int* d_key = d_frame_rows + frame_rows.size();
+      const HaarKeys keys{d_key, d_key + ninst, d_key + 2 * ninst, d_key + 3 * ninst, reinterpret_cast<const unsigned*>(d_key + 4 * ninst)};
       unsigned* lists_n = c->d_haar_counts.as<unsigned>();   // [0], [1]: lengths of the two work lists; [4...]: candidates per frame
       int* fcount = c->d_haar_counts.as<int>() + 4;
       CU(cudaMemsetAsync(lists_n, 0, 4 * sizeof(unsigned), s));
@@ -972,22 +1049,19 @@ static int detect_frames(crf_ctx* c, const crf_cascade* cas, const uint8_t* cons
       uint32_t* Q = c->d_haar_Q.as<uint32_t>();
       uint8_t* flags = c->d_haar_flags.as<uint8_t>();
       uint2* list[2] = {c->d_haar_list[0].as<uint2>(), c->d_haar_list[1].as<uint2>()};
-      for (const HaarLevel& L : plan.levels) {
-        k_haar_rows<<<dim3((L.sh + 7) / 8, nf), 256, 0, s>>>(c->d_haar_frames.as<uint8_t>(), fb, rows, cols, step, L, S, Q);
-        k_haar_cols<<<dim3((L.sw + 1 + 31) / 32, nf), dim3(32, 32), 0, s>>>(L, S, Q);
-        k_haar_eval_first<<<dim3((L.nx + 127) / 128, L.ny, nf), 128, 0, s>>>(L, S, Q, dev, bounds[0], flags, list[0], lists_n);
-        KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 3);
-      }
-      const HaarLevel* d_levels = c->d_haar_levels.as<HaarLevel>();
+      k_haar_rows<<<brows, 256, 0, s>>>(d_inst, keys, ninst, c->d_haar_frames.as<uint8_t>(), S, Q);
+      k_haar_cols<<<bcols, dim3(32, 32), 0, s>>>(d_inst, keys, ninst, S, Q);
+      k_haar_eval_first<<<beval, 128, 0, s>>>(d_inst, keys, ninst, S, Q, dev, bounds[0], flags, list[0], lists_n);
+      KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 3);
       for (size_t g = 1; g < bounds.size(); g++) {
         const int in = (int)((g - 1) & 1), out = (int)(g & 1);
         if (g >= 2) CU(cudaMemsetAsync(lists_n + out, 0, sizeof(unsigned), s));
-        k_haar_eval_list<<<c->sm_count * 8, 128, 0, s>>>(d_levels, nl, S, dev, bounds[g - 1], bounds[g], list[in], lists_n + in, flags, list[out], lists_n + out);
+        k_haar_eval_list<<<c->sm_count * 8, 128, 0, s>>>(d_inst, keys, ninst, S, dev, bounds[g - 1], bounds[g], list[in], lists_n + in, flags, list[out], lists_n + out);
         KCHECK(); count_launch(c, CRF_STAGE_RESIZE);
       }
       int* d_rows = c->d_haar_rows.as<int>();
-      k_haar_scan<true><<<(nrows + 7) / 8, 256, 0, s>>>(d_levels, nl, nrows, plan.rows_pf, flags, d_rows, nullptr, nullptr);
-      k_haar_row_offsets<<<nf, 1024, 0, s>>>(plan.rows_pf, d_rows, fcount);
+      k_haar_scan<true><<<(nrows + 7) / 8, 256, 0, s>>>(d_inst, keys, ninst, nrows, flags, d_rows, nullptr, nullptr);
+      k_haar_row_offsets<<<nf, 1024, 0, s>>>(d_frame_rows, d_rows, fcount);
       KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 2);
       frame_count.assign((size_t)nf, 0);
       CU(cudaMemcpyAsync(frame_count.data(), fcount, (size_t)nf * 4, cudaMemcpyDeviceToHost, s));
@@ -995,7 +1069,7 @@ static int detect_frames(crf_ctx* c, const crf_cascade* cas, const uint8_t* cons
       size_t total = 0;
       for (int v : frame_count) total += (size_t)v;
       if ((rc = c->d_haar_cand.reserve(std::max<size_t>(total, 1) * sizeof(crf_rect_t)))) return rc;
-      k_haar_scan<false><<<(nrows + 7) / 8, 256, 0, s>>>(d_levels, nl, nrows, plan.rows_pf, flags, d_rows, fcount, c->d_haar_cand.as<crf_rect_t>());
+      k_haar_scan<false><<<(nrows + 7) / 8, 256, 0, s>>>(d_inst, keys, ninst, nrows, flags, d_rows, fcount, c->d_haar_cand.as<crf_rect_t>());
       KCHECK(); count_launch(c, CRF_STAGE_RESIZE);
       std::vector<crf_rect_t> cand(total);
       if (total) CU(cudaMemcpyAsync(cand.data(), c->d_haar_cand.p, total * sizeof(crf_rect_t), cudaMemcpyDeviceToHost, s));
@@ -1007,7 +1081,7 @@ static int detect_frames(crf_ctx* c, const crf_cascade* cas, const uint8_t* cons
       for (int v : frame_count) work += (size_t)v * v;
       parallel_for(nf, work * 64, [&](int k) { group_rectangles(boxes[(size_t)k], min_neighbors, 0.2); });
     }
-    if ((rc = per_group(f0, nf, boxes))) return rc;
+    if ((rc = per_group(f0, nf, off, boxes))) return rc;
   }
   return CRF_OK;
 }
@@ -1020,13 +1094,32 @@ static crf_rect_t enlarge_detection(const crf_rect_t& r, int rows, int cols) {
   return x1 > x0 && y1 > y0 ? crf_rect_t{x0, y0, x1 - x0, y1 - y0} : crf_rect_t{0, 0, 0, 0};
 }
 
-static int detect_args(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, double scale_factor, int cap,
-                       const void* out) {
+static int detect_args(crf_ctx* c, const crf_cascade* cas, const crf_image_t* images, int n_images, double scale_factor, int cap, const void* out) {
   if (!c) return fail(CRF_ERR_STATE, "context is not initialised");
-  if (!cas || n_images < 0 || (n_images > 0 && !images) || rows < 1 || cols < 1 || step < (size_t)cols * 3 || !(scale_factor > 1.0) || cap < 0 || (cap > 0 && !out))
-    return fail(CRF_ERR_ARG, "bad argument");
-  for (int i = 0; i < n_images; i++) if (!images[i]) return fail(CRF_ERR_ARG, "null frame");
+  if (!cas || n_images < 0 || (n_images > 0 && !images) || !(scale_factor > 1.0) || cap < 0 || (cap > 0 && !out)) return fail(CRF_ERR_ARG, "bad argument");
+  return image_args(images, n_images);
+}
+
+// the equal-size calls check their one geometry even without frames
+static int same_size_args(const crf_ctx* c, int rows, int cols, size_t step) {
+  if (c && (rows < 1 || cols < 1 || step < (size_t)cols * 3)) return fail(CRF_ERR_ARG, "bad argument");
   return CRF_OK;
+}
+
+// detectMultiScale on n_images frames: returns the total box count, the first `cap` boxes in out and, when image_of_box is given, their frames
+static int detect_boxes(crf_ctx* c, const crf_cascade* cas, const crf_image_t* images, int n_images, double scale_factor, int min_neighbors, int min_size,
+                        crf_rect_t* out, int* image_of_box, int cap) {
+  int total = 0;
+  const int rc = detect_frames(c, cas, images, n_images, scale_factor, min_neighbors, min_size,
+                               [&](int f0, int nf, const std::vector<size_t>&, std::vector<std::vector<crf_rect_t>>& boxes) -> int {
+    for (int k = 0; k < nf; k++)
+      for (const crf_rect_t& r : boxes[(size_t)k]) {
+        if (total < cap) { out[total] = r; if (image_of_box) image_of_box[total] = f0 + k; }
+        total++;
+      }
+    return CRF_OK;
+  });
+  return rc ? rc : total;
 }
 }  // namespace crf
 
@@ -1040,7 +1133,9 @@ extern "C" {
 int crf_cascade_load(const char* path, crf_cascade** out) {
   if (!path || !out) return fail(CRF_ERR_ARG, "null argument");
   *out = nullptr;
+  static std::atomic<unsigned long long> next_id{1};
   std::unique_ptr<crf_cascade> c(new crf_cascade());
+  c->id = next_id++;
   std::string err;
   const int rc = load_cascade(path, c->c, err);
   if (rc) return fail(rc, err);
@@ -1058,61 +1153,57 @@ int crf_cascade_info(const crf_cascade* c, int* win_w, int* win_h, int* nstages,
   return CRF_OK;
 }
 
+int crf_detect_faces_batch_mixed(crf_ctx* c, const crf_cascade* cas, const crf_image_t* images, int n_images, double scale_factor, int min_neighbors,
+                                 int min_size, crf_rect_t* out, int* image_of_box, int cap) {
+  if (int rc = detect_args(c, cas, images, n_images, scale_factor, cap, out)) return rc;
+  if (cap > 0 && !image_of_box) return fail(CRF_ERR_ARG, "bad argument");
+  return detect_boxes(c, cas, images, n_images, scale_factor, min_neighbors, min_size, out, image_of_box, cap);
+}
+
 int crf_detect_faces(crf_ctx* c, const crf_cascade* cas, const uint8_t* bgr, int rows, int cols, size_t step, double scale_factor, int min_neighbors, int min_size,
                      crf_rect_t* out, int cap) {
-  if (int rc = detect_args(c, cas, &bgr, 1, rows, cols, step, scale_factor, cap, out)) return rc;
-  int total = 0;
-  const int rc = detect_frames(c, cas, &bgr, 1, rows, cols, step, scale_factor, min_neighbors, min_size, [&](int, int, std::vector<std::vector<crf_rect_t>>& boxes) -> int {
-    for (const crf_rect_t& r : boxes[0]) { if (total < cap) out[total] = r; total++; }
-    return CRF_OK;
-  });
-  return rc ? rc : total;
+  const crf_image_t im{bgr, rows, cols, step};
+  if (int rc = detect_args(c, cas, &im, 1, scale_factor, cap, out)) return rc;
+  return detect_boxes(c, cas, &im, 1, scale_factor, min_neighbors, min_size, out, nullptr, cap);
 }
 
 int crf_detect_faces_batch(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, double scale_factor,
                            int min_neighbors, int min_size, crf_rect_t* out, int* image_of_box, int cap) {
-  if (int rc = detect_args(c, cas, images, n_images, rows, cols, step, scale_factor, cap, out)) return rc;
-  if (cap > 0 && !image_of_box) return fail(CRF_ERR_ARG, "bad argument");
-  int total = 0;
-  const int rc = detect_frames(c, cas, images, n_images, rows, cols, step, scale_factor, min_neighbors, min_size, [&](int f0, int nf, std::vector<std::vector<crf_rect_t>>& boxes) -> int {
-    for (int k = 0; k < nf; k++)
-      for (const crf_rect_t& r : boxes[(size_t)k]) {
-        if (total < cap) { out[total] = r; image_of_box[total] = f0 + k; }
-        total++;
-      }
-    return CRF_OK;
-  });
-  return rc ? rc : total;
+  if (int rc = same_size_args(c, rows, cols, step)) return rc;
+  std::vector<crf_image_t> v;
+  return crf_detect_faces_batch_mixed(c, cas, same_size(images, n_images, rows, cols, step, v), n_images, scale_factor, min_neighbors, min_size, out, image_of_box, cap);
 }
 
-int crf_analyze_images(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, double scale_factor,
-                       int min_neighbors, int min_size, crf_rect_t* boxes, int* image_of_box, crf_face_t* out, int cap) {
-  if (int rc = detect_args(c, cas, images, n_images, rows, cols, step, scale_factor, cap, boxes)) return rc;
+int crf_analyze_images_mixed(crf_ctx* c, const crf_cascade* cas, const crf_image_t* images, int n_images, double scale_factor, int min_neighbors, int min_size,
+                             crf_rect_t* boxes, int* image_of_box, crf_face_t* out, int cap) {
+  if (int rc = detect_args(c, cas, images, n_images, scale_factor, cap, boxes)) return rc;
   if (cap > 0 && (!image_of_box || !out)) return fail(CRF_ERR_ARG, "bad argument");
   if (!c->full_model) return fail(CRF_ERR_STATE, "analyzeFace needs the head-pose forest and the 5 pose forests; this context holds a single forest");
-  const size_t fb = (size_t)rows * step;
   int total = 0;
-  const int rc = detect_frames(c, cas, images, n_images, rows, cols, step, scale_factor, min_neighbors, min_size, [&](int f0, int nf, std::vector<std::vector<crf_rect_t>>& det) -> int {
+  const int rc = detect_frames(c, cas, images, n_images, scale_factor, min_neighbors, min_size,
+                               [&](int f0, int nf, const std::vector<size_t>& off, std::vector<std::vector<crf_rect_t>>& det) -> int {
     // FaceDescs point into the group's device frames: the analysis reads the copy made for detection
     std::vector<FaceDesc> descs;
     std::vector<int> slot;   // output index of descs[i]
     int Hmax = 0;
-    for (int k = 0; k < nf; k++)
+    for (int k = 0; k < nf; k++) {
+      const crf_image_t& im = images[f0 + k];
       for (const crf_rect_t& r : det[(size_t)k]) {
         if (total < cap) {
-          const crf_rect_t e = enlarge_detection(r, rows, cols);
+          const crf_rect_t e = enlarge_detection(r, im.rows, im.cols);
           boxes[total] = e; image_of_box[total] = f0 + k; out[total] = crf_face_t{};
-          if (box_error(rows, cols, e)) {
+          if (box_error(im.rows, im.cols, e)) {
             out[total].flags = CRF_FACE_NOT_ANALYSED;
           } else {
             FaceDesc d;
-            if (int rc2 = make_desc(c, rows, cols, step, (size_t)k * fb, e, d)) return rc2;
+            if (int rc2 = make_desc(c, im.rows, im.cols, im.step, off[(size_t)k], e, d)) return rc2;
             descs.push_back(d); slot.push_back(total);
             Hmax = std::max(Hmax, d.H);
           }
         }
         total++;
       }
+    }
     if (descs.empty()) return CRF_OK;
     int rc2;
     if ((rc2 = c->d_faces.reserve(descs.size() * sizeof(crf_face_t)))) return rc2;
@@ -1126,6 +1217,14 @@ int crf_analyze_images(crf_ctx* c, const crf_cascade* cas, const uint8_t* const*
     return CRF_OK;
   });
   return rc ? rc : total;
+}
+
+int crf_analyze_images(crf_ctx* c, const crf_cascade* cas, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, double scale_factor,
+                       int min_neighbors, int min_size, crf_rect_t* boxes, int* image_of_box, crf_face_t* out, int cap) {
+  if (int rc = same_size_args(c, rows, cols, step)) return rc;
+  std::vector<crf_image_t> v;
+  return crf_analyze_images_mixed(c, cas, same_size(images, n_images, rows, cols, step, v), n_images, scale_factor, min_neighbors, min_size, boxes, image_of_box,
+                                  out, cap);
 }
 
 const char* crf_last_error(void) { return g_last_error.c_str(); }
@@ -1603,22 +1702,36 @@ void crf_host_free(void* p) { if (p) cudaFreeHost(p); }
 
 int crf_analyze_faces(crf_ctx* c, const uint8_t* bgr, int rows, int cols, size_t step, const crf_rect_t* boxes, int n, crf_face_t* out) {
   std::vector<int> zero((size_t)std::max(n, 0), 0);
-  const uint8_t* imgs[1] = {bgr};
-  return analyze_host(c, imgs, 1, rows, cols, step, boxes, zero.data(), n, out, false);
+  const crf_image_t im{bgr, rows, cols, step};
+  return analyze_host(c, &im, 1, boxes, zero.data(), n, out, false);
+}
+
+int crf_analyze_batch_mixed(crf_ctx* c, const crf_image_t* images, int n_images, const crf_rect_t* boxes, const int* image_of_box, int n, crf_face_t* out) {
+  if (!image_of_box && n > 0) return fail(CRF_ERR_ARG, "null argument");
+  if (n_images > 0 && !images) return fail(CRF_ERR_ARG, "null argument");
+  if (int rc = image_args(images, n_images)) return rc;
+  return analyze_host(c, images, n_images, boxes, image_of_box, n, out, false);
 }
 
 int crf_analyze_batch(crf_ctx* c, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, const crf_rect_t* boxes,
                       const int* image_of_box, int n, crf_face_t* out) {
   if (!image_of_box && n > 0) return fail(CRF_ERR_ARG, "null argument");
-  return analyze_host(c, images, n_images, rows, cols, step, boxes, image_of_box, n, out, false);
+  std::vector<crf_image_t> v;
+  return analyze_host(c, same_size(images, n_images, rows, cols, step, v), n_images, boxes, image_of_box, n, out, false);
+}
+
+// n crops back to back in bgr_batch, one frame per crop
+static const crf_image_t* crop_frames(const uint8_t* bgr_batch, int n, int rows, int cols, std::vector<crf_image_t>& v) {
+  v.resize((size_t)std::max(n, 0));
+  for (int i = 0; i < n; i++) v[(size_t)i] = crf_image_t{bgr_batch + (size_t)i * rows * cols * 3, rows, cols, (size_t)cols * 3};
+  return v.data();
 }
 
 static int crops_host(crf_ctx* c, const uint8_t* bgr_batch, int n, int rows, int cols, crf_face_t* out, bool hp_only) {
   if (n < 0 || (n > 0 && !bgr_batch)) return fail(CRF_ERR_ARG, "null argument");
-  std::vector<const uint8_t*> imgs((size_t)std::max(n, 0));
+  std::vector<crf_image_t> imgs;
   std::vector<crf_rect_t> boxes((size_t)std::max(n, 0), crf_rect_t{0, 0, cols, rows});
-  for (int i = 0; i < n; i++) imgs[i] = bgr_batch + (size_t)i * rows * cols * 3;
-  return analyze_host(c, imgs.data(), n, rows, cols, (size_t)cols * 3, boxes.data(), nullptr, n, out, hp_only);
+  return analyze_host(c, crop_frames(bgr_batch, n, rows, cols, imgs), n, boxes.data(), nullptr, n, out, hp_only);
 }
 
 int crf_analyze_crops(crf_ctx* c, const uint8_t* bgr_batch, int n, int rows, int cols, crf_face_t* out) { return crops_host(c, bgr_batch, n, rows, cols, out, false); }
@@ -1679,8 +1792,8 @@ int crf_multi_create(const crf_model* model, const int* devices, int n_devices, 
 int crf_multi_device_count(const crf_multi* m) { return m ? (int)m->ctx.size() : 0; }
 crf_ctx* crf_multi_ctx(crf_multi* m, int i) { return m && i >= 0 && i < (int)m->ctx.size() ? m->ctx[(size_t)i] : nullptr; }
 
-static int multi_run(crf_multi* m, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, const crf_rect_t* boxes, const int* image_of_box, int n,
-                     crf_face_t* out, bool headpose_only) {
+static int multi_run(crf_multi* m, const crf_image_t* images, int n_images, const crf_rect_t* boxes, const int* image_of_box, int n, crf_face_t* out,
+                     bool headpose_only) {
   if (!m || m->ctx.empty()) return fail(CRF_ERR_STATE, "context is not initialised");
   if (n < 0 || (n > 0 && (!images || !boxes || !out))) return fail(CRF_ERR_ARG, "null argument");
   const int G = (int)m->ctx.size();
@@ -1698,13 +1811,19 @@ static int multi_run(crf_multi* m, const uint8_t* const* images, int n_images, i
     }
     cut[(size_t)g] = std::max(c, cut[(size_t)g - 1]);
   }
+  // all-or-nothing: every shard's boxes are checked before any shard writes into out
+  for (int g = 0; g < G; g++) {
+    const int f0 = cut[(size_t)g], f1 = cut[(size_t)g + 1];
+    if (f1 > f0 && box_args(image_of_box ? images : images + f0, image_of_box ? n_images : f1 - f0, boxes + f0, image_of_box ? image_of_box + f0 : nullptr, f1 - f0))
+      return fail(CRF_ERR_ARG, "GPU shard " + std::to_string(g) + ": " + g_last_error);
+  }
   std::vector<int> rcs((size_t)G, CRF_OK);
   std::vector<std::string> errs((size_t)G);
   auto work = [&](int g) {
     const int f0 = cut[(size_t)g], f1 = cut[(size_t)g + 1];
     if (f1 <= f0) return;
     // a shard names its frames through the caller's image_of_box; crops (image_of_box == NULL) are one frame per face
-    rcs[(size_t)g] = analyze_host(m->ctx[(size_t)g], image_of_box ? images : images + f0, image_of_box ? n_images : f1 - f0, rows, cols, step, boxes + f0,
+    rcs[(size_t)g] = analyze_host(m->ctx[(size_t)g], image_of_box ? images : images + f0, image_of_box ? n_images : f1 - f0, boxes + f0,
                                   image_of_box ? image_of_box + f0 : nullptr, f1 - f0, out + f0, headpose_only);
     if (rcs[(size_t)g]) errs[(size_t)g] = g_last_error;   // thread-local in the worker: hand it to the caller
   };
@@ -1717,18 +1836,26 @@ static int multi_run(crf_multi* m, const uint8_t* const* images, int n_images, i
   return CRF_OK;
 }
 
+int crf_multi_analyze_batch_mixed(crf_multi* m, const crf_image_t* images, int n_images, const crf_rect_t* boxes, const int* image_of_box, int n,
+                                  crf_face_t* out) {
+  if (!image_of_box && n > 0) return fail(CRF_ERR_ARG, "null argument");
+  if (n_images > 0 && !images) return fail(CRF_ERR_ARG, "null argument");
+  if (int rc = image_args(images, n_images)) return rc;
+  return multi_run(m, images, n_images, boxes, image_of_box, n, out, false);
+}
+
 int crf_multi_analyze_batch(crf_multi* m, const uint8_t* const* images, int n_images, int rows, int cols, size_t step, const crf_rect_t* boxes,
                             const int* image_of_box, int n, crf_face_t* out) {
   if (!image_of_box && n > 0) return fail(CRF_ERR_ARG, "null argument");
-  return multi_run(m, images, n_images, rows, cols, step, boxes, image_of_box, n, out, false);
+  std::vector<crf_image_t> v;
+  return multi_run(m, same_size(images, n_images, rows, cols, step, v), n_images, boxes, image_of_box, n, out, false);
 }
 
 int crf_multi_analyze_crops(crf_multi* m, const uint8_t* bgr_batch, int n, int rows, int cols, crf_face_t* out, int headpose_only) {
   if (n < 0 || (n > 0 && !bgr_batch)) return fail(CRF_ERR_ARG, "null argument");
-  std::vector<const uint8_t*> imgs((size_t)std::max(n, 0));
+  std::vector<crf_image_t> imgs;
   std::vector<crf_rect_t> boxes((size_t)std::max(n, 0), crf_rect_t{0, 0, cols, rows});
-  for (int i = 0; i < n; i++) imgs[(size_t)i] = bgr_batch + (size_t)i * rows * cols * 3;
-  return multi_run(m, imgs.data(), n, rows, cols, (size_t)cols * 3, boxes.data(), nullptr, n, out, headpose_only != 0);
+  return multi_run(m, crop_frames(bgr_batch, n, rows, cols, imgs), n, boxes.data(), nullptr, n, out, headpose_only != 0);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -5,8 +5,8 @@
 // The algorithm is OpenCV's (objdetect/cascadedetect.cpp; not under /root/reference): per scale factor = 1.3^k a bilinear
 // pyramid level of the gray frame, integral images of values and squares, then every window position of the level's
 // ystep grid walks the 22 stages / 2135 stumps until a stage sum falls below its threshold; surviving windows are grouped
-// by cv::groupRectangles.  Here a group of frames goes through each step in one launch: pyramid level + row scan, column
-// scan, the first stage group over every window (one thread per window position, adjacent threads = adjacent windows, so
+// by cv::groupRectangles.  Here a group of frames of any sizes goes through each step in one launch over all its (frame, level)
+// instances: pyramid + row scan, column scan, the first stage group over every window (one thread per window position, adjacent threads = adjacent windows, so
 // the corner loads of a stump coalesce; the cascade tables are broadcast loads), later stage groups on compacted work lists
 // of the survivors, then OpenCV's "skip one more step after a stage-0 reject" scan rule and the candidate compaction on the
 // device.  Only the candidate rectangles come back; grouping (cv::groupRectangles) runs on the host, a frame per thread.
@@ -109,24 +109,48 @@ static int load_cascade(const std::string& path, Cascade& c, std::string& err) {
 }
 
 // ---- kernels ---------------------------------------------------------------------------------------------------------------
-// The frames of a group (equal size) are detected together; every buffer holds all frames of the group, level by level:
-//   S, Q   [level][frame][(sh + 1) x (sw + 1)] u32 integrals of values and squares (pitch sw + 1)
-//   flags  [level][frame][ny][nx] u8 per window of the level's ystep grid: bit 0 = passed every stage, bit 1 = rejected by stage 0
-//   rows   [frame][level][iy] candidates per window row, then their offsets within the frame
-// Launches per group: 3 per pyramid level, 1 per later stage group, 3 for the scan rule and the candidate compaction, whatever
-// the number of frames.
-struct HaarLevel {
+// The frames of a group (any sizes) are detected together.  The group is a table of (frame, level) instances, frame-major then level;
+// every buffer holds all instances of the group in that order:
+//   frames [frame] BGR rows of frame f at its img_off (prefix sums of rows x step, no padding)
+//   S, Q   [instance][(sh + 1) x (sw + 1)] u32 integrals of values and squares (pitch sw + 1)
+//   flags  [instance][ny][nx] u8 per window of the level's ystep grid: bit 0 = passed every stage, bit 1 = rejected by stage 0
+//   rows   [instance][iy] candidates per window row, then their offsets within the frame (a frame's rows are contiguous)
+// Each pyramid pass is one launch over every instance of the group; a block finds its instance by binary search on the instance's first
+// block of that launch.  Launches per group: 3 for the pyramid passes, 1 per later stage group, 3 for the scan rule and the candidate
+// compaction, whatever the number, sizes and levels of the frames.
+struct HaarInst {
   double factor, scale_x, scale_y;
   int sw, sh, nx, ny, ystep, win_w, win_h;
-  int row_off;                // first window row of the level among a frame's rows
-  size_t int_off, int_fs;     // S / Q of frame f at int_off + f * int_fs
-  size_t flag_off;            // flags of frame f at flag_off + f * nx * ny
+  int rows, cols;             // the instance's frame
+  size_t img_off, step;       // the frame's BGR rows in the group's device copy
+  size_t int_off;             // S / Q of the instance
+  size_t flag_off;            // flags of the instance
+  int frame;                  // frame index within the group
+  int row_off;                // first window row of the instance among the group's rows
+  int blk_rows, blk_cols, blk_eval;   // first block of the instance in k_haar_rows / k_haar_cols / k_haar_eval_first
 };
 
 struct HaarDev { const HaarStage* stages; const HaarWeak* weak; const HaarFeature* feats; int nstages, win_w, win_h; };
 
+// The search keys of the instance table, one compact array per key (a few KB, so the searches stay in L1): key[i] is the instance's
+// blk_rows / blk_cols / blk_eval / row_off / flag_off.  Each array is sorted, as the table is ordered by every offset.
+struct HaarKeys { const int *blk_rows, *blk_cols, *blk_eval, *row_off; const unsigned* flag_off; };
+
+// index of the last instance whose key is <= v
+template <class T>
+__device__ __forceinline__ int haar_inst_of(const T* __restrict__ key, int ninst, T v) {
+  int lo = 0, hi = ninst - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (key[mid] <= v) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
 // pyramid pixel: BGR2GRAY of the source pixels, then INTER_LINEAR (k_gray_resize's arithmetic) to sw x sh
-__device__ __forceinline__ int haar_level_px(const uint8_t* __restrict__ bgr, int rows, int cols, size_t step, const HaarLevel& L, int dx, int dy) {
+__device__ __forceinline__ int haar_level_px(const uint8_t* __restrict__ bgr, const HaarInst& L, int dx, int dy) {
+  const int rows = L.rows, cols = L.cols;
+  const size_t step = L.step;
   if (L.sw == cols && L.sh == rows) return gray_at(bgr, step, dy, dx);
   float fx = (float)((dx + 0.5) * L.scale_x - 0.5);
   int sx = (int)floorf(fx);
@@ -146,21 +170,23 @@ __device__ __forceinline__ int haar_level_px(const uint8_t* __restrict__ bgr, in
 }
 
 // Pyramid level fused with the row pass of its integrals: one warp per level row builds the row's pixels and scans them along x.
-// grid (ceil(sh / 8), frames), 256 threads.
-__global__ void __launch_bounds__(256) k_haar_rows(const uint8_t* __restrict__ frames, size_t frame_bytes, int rows, int cols, size_t step, HaarLevel L,
+// ceil(sh / 8) blocks per instance, 256 threads.
+__global__ void __launch_bounds__(256) k_haar_rows(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, const uint8_t* __restrict__ frames,
                                                    uint32_t* __restrict__ S, uint32_t* __restrict__ Q) {
-  const int y = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31, f = blockIdx.y;
+  const int b = (int)blockIdx.x;
+  const HaarInst L = inst[haar_inst_of(keys.blk_rows, ninst, b)];
+  const int y = (b - L.blk_rows) * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (y >= L.sh) return;
-  const uint8_t* __restrict__ bgr = frames + (size_t)f * frame_bytes;
+  const uint8_t* __restrict__ bgr = frames + L.img_off;
   const size_t P = (size_t)L.sw + 1;
-  uint32_t* __restrict__ s = S + L.int_off + (size_t)f * L.int_fs;
-  uint32_t* __restrict__ q = Q + L.int_off + (size_t)f * L.int_fs;
+  uint32_t* __restrict__ s = S + L.int_off;
+  uint32_t* __restrict__ q = Q + L.int_off;
   if (y == 0) for (size_t x = lane; x < P; x += 32) { s[x] = 0; q[x] = 0; }
   if (lane == 0) { s[(size_t)(y + 1) * P] = 0; q[(size_t)(y + 1) * P] = 0; }
   uint32_t cs = 0, cq = 0;
   for (int x0 = 0; x0 < L.sw; x0 += 32) {
     const int x = x0 + lane;
-    uint32_t v = x < L.sw ? (uint32_t)haar_level_px(bgr, rows, cols, step, L, x, y) : 0u, sq = v * v;
+    uint32_t v = x < L.sw ? (uint32_t)haar_level_px(bgr, L, x, y) : 0u, sq = v * v;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
       const uint32_t nv = __shfl_up_sync(0xffffffffu, v, o), nq = __shfl_up_sync(0xffffffffu, sq, o);
@@ -175,15 +201,18 @@ __global__ void __launch_bounds__(256) k_haar_rows(const uint8_t* __restrict__ f
 // Column pass: a CTA owns 32 columns, its 32 warps 32 consecutive chunks of rows.  Each thread sums its chunk of one column, the chunk
 // totals of a column are scanned in shared memory, then every chunk is walked again with its carry.  S and Q are u32 sums modulo 2^32
 // (OpenCV keeps the square sums in 32 bits too) and integer addition is associative, so any summation order gives the bits of a serial
-// walk down the column.  grid (ceil((sw + 1) / 32), frames), block (32, 32).
-__global__ void __launch_bounds__(1024) k_haar_cols(HaarLevel L, uint32_t* __restrict__ S, uint32_t* __restrict__ Q) {
+// walk down the column.  ceil((sw + 1) / 32) blocks per instance, block (32, 32).
+__global__ void __launch_bounds__(1024) k_haar_cols(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, uint32_t* __restrict__ S, uint32_t* __restrict__ Q) {
   __shared__ uint32_t ts[32][32], tq[32][32];
-  const int tx = threadIdx.x, ty = threadIdx.y, x = blockIdx.x * 32 + tx, f = blockIdx.y;
-  const size_t P = (size_t)L.sw + 1;
-  const int R = (L.sh + 31) / 32, y0 = 1 + ty * R, y1 = min(L.sh + 1, y0 + R);
+  const int b = (int)blockIdx.x;
+  const HaarInst& L = inst[haar_inst_of(keys.blk_cols, ninst, b)];
+  const int sw = L.sw, sh = L.sh;
+  const int tx = threadIdx.x, ty = threadIdx.y, x = (b - L.blk_cols) * 32 + tx;
+  const size_t P = (size_t)sw + 1;
+  const int R = (sh + 31) / 32, y0 = 1 + ty * R, y1 = min(sh + 1, y0 + R);
   const bool col = x < (int)P;
-  uint32_t* __restrict__ s = S + L.int_off + (size_t)f * L.int_fs + x;
-  uint32_t* __restrict__ q = Q + L.int_off + (size_t)f * L.int_fs + x;
+  uint32_t* __restrict__ s = S + L.int_off + x;
+  uint32_t* __restrict__ q = Q + L.int_off + x;
   uint32_t as = 0, aq = 0;
   if (col)
     for (int y = y0; y < y1; y++) { as += s[(size_t)y * P]; aq += q[(size_t)y * P]; }
@@ -236,17 +265,20 @@ __device__ __forceinline__ void haar_append(bool keep, uint2 item, uint2* __rest
   if (keep) list[base + __popc(m & ((1u << lane) - 1u))] = item;
 }
 
-// First stage group, every window of one level of every frame of the group: HaarEvaluator::setWindow's variance normalisation over the
-// inner (w - 2) x (h - 2) rect, stages [0, s_end); writes the window's flag byte and appends the survivors (flag index, 1 / nf) to the
-// work list of the next stage group.  grid (ceil(nx / 128), ny, frames), 128 threads.
-__global__ void __launch_bounds__(128) k_haar_eval_first(HaarLevel L, const uint32_t* __restrict__ S, const uint32_t* __restrict__ Q, HaarDev K, int s_end,
-                                                         uint8_t* __restrict__ flags, uint2* __restrict__ list, unsigned* __restrict__ count) {
-  const int ix = blockIdx.x * blockDim.x + threadIdx.x, iy = blockIdx.y, f = blockIdx.z;
+// First stage group, every window of every instance of the group: HaarEvaluator::setWindow's variance normalisation over the inner
+// (w - 2) x (h - 2) rect, stages [0, s_end); writes the window's flag byte and appends the survivors (flag index, 1 / nf) to the work list
+// of the next stage group.  ceil(nx / 128) x ny blocks per instance, 128 threads.
+__global__ void __launch_bounds__(128) k_haar_eval_first(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, const uint32_t* __restrict__ S, const uint32_t* __restrict__ Q,
+                                                         HaarDev K, int s_end, uint8_t* __restrict__ flags, uint2* __restrict__ list, unsigned* __restrict__ count) {
+  const int b = (int)blockIdx.x;
+  const HaarInst& L = inst[haar_inst_of(keys.blk_eval, ninst, b)];
+  const int nx = L.nx, ystep = L.ystep, bx = (nx + 127) / 128, lb = b - L.blk_eval, iy = lb / bx;
+  const int ix = (lb - iy * bx) * 128 + threadIdx.x;
   bool keep = false;
   uint2 item = make_uint2(0u, 0u);
-  if (ix < L.nx) {
+  if (ix < nx) {
     const size_t P = (size_t)L.sw + 1;
-    const size_t o = L.int_off + (size_t)f * L.int_fs + (size_t)(iy * L.ystep) * P + (size_t)ix * L.ystep;
+    const size_t o = L.int_off + (size_t)(iy * ystep) * P + (size_t)ix * ystep;
     const uint32_t* __restrict__ s0 = S + o;
     const uint32_t* __restrict__ q0 = Q + o;
     const double area = (double)((K.win_w - 2) * (K.win_h - 2));
@@ -262,28 +294,17 @@ __global__ void __launch_bounds__(128) k_haar_eval_first(HaarLevel L, const uint
         else if (r == 0) out = 2;
       }
     }
-    const size_t idx = L.flag_off + (size_t)f * L.nx * L.ny + (size_t)iy * L.nx + ix;
+    const size_t idx = L.flag_off + (size_t)iy * nx + ix;
     flags[idx] = out;
     item = make_uint2((unsigned)idx, __float_as_uint(inv));
   }
   haar_append(keep, item, list, count);
 }
 
-// index of the last level whose field is <= v (the level tables are sorted by every offset)
-template <class T, class G>
-__device__ __forceinline__ int haar_level_of(const HaarLevel* __restrict__ levels, int nlevels, T v, G field) {
-  int lo = 0, hi = nlevels - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (field(levels[mid]) <= v) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
-
 // A later stage group [s_begin, s_end) on the previous group's survivors, grid-stride over the list (its length is on the device, so the
 // launch does not wait for the host).  Compaction changes which thread handles a window, never the order of its arithmetic.  Survivors of
 // the last group get bit 0 of their flag; the others are appended to the next list.
-__global__ void __launch_bounds__(128) k_haar_eval_list(const HaarLevel* __restrict__ levels, int nlevels, const uint32_t* __restrict__ S, HaarDev K,
+__global__ void __launch_bounds__(128) k_haar_eval_list(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, const uint32_t* __restrict__ S, HaarDev K,
                                                         int s_begin, int s_end, const uint2* __restrict__ list_in, const unsigned* __restrict__ count_in,
                                                         uint8_t* __restrict__ flags, uint2* __restrict__ list_out, unsigned* __restrict__ count_out) {
   const unsigned n = *count_in;
@@ -294,11 +315,11 @@ __global__ void __launch_bounds__(128) k_haar_eval_list(const HaarLevel* __restr
     uint2 it = make_uint2(0u, 0u);
     if (i < n) {
       it = list_in[i];
-      const HaarLevel& L = levels[haar_level_of(levels, nlevels, (size_t)it.x, [](const HaarLevel& l) { return l.flag_off; })];
-      const size_t r = it.x - L.flag_off, nxy = (size_t)L.nx * L.ny, f = r / nxy, w = r - f * nxy;
+      const HaarInst& L = inst[haar_inst_of(keys.flag_off, ninst, it.x)];
+      const size_t w = it.x - L.flag_off;
       const int iy = (int)(w / L.nx), ix = (int)(w - (size_t)iy * L.nx);
       const size_t P = (size_t)L.sw + 1;
-      const uint32_t* __restrict__ s0 = S + L.int_off + f * L.int_fs + (size_t)(iy * L.ystep) * P + (size_t)ix * L.ystep;
+      const uint32_t* __restrict__ s0 = S + L.int_off + (size_t)(iy * L.ystep) * P + (size_t)ix * L.ystep;
       if (haar_stages(s0, P, __uint_as_float(it.y), K, s_begin, s_end) < 0) {
         if (last) flags[it.x] = 1; else keep = true;
       }
@@ -321,28 +342,27 @@ __device__ __forceinline__ unsigned haar_visited(unsigned rej0, bool& carry) {
   return vis;
 }
 
-// One warp per window row (frame-major, then level, then iy): candidates = visited windows that passed every stage.  COUNT: the row's
-// candidate count into rows[].  Otherwise: the candidate rectangles, in (level, iy, ix) order per frame and frame after frame, at the
-// row's offset (rows[] after k_haar_row_offsets) plus the counts of the frames before.  grid ceil(frames * rows_pf / 8), 256 threads.
+// One warp per window row of the group (instance by instance, then iy): candidates = visited windows that passed every stage.  COUNT: the
+// row's candidate count into rows[].  Otherwise: the candidate rectangles, in (level, iy, ix) order per frame and frame after frame, at the
+// row's offset (rows[] after k_haar_row_offsets) plus the counts of the frames before.  grid ceil(nrows / 8), 256 threads.
 template <bool COUNT>
-__global__ void __launch_bounds__(256) k_haar_scan(const HaarLevel* __restrict__ levels, int nlevels, int nrows, int rows_pf, const uint8_t* __restrict__ flags,
+__global__ void __launch_bounds__(256) k_haar_scan(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, int nrows, const uint8_t* __restrict__ flags,
                                                    int* __restrict__ rows, const int* __restrict__ frame_count, crf_rect_t* __restrict__ cand) {
   const int rid = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (rid >= nrows) return;
-  const int f = rid / rows_pf, rr = rid - f * rows_pf;
-  const HaarLevel& L = levels[haar_level_of(levels, nlevels, rr, [](const HaarLevel& l) { return l.row_off; })];
-  const int iy = rr - L.row_off;
-  const uint8_t* __restrict__ fl = flags + L.flag_off + (size_t)f * L.nx * L.ny + (size_t)iy * L.nx;
+  const HaarInst& L = inst[haar_inst_of(keys.row_off, ninst, rid)];
+  const int iy = rid - L.row_off, nx = L.nx;
+  const uint8_t* __restrict__ fl = flags + L.flag_off + (size_t)iy * nx;
   int base = 0;
   if (!COUNT) {
     base = rows[rid];
-    for (int k = 0; k < f; k++) base += frame_count[k];
+    for (int k = 0; k < L.frame; k++) base += frame_count[k];
   }
   bool carry = true;
   int n = 0;
-  for (int x0 = 0; x0 < L.nx; x0 += 32) {
+  for (int x0 = 0; x0 < nx; x0 += 32) {
     const int ix = x0 + lane;
-    const uint8_t v = ix < L.nx ? fl[ix] : 0;
+    const uint8_t v = ix < nx ? fl[ix] : 0;
     const unsigned rej0 = __ballot_sync(0xffffffffu, v & 2), pass = __ballot_sync(0xffffffffu, v & 1);
     const unsigned c = haar_visited(rej0, carry) & pass;
     if (!COUNT && ((c >> lane) & 1u))
@@ -352,15 +372,17 @@ __global__ void __launch_bounds__(256) k_haar_scan(const HaarLevel* __restrict__
   if (COUNT && lane == 0) rows[rid] = n;
 }
 
-// Exclusive scan of one frame's row counts in place (row offsets within the frame) and the frame's candidate count.  grid frames, 1024 threads.
-__global__ void __launch_bounds__(1024) k_haar_row_offsets(int rows_pf, int* __restrict__ rows, int* __restrict__ frame_count) {
+// Exclusive scan of one frame's row counts in place (row offsets within the frame) and the frame's candidate count.  Frame f owns the rows
+// [frame_rows[f], frame_rows[f + 1]).  grid frames, 1024 threads.
+__global__ void __launch_bounds__(1024) k_haar_row_offsets(const int* __restrict__ frame_rows, int* __restrict__ rows, int* __restrict__ frame_count) {
   __shared__ int wsum[32];
-  int* __restrict__ r = rows + (size_t)blockIdx.x * rows_pf;
+  const int r0 = frame_rows[blockIdx.x], nr = frame_rows[blockIdx.x + 1] - r0;
+  int* __restrict__ r = rows + r0;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   int carry = 0;
-  for (int b = 0; b < rows_pf; b += 1024) {
+  for (int b = 0; b < nr; b += 1024) {
     const int i = b + threadIdx.x;
-    const int v = i < rows_pf ? r[i] : 0;
+    const int v = i < nr ? r[i] : 0;
     int x = v;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
@@ -373,7 +395,7 @@ __global__ void __launch_bounds__(1024) k_haar_row_offsets(int rows_pf, int* __r
       wsum[lane] = t;
     }
     __syncthreads();
-    if (i < rows_pf) r[i] = carry + (warp ? wsum[warp - 1] : 0) + x - v;
+    if (i < nr) r[i] = carry + (warp ? wsum[warp - 1] : 0) + x - v;
     carry += wsum[31];
     __syncthreads();
   }
@@ -430,4 +452,5 @@ static void group_rectangles(std::vector<crf_rect_t>& rects, int group_threshold
 
 }  // namespace crf
 
-struct crf_cascade { crf::Cascade c; };
+// id: unique per load, so that a context's device copy of a freed cascade is never taken for a new one at the same address
+struct crf_cascade { crf::Cascade c; unsigned long long id = 0; };

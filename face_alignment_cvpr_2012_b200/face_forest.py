@@ -222,6 +222,14 @@ def _options(o: FaceForestOptions | None, hp_stride=None, ffd_stride=None, max_c
     return opt
 
 
+def _frame_list(frames) -> list:
+    """C-contiguous u8 copies (where needed) of the BGR frames of a list or an [n, rows, cols, 3] array.  An array's frames stay back to
+    back in memory, so that they go up in one copy."""
+    if isinstance(frames, np.ndarray):
+        frames = np.ascontiguousarray(frames, np.uint8)
+    return [np.ascontiguousarray(f, np.uint8) for f in frames]
+
+
 class Context:
     """One GPU's packed forests + work buffers (crf_ctx)."""
 
@@ -290,17 +298,14 @@ class Context:
         capi.check(capi.lib().crf_analyze_faces(self.h, bgr.ctypes.data, rows, cols, cols * 3, rects, n, out.ctypes.data))
         return out
 
-    def analyze_batch(self, frames: np.ndarray, boxes, image_of_box) -> np.ndarray:
-        """frames: [n_images, rows, cols, 3] u8 (or a list of equal-size frames)."""
-        frames = [np.ascontiguousarray(f, np.uint8) for f in frames] if not isinstance(frames, np.ndarray) else np.ascontiguousarray(frames, np.uint8)
-        n_images = len(frames)
-        rows, cols = frames[0].shape[:2]
-        ptrs = (C.c_void_p * n_images)(*[f.ctypes.data for f in frames])
+    def analyze_batch(self, frames, boxes, image_of_box) -> np.ndarray:
+        """frames: [n_images, rows, cols, 3] u8, or a list of BGR frames of any sizes; box i lies in frame image_of_box[i]."""
+        frames = _frame_list(frames)
         n = len(boxes)
         rects = (Rect * max(n, 1))(*[Rect(int(b[0]), int(b[1]), int(b[2]), int(b[3])) for b in boxes])
         iob = np.ascontiguousarray(image_of_box, np.int32)
         out = np.zeros(n, FACE_DTYPE)
-        capi.check(capi.lib().crf_analyze_batch(self.h, ptrs, n_images, rows, cols, cols * 3, rects, capi.ptr(iob, C.c_int32), n, out.ctypes.data))
+        capi.check(capi.lib().crf_analyze_batch_mixed(self.h, capi.images(frames), len(frames), rects, capi.ptr(iob, C.c_int32), n, out.ctypes.data))
         return out
 
     # ---- stages (parity tests)
@@ -468,25 +473,18 @@ class CascadeClassifier:
             capi.check(n)
         return [(r.x, r.y, r.width, r.height) for r in out[: min(n, cap)]]
 
-    def _frames(self, frames):
-        frames = [np.ascontiguousarray(f, np.uint8) for f in frames]
-        if frames and any(f.shape != frames[0].shape for f in frames):
-            raise ValueError("frames of one call must have equal sizes")
-        return frames, (C.c_void_p * max(len(frames), 1))(*[f.ctypes.data for f in frames])
-
     def detectMultiScaleBatch(self, ctx: "Context", frames, scaleFactor: float = 1.1, minNeighbors: int = 3, minSize=(0, 0)) -> list:
-        """detectMultiScale on every frame of `frames` (equal-size BGR frames: a list or an [n, rows, cols, 3] array) in one call
-        (crf_detect_faces_batch): one list of (x, y, w, h) per frame, each equal to detectMultiScale on that frame."""
-        frames, ptrs = self._frames(frames)
+        """detectMultiScale on every frame of `frames` (BGR frames of any sizes: a list or an [n, rows, cols, 3] array) in one call
+        (crf_detect_faces_batch_mixed): one list of (x, y, w, h) per frame, each equal to detectMultiScale on that frame."""
+        frames = _frame_list(frames)
         if not frames:
             return []
-        rows, cols = frames[0].shape[:2]
         L = capi.lib()
-        args = (ctx.h, self.h, ptrs, len(frames), rows, cols, cols * 3, float(scaleFactor), int(minNeighbors), int(max(minSize)))
+        args = (ctx.h, self.h, capi.images(frames), len(frames), float(scaleFactor), int(minNeighbors), int(max(minSize)))
         cap = 64 * len(frames)
         while True:
             out, iob = (Rect * cap)(), np.zeros(cap, np.int32)
-            n = L.crf_detect_faces_batch(*args, out, capi.ptr(iob, C.c_int32), cap)
+            n = L.crf_detect_faces_batch_mixed(*args, out, capi.ptr(iob, C.c_int32), cap)
             if n < 0:
                 capi.check(n)
             if n <= cap:
@@ -533,15 +531,14 @@ class MultiContext:
         capi.check(capi.lib().crf_multi_analyze_crops(self.h, host_ptr, n, rows, cols, out.ctypes.data, int(headpose_only)))
 
     def analyze_batch(self, frames, boxes, image_of_box) -> np.ndarray:
-        frames = [np.ascontiguousarray(f, np.uint8) for f in frames] if not isinstance(frames, np.ndarray) else np.ascontiguousarray(frames, np.uint8)
-        n_images = len(frames)
-        rows, cols = frames[0].shape[:2]
-        ptrs = (C.c_void_p * n_images)(*[f.ctypes.data for f in frames])
+        """Context.analyze_batch sharded over the GPUs: frames of any sizes."""
+        frames = _frame_list(frames)
         n = len(boxes)
         rects = (Rect * max(n, 1))(*[Rect(int(b[0]), int(b[1]), int(b[2]), int(b[3])) for b in boxes])
         iob = np.ascontiguousarray(image_of_box, np.int32)
         out = np.zeros(n, FACE_DTYPE)
-        capi.check(capi.lib().crf_multi_analyze_batch(self.h, ptrs, n_images, rows, cols, cols * 3, rects, capi.ptr(iob, C.c_int32), n, out.ctypes.data))
+        capi.check(capi.lib().crf_multi_analyze_batch_mixed(self.h, capi.images(frames), len(frames), rects, capi.ptr(iob, C.c_int32), n,
+                                                            out.ctypes.data))
         return out
 
 
@@ -611,8 +608,8 @@ class FaceForest:
         return out
 
     def analyzeImages(self, frames) -> list:
-        """analyzeImage(img) with the Haar cascade of fd_option for every frame of `frames` (equal-size BGR frames) in one call
-        (crf_analyze_images): the frames cross PCIe once, for detection and analysis.  One list of Face per frame, in
+        """analyzeImage(img) with the Haar cascade of fd_option for every frame of `frames` (BGR frames of any sizes) in one call
+        (crf_analyze_images_mixed): the frames cross PCIe once, for detection and analysis.  One list of Face per frame, in
         detectMultiScale's order.  A detection whose enlarged box the analysis path cannot take (a face cut by the bottom border) comes
         back with a zero record whose flags carry capi.FACE_NOT_ANALYSED, where analyzeImage would raise."""
         if not self.is_inizialized:
@@ -620,17 +617,16 @@ class FaceForest:
         if self.m_face_cascade is None:
             raise AssertionError("no face cascade loaded: set fd_option.path_face_cascade")
         fd = self.option.fd_option
-        frames, ptrs = self.m_face_cascade._frames(frames)
+        frames = _frame_list(frames)
         if not frames:
             return []
-        rows, cols = frames[0].shape[:2]
         L = capi.lib()
-        args = (self.ctx.h, self.m_face_cascade.h, ptrs, len(frames), rows, cols, cols * 3, float(fd.search_scale_factor), int(fd.min_neighbors),
+        args = (self.ctx.h, self.m_face_cascade.h, capi.images(frames), len(frames), float(fd.search_scale_factor), int(fd.min_neighbors),
                 int(fd.min_feature_size))
         cap = 64 * len(frames)
         while True:   # a second call only when the frames hold more than 64 faces each on average
             boxes, iob, recs = (Rect * cap)(), np.zeros(cap, np.int32), np.zeros(cap, FACE_DTYPE)
-            n = L.crf_analyze_images(*args, boxes, capi.ptr(iob, C.c_int32), recs.ctypes.data, cap)
+            n = L.crf_analyze_images_mixed(*args, boxes, capi.ptr(iob, C.c_int32), recs.ctypes.data, cap)
             if n < 0:
                 capi.check(n)
             if n <= cap:

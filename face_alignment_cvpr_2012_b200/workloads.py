@@ -152,3 +152,17 @@ def make_mixed(n_images: int = 64, seed: int = 2015):
         fr, boxes, _, tag = make_frames(1, rows, cols, int(rng.integers(1, 9)), seed=seed * 1000 + i, wmin=64, wmax=min(1500, rows * 2 // 3))
         out.append((fr[0], boxes))
     return out, tag
+
+
+def make_ragged(n_images: int = 64, seed: int = 2017):
+    """R64: n_images frames of n_images distinct sizes, 240 x 320 up to 2160 x 3840 (both sides evenly spaced, so no two frames share a
+    size), in seeded order, with 1-8 boxes each like make_mixed.  Returns a list of (frame, boxes[k,4])."""
+    rng = np.random.default_rng(seed)
+    rows = np.linspace(240, 2160, n_images).round().astype(int)
+    cols = np.linspace(320, 3840, n_images).round().astype(int)
+    out = []
+    for k, i in enumerate(rng.permutation(n_images)):
+        r, c = int(rows[i]), int(cols[i])
+        fr, boxes, _, _ = make_frames(1, r, c, int(rng.integers(1, 9)), seed=seed * 1000 + k, wmin=64, wmax=min(1500, r * 2 // 3))
+        out.append((fr[0], boxes))
+    return out

@@ -45,6 +45,8 @@ typedef struct crf_model crf_model; /* host-side forests: what FaceForest's ctor
 typedef struct crf_ctx crf_ctx;     /* per-GPU context: packed forests + work buffers                */
 
 typedef struct { int x, y, width, height; } crf_rect_t; /* cv::Rect  include/opencv_serialization.hpp:65-72 */
+/* one BGR frame (cv::Mat CV_8UC3) of any size: rows x cols pixels, step bytes from one row to the next (step >= cols * 3) */
+typedef struct { const uint8_t* bgr; int rows, cols; size_t step; } crf_image_t;
 
 /* HeadPoseEstimatorOption + MultiPartEstimatorOption (include/FaceForest.hpp:33-58) and
  * MeanShiftOption (include/MeanShift.hpp:16-25); crf_options_default() fills the reference defaults. */
@@ -176,6 +178,11 @@ int crf_analyze_faces(crf_ctx* ctx, const uint8_t* bgr, int rows, int cols, size
 /* n boxes spread over n_images equal-size frames; image_of_box[i] selects the frame of box i. */
 int crf_analyze_batch(crf_ctx* ctx, const uint8_t* const* images, int n_images, int rows, int cols, size_t step,
                       const crf_rect_t* boxes, const int* image_of_box, int n, crf_face_t* out);
+/* crf_analyze_batch on frames of any sizes: images[k] describes frame k, and each box is validated against its own frame.  Argument
+ * checking is all-or-nothing as above; every descriptor needs a non-null bgr, rows, cols >= 1 and step >= cols * 3.
+ * Pinned and pageable frames may be mixed.  crf_analyze_faces, crf_analyze_batch and the crops calls are this call on equal-size frames. */
+int crf_analyze_batch_mixed(crf_ctx* ctx, const crf_image_t* images, int n_images, const crf_rect_t* boxes, const int* image_of_box, int n,
+                            crf_face_t* out);
 /* n equal-size crops stored back to back (n x rows x cols x 3), box = whole crop. */
 int crf_analyze_crops(crf_ctx* ctx, const uint8_t* bgr_batch, int n, int rows, int cols, crf_face_t* out);
 /* stop after getHeadPoseVotesMT (src/face_utils.cpp:183-242): fills headpose, variance, scaled_*, scale. */
@@ -197,13 +204,19 @@ int crf_detect_faces(crf_ctx* ctx, const crf_cascade* c, const uint8_t* bgr, int
                      int min_neighbors, int min_size, crf_rect_t* out, int cap);
 /* detectMultiScale on n_images equal-size frames in one call.  Boxes are grouped by frame in frame order; within a frame they are
  * exactly what crf_detect_faces returns for that frame, in the same order.  image_of_box[i] = frame of box i.
- * Each frame crosses PCIe once.  Frames are processed in groups of at most 64 (fewer when half the context's work budget, min(64 GB,
- * half the free memory), cannot hold 64); each pyramid level, cascade stage group and scan step of a group is one launch.
+ * Each frame crosses PCIe once.  Frames are processed in groups of consecutive frames: at most 64, no more than half the context's work
+ * budget (min(64 GB, half the free memory)) holds, and fewer than 2^32 windows.  A group is a table of (frame, pyramid level)
+ * instances; each pyramid pass, cascade stage group and scan step of a group is one launch over all of them.
  * cap smaller than the box count: every frame is still searched, the true count is returned and the first `cap` boxes are written
  * (cap = 0 sizes a buffer).  Returns the total box count or a negative status. */
 int crf_detect_faces_batch(crf_ctx* ctx, const crf_cascade* c, const uint8_t* const* images, int n_images, int rows, int cols,
                            size_t step, double scale_factor, int min_neighbors, int min_size,
                            crf_rect_t* out, int* image_of_box, int cap);
+/* crf_detect_faces_batch on frames of any sizes (photo collections, mixed camera feeds), in one call.  Every descriptor needs a non-null
+ * bgr, rows, cols >= 1 and step >= cols * 3.  A frame smaller than every window returns no boxes.  crf_detect_faces and
+ * crf_detect_faces_batch are this call on equal-size frames. */
+int crf_detect_faces_batch_mixed(crf_ctx* ctx, const crf_cascade* c, const crf_image_t* images, int n_images, double scale_factor,
+                                 int min_neighbors, int min_size, crf_rect_t* out, int* image_of_box, int cap);
 /* FaceForest::analyzeImage(img, faces) for n_images frames: detection as above, detectFace's enlargement + clipping
  * (src/FaceForest.cpp:147-157), then analyzeFace for every box, reading the frames from the device copy made for detection (no second
  * upload).  boxes (the enlarged boxes) / image_of_box / out: cap entries, in the order of crf_detect_faces_batch.
@@ -214,6 +227,10 @@ int crf_detect_faces_batch(crf_ctx* ctx, const crf_cascade* c, const uint8_t* co
 int crf_analyze_images(crf_ctx* ctx, const crf_cascade* c, const uint8_t* const* images, int n_images, int rows, int cols,
                        size_t step, double scale_factor, int min_neighbors, int min_size,
                        crf_rect_t* boxes, int* image_of_box, crf_face_t* out, int cap);
+/* crf_analyze_images on frames of any sizes (descriptors as in crf_detect_faces_batch_mixed): each detection is enlarged, clipped and
+ * checked against its own frame.  crf_analyze_images is this call on equal-size frames. */
+int crf_analyze_images_mixed(crf_ctx* ctx, const crf_cascade* c, const crf_image_t* images, int n_images, double scale_factor,
+                             int min_neighbors, int min_size, crf_rect_t* boxes, int* image_of_box, crf_face_t* out, int cap);
 
 /* ---- several GPUs behind one caller (SURVEY 8e): one context + one host thread per GPU, contiguous shards of the faces (cut at frame
  * boundaries when the boxes are grouped by frame), a forest replica per GPU, records written straight into `out`.  No collective:
@@ -226,6 +243,9 @@ int crf_multi_device_count(const crf_multi* mg);
 crf_ctx* crf_multi_ctx(crf_multi* mg, int i);   /* shard i's context (counters, profiling) */
 int crf_multi_analyze_batch(crf_multi* mg, const uint8_t* const* images, int n_images, int rows, int cols, size_t step,
                             const crf_rect_t* boxes, const int* image_of_box, int n, crf_face_t* out);
+/* crf_multi_analyze_batch on frames of any sizes (descriptors as in crf_analyze_batch_mixed) */
+int crf_multi_analyze_batch_mixed(crf_multi* mg, const crf_image_t* images, int n_images, const crf_rect_t* boxes, const int* image_of_box,
+                                  int n, crf_face_t* out);
 int crf_multi_analyze_crops(crf_multi* mg, const uint8_t* bgr_batch, int n, int rows, int cols, crf_face_t* out, int headpose_only);
 
 /* ---- stage-level entry points (device results copied back) used by the parity tests and by the

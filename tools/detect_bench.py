@@ -3,11 +3,14 @@
   (a) per frame: crf_detect_faces, detectFace's enlargement on the host, crf_analyze_faces on the boxes the analysis path takes
   (b) crf_detect_faces_batch on all frames of a resolution in one call
   (c) crf_analyze_images on the same frames in one call
+  (d) crf_detect_faces_batch_mixed and crf_analyze_images_mixed on all frames of the set in one call, whatever their sizes
 plus the latency of crf_detect_faces on one frame, and (b) for a few cascade stage-group splits (CRF_HAAR_SPLIT).  Frames: the C3 set
-(workloads.make_frames, 64 x 1080p) and the C5 mixed-resolution set (workloads.make_mixed, one call per resolution); whether their faces
-are LFW-based or procedural is in the output's `data`.  Every call ends in a device synchronise, so host clocks time the whole call.
-With --lib pointing at the library of an earlier build, only the entry points that build has are measured ((a) and the single-frame
-latency), to give the "before" numbers on the same frames.
+(workloads.make_frames, 64 x 1080p), the C5 mixed-resolution set (workloads.make_mixed: 5 sizes, so (b) and (c) make one call per
+resolution) and the R64 set (workloads.make_ragged: 64 distinct sizes, so (b) and (c) go frame by frame); whether their faces are
+LFW-based or procedural is in the output's `data`.  C5 with its boxes given: one crf_analyze_faces call per image against one
+crf_analyze_batch_mixed call.  Every call ends in a device synchronise, so host clocks time the whole call.
+With --lib pointing at the library of an earlier build, entry points that build lacks are skipped, to give the "before" numbers on the
+same frames.
 
   python tools/detect_bench.py [--lib path/to/libcrf_b200.so] [--reps 3] [--out detect_bench.json]
 """
@@ -34,6 +37,14 @@ class Rect(C.Structure):
     _fields_ = [("x", C.c_int), ("y", C.c_int), ("width", C.c_int), ("height", C.c_int)]
 
 
+class Image(C.Structure):
+    _fields_ = [("bgr", C.c_void_p), ("rows", C.c_int), ("cols", C.c_int), ("step", C.c_size_t)]
+
+
+def images(frames):
+    return (Image * len(frames))(*[Image(f.ctypes.data, f.shape[0], f.shape[1], f.strides[0]) for f in frames])
+
+
 def load(path: str):
     L = C.CDLL(path)
     vp = C.c_void_p
@@ -50,6 +61,10 @@ def load(path: str):
                                              C.POINTER(Rect), vp, C.c_int]
         L.crf_analyze_images.argtypes = [vp, vp, C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_double, C.c_int, C.c_int,
                                          C.POINTER(Rect), vp, vp, C.c_int]
+    if hasattr(L, "crf_detect_faces_batch_mixed"):
+        L.crf_detect_faces_batch_mixed.argtypes = [vp, vp, C.POINTER(Image), C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(Rect), vp, C.c_int]
+        L.crf_analyze_images_mixed.argtypes = [vp, vp, C.POINTER(Image), C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(Rect), vp, vp, C.c_int]
+        L.crf_analyze_batch_mixed.argtypes = [vp, C.POINTER(Image), C.c_int, C.POINTER(Rect), vp, C.c_int, vp]
     return L
 
 
@@ -111,6 +126,44 @@ def batch_analyze(L, ctx, cas, frames):
     return n, time.perf_counter() - t0
 
 
+def mixed_detect(L, ctx, cas, frames):
+    im = images(frames)
+    t0 = time.perf_counter()
+    n = check(L, L.crf_detect_faces_batch_mixed(ctx, cas, im, len(frames), SF, MN, MS, None, None, 0))
+    return n, time.perf_counter() - t0
+
+
+def mixed_analyze(L, ctx, cas, frames):
+    im = images(frames)
+    cap = 64 * len(frames)
+    boxes, iob, rec = (Rect * cap)(), np.zeros(cap, np.int32), np.zeros(cap * RECORD, np.uint8)
+    t0 = time.perf_counter()
+    n = check(L, L.crf_analyze_images_mixed(ctx, cas, im, len(frames), SF, MN, MS, boxes, iob.ctypes.data, rec.ctypes.data, cap))
+    return n, time.perf_counter() - t0
+
+
+def boxes_per_image(L, ctx, data):
+    """C5 with boxes given, one crf_analyze_faces call per image: (faces, seconds)"""
+    rec = np.zeros(64 * RECORD, np.uint8)
+    t0 = time.perf_counter()
+    for f, b in data:
+        rb = (Rect * len(b))(*[Rect(*map(int, x)) for x in b])
+        check(L, L.crf_analyze_faces(ctx, f.ctypes.data, f.shape[0], f.shape[1], f.strides[0], rb, len(b), rec.ctypes.data))
+    return sum(len(b) for _, b in data), time.perf_counter() - t0
+
+
+def boxes_one_call(L, ctx, data):
+    """C5 with boxes given, all images in one crf_analyze_batch_mixed call: (faces, seconds)"""
+    frames = [f for f, _ in data]
+    rb = [Rect(*map(int, x)) for _, b in data for x in b]
+    iob = np.array([k for k, (_, b) in enumerate(data) for _ in b], np.int32)
+    rects, rec = (Rect * len(rb))(*rb), np.zeros(len(rb) * RECORD, np.uint8)
+    im = images(frames)
+    t0 = time.perf_counter()
+    check(L, L.crf_analyze_batch_mixed(ctx, im, len(frames), rects, iob.ctypes.data, len(rb), rec.ctypes.data))
+    return len(rb), time.perf_counter() - t0
+
+
 def med(fn, reps):
     """fn() -> (value..., seconds); median of the seconds over reps runs after one warm-up run"""
     fn()
@@ -140,6 +193,7 @@ def main():
 
     L = load(a.lib)
     batched = hasattr(L, "crf_detect_faces_batch")
+    ragged = hasattr(L, "crf_detect_faces_batch_mixed")
     vp = C.c_void_p
     model = vp()
     packed = wl.staged_model_path()
@@ -165,10 +219,13 @@ def main():
     c3, _, _, tag = wl.make_frames(a.frames, 1080, 1920, 16)
     c3 = [np.ascontiguousarray(f) for f in c3]
     mixed, _ = wl.make_mixed(64)
+    mixed = [(np.ascontiguousarray(f), b) for f, b in mixed]
     by_res = {}
     for fr, _ in mixed:
-        by_res.setdefault(fr.shape[:2], []).append(np.ascontiguousarray(fr))
-    res = {"gpu": gpu_info(), "library": "this build" if batched else "earlier build (--lib)", "data": tag, "model": model_tag, "cascade": xml.name, "reps": a.reps,
+        by_res.setdefault(fr.shape[:2], []).append(fr)
+    r64 = [(np.ascontiguousarray(f), b) for f, b in wl.make_ragged(64)]
+    this_build = Path(a.lib).resolve() == (ROOT / "face_alignment_cvpr_2012_b200" / "_lib" / "libcrf_b200.so").resolve()
+    res = {"gpu": gpu_info(), "library": "this build" if this_build else "earlier build (--lib)", "data": tag, "model": model_tag, "cascade": xml.name, "reps": a.reps,
            "params": {"scale_factor": SF, "min_neighbors": MN, "min_size": MS}, "sets": {}}
 
     def run_set(name, groups):
@@ -185,11 +242,26 @@ def main():
             fc = [med(lambda g=g: batch_analyze(L, ctx, cas, g), a.reps) for g in groups]
             n, t = sum(v[0] for v in fc), sum(v[1] for v in fc)
             row["c_analyze_images"] = {"faces_found": n, "frames_per_s": nfr / t, "ms_per_frame": 1e3 * t / nfr}
+        if ragged:
+            frames = [f for g in groups for f in g]
+            n, t = med(lambda: mixed_detect(L, ctx, cas, frames), a.reps)
+            row["d_detect_mixed_one_call"] = {"faces_found": n, "frames_per_s": nfr / t, "detect_ms_per_frame": 1e3 * t / nfr}
+            n, t = med(lambda: mixed_analyze(L, ctx, cas, frames), a.reps)
+            row["d_analyze_images_mixed_one_call"] = {"faces_found": n, "frames_per_s": nfr / t, "ms_per_frame": 1e3 * t / nfr}
         res["sets"][name] = row
         print(name, json.dumps(row), flush=True)
 
     run_set(f"C3_{a.frames}x1080p", [c3])
     run_set("C5_mixed_64", list(by_res.values()))
+    run_set("R64_ragged_64", [[f] for f, _ in r64])
+    given = {}
+    n, t = med(lambda: boxes_per_image(L, ctx, mixed), a.reps)
+    given["per_image_analyze_faces"] = {"faces": n, "faces_per_s": n / t, "ms_per_call_set": 1e3 * t}
+    if ragged:
+        n, t = med(lambda: boxes_one_call(L, ctx, mixed), a.reps)
+        given["one_call_analyze_batch_mixed"] = {"faces": n, "faces_per_s": n / t, "ms_per_call_set": 1e3 * t}
+    res["C5_boxes_given"] = given
+    print("C5 boxes given", json.dumps(given), flush=True)
     out = (Rect * 4096)()
     f0 = c3[0]
     lat = []
