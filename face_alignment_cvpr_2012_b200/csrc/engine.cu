@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <memory>
+#include <sstream>
 #include <string>
 #include <thread>
 #include <unordered_map>
@@ -198,8 +199,9 @@ struct crf_ctx {
   size_t work_budget = (size_t)64 << 30;  // bytes of work buffers a launch may use (min(64 GB, half of the free memory at creation))
   StageTimer timer;
   // face-box source (haar.cuh): device image of the last cascade used + the buffers of a group of frames
-  unsigned long long haar_cached = 0;   // crf_cascade::id of the cascade in d_haar_stages / weak / feats (0 = none)
-  Buf d_haar_stages, d_haar_weak, d_haar_feats, d_haar_frames, d_haar_S, d_haar_Q, d_haar_flags, d_haar_list[2], d_haar_rows, d_haar_levels, d_haar_counts, d_haar_cand;
+  unsigned long long haar_cached = 0;   // crf_cascade::id of the cascade in d_haar_stages / weak / feats / nodes / leaves / tilt (0 = none)
+  // d_haar_weak: HaarWeak of a stump cascade or HaarTree of a tree cascade; d_haar_T: tilted integrals, for cascades with tilted features
+  Buf d_haar_stages, d_haar_weak, d_haar_feats, d_haar_nodes, d_haar_leaves, d_haar_tilt, d_haar_T, d_haar_frames, d_haar_S, d_haar_Q, d_haar_flags, d_haar_list[2], d_haar_rows, d_haar_levels, d_haar_counts, d_haar_cand;
   // first stage of each cascade stage group after the first (CRF_HAAR_SPLIT="a,b,..."; measured, DESIGN §4.5)
   std::vector<int> haar_split{3, 8};
 };
@@ -980,16 +982,28 @@ static int detect_frames(crf_ctx* c, const crf_cascade* cas, const crf_image_t* 
   c->w = &c->ws[0];
   cudaStream_t s = c->w->stream;
   int rc;
+  // the kernel variant follows what the cascade holds: stumps or trees, upright features only or some tilted ones
+  const bool tree = K.is_tree(), tilt = K.has_tilted;
   if (c->haar_cached != cas->id) {
-    if ((rc = upload(c->d_haar_stages, K.stages, s)) || (rc = upload(c->d_haar_weak, K.weak, s)) || (rc = upload(c->d_haar_feats, K.features, s))) return rc;
+    if ((rc = upload(c->d_haar_stages, K.stages, s)) || (rc = upload(c->d_haar_feats, K.features, s))) return rc;
+    if (tree ? (rc = upload(c->d_haar_weak, K.trees, s)) || (rc = upload(c->d_haar_nodes, K.nodes, s)) || (rc = upload(c->d_haar_leaves, K.leaves, s))
+             : (rc = upload(c->d_haar_weak, K.weak, s)))
+      return rc;
+    if (tilt && (rc = upload(c->d_haar_tilt, K.tilted, s))) return rc;
     c->haar_cached = cas->id;
   }
-  const HaarDev dev{c->d_haar_stages.as<HaarStage>(), c->d_haar_weak.as<HaarWeak>(), c->d_haar_feats.as<HaarFeature>(), (int)K.stages.size(), K.win_w, K.win_h};
+  const HaarDev dev{c->d_haar_stages.as<HaarStage>(), tree ? nullptr : c->d_haar_weak.as<HaarWeak>(), c->d_haar_feats.as<HaarFeature>(), (int)K.stages.size(), K.win_w, K.win_h,
+                    tree ? c->d_haar_weak.as<HaarTree>() : nullptr, tree ? c->d_haar_nodes.as<HaarNode>() : nullptr, tree ? c->d_haar_leaves.as<float>() : nullptr,
+                    tilt ? c->d_haar_tilt.as<uint8_t>() : nullptr};
+  auto eval_first = tree ? (tilt ? k_haar_eval_first<true, true> : k_haar_eval_first<true, false>) : (tilt ? k_haar_eval_first<false, true> : k_haar_eval_first<false, false>);
+  auto eval_list = tree ? (tilt ? k_haar_eval_list<true, true> : k_haar_eval_list<true, false>) : (tilt ? k_haar_eval_list<false, true> : k_haar_eval_list<false, false>);
   // stage groups: [0, split[0]), [split[0], split[1]), ..., up to the last stage
   std::vector<int> bounds;
   for (int b : c->haar_split) if (b > (bounds.empty() ? 0 : bounds.back()) && b < dev.nstages) bounds.push_back(b);
   bounds.push_back(dev.nstages);
-  auto footprint = [&](int i) { const FramePlan& p = plans[(size_t)i]; return image_bytes(images[i]) + p.nint * 8 + p.nwin * (1 + 2 * sizeof(uint2)) + (size_t)p.nrows * 4; };
+  // integrals: S and Q, plus T for a tilted cascade
+  const size_t int_bytes = tilt ? 12 : 8;
+  auto footprint = [&](int i) { const FramePlan& p = plans[(size_t)i]; return image_bytes(images[i]) + p.nint * int_bytes + p.nwin * (1 + 2 * sizeof(uint2)) + (size_t)p.nrows * 4; };
   std::vector<std::vector<crf_rect_t>> boxes;
   std::vector<int> frame_count;
   for (int f0 = 0, f1; f0 < n_images; f0 = f1) {
@@ -1006,7 +1020,8 @@ static int detect_frames(crf_ctx* c, const crf_cascade* cas, const crf_image_t* 
     std::vector<size_t> off((size_t)nf + 1, 0);
     std::vector<int> frame_rows((size_t)nf + 1, 0);
     size_t io = 0, fo = 0;
-    int nrows = 0, brows = 0, bcols = 0, beval = 0;
+    int nrows = 0, brows = 0, bcols = 0, beval = 0, btilt = 0;
+    std::vector<int> blk_tilt;   // first block of each instance in k_haar_tilted
     for (int k = 0; k < nf; k++) {
       off[(size_t)k + 1] = off[(size_t)k] + image_bytes(images[f0 + k]);
       for (HaarInst L : plans[(size_t)(f0 + k)].levels) {
@@ -1017,24 +1032,27 @@ static int detect_frames(crf_ctx* c, const crf_cascade* cas, const crf_image_t* 
         L.blk_rows = brows; brows += (L.sh + 7) / 8;
         L.blk_cols = bcols; bcols += (L.sw + 1 + 31) / 32;
         L.blk_eval = beval; beval += (L.nx + 127) / 128 * L.ny;
+        if (tilt) { blk_tilt.push_back(btilt); btilt += 2 * ((L.sw + L.sh + 31) / 32); }
         inst.push_back(L);
       }
       frame_rows[(size_t)k + 1] = nrows;
     }
     if (!inst.empty()) {
       const int ninst = (int)inst.size();
-      // one upload: the instances, then the frames' row ranges, then the search keys (HaarKeys)
+      // one upload: the instances, then the frames' row ranges, then the search keys (HaarKeys, then blk_tilt for a tilted cascade)
       const size_t tab = ((size_t)ninst * sizeof(HaarInst) + 15) & ~(size_t)15;
       std::vector<int> ints(frame_rows);
       for (int k = 0; k < 5; k++)
         for (const HaarInst& L : inst)
           ints.push_back(k == 0 ? L.blk_rows : k == 1 ? L.blk_cols : k == 2 ? L.blk_eval : k == 3 ? L.row_off : (int)(unsigned)L.flag_off);
+      ints.insert(ints.end(), blk_tilt.begin(), blk_tilt.end());
       std::vector<uint8_t> table(tab + ints.size() * sizeof(int));
       std::memcpy(table.data(), inst.data(), (size_t)ninst * sizeof(HaarInst));
       std::memcpy(table.data() + tab, ints.data(), ints.size() * sizeof(int));
       if ((rc = c->d_haar_frames.reserve(off[(size_t)nf])) || (rc = c->d_haar_S.reserve(io * 4)) || (rc = c->d_haar_Q.reserve(io * 4)) ||
           (rc = c->d_haar_flags.reserve(fo)) || (rc = c->d_haar_list[0].reserve(fo * sizeof(uint2))) || (rc = c->d_haar_list[1].reserve(fo * sizeof(uint2))) ||
-          (rc = c->d_haar_rows.reserve((size_t)nrows * 4)) || (rc = c->d_haar_counts.reserve((size_t)(kDetectGroupFrames + 4) * 4)))
+          (rc = c->d_haar_rows.reserve((size_t)nrows * 4)) || (rc = c->d_haar_counts.reserve((size_t)(kDetectGroupFrames + 4) * 4)) ||
+          (tilt && (rc = c->d_haar_T.reserve(io * 4))))
         return rc;
       if ((rc = upload_frames(c, images, f0, nf, off, s))) return rc;
       if ((rc = upload(c->d_haar_levels, table, s))) return rc;
@@ -1049,14 +1067,23 @@ static int detect_frames(crf_ctx* c, const crf_cascade* cas, const crf_image_t* 
       uint32_t* Q = c->d_haar_Q.as<uint32_t>();
       uint8_t* flags = c->d_haar_flags.as<uint8_t>();
       uint2* list[2] = {c->d_haar_list[0].as<uint2>(), c->d_haar_list[1].as<uint2>()};
-      k_haar_rows<<<brows, 256, 0, s>>>(d_inst, keys, ninst, c->d_haar_frames.as<uint8_t>(), S, Q);
+      uint32_t* T = tilt ? c->d_haar_T.as<uint32_t>() : nullptr;
+      if (tilt) {
+        // the tilted integrals from the row prefixes k_haar_rows leaves in S, before k_haar_cols turns them into the integrals
+        k_haar_rows<true><<<brows, 256, 0, s>>>(d_inst, keys, ninst, c->d_haar_frames.as<uint8_t>(), S, Q, T);
+        k_haar_tilted<<<btilt, dim3(32, 32), 0, s>>>(d_inst, d_key + 5 * ninst, ninst, S, T);
+        KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 2);
+      } else {
+        k_haar_rows<false><<<brows, 256, 0, s>>>(d_inst, keys, ninst, c->d_haar_frames.as<uint8_t>(), S, Q, nullptr);
+        KCHECK(); count_launch(c, CRF_STAGE_RESIZE);
+      }
       k_haar_cols<<<bcols, dim3(32, 32), 0, s>>>(d_inst, keys, ninst, S, Q);
-      k_haar_eval_first<<<beval, 128, 0, s>>>(d_inst, keys, ninst, S, Q, dev, bounds[0], flags, list[0], lists_n);
-      KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 3);
+      eval_first<<<beval, 128, 0, s>>>(d_inst, keys, ninst, S, Q, T, dev, bounds[0], flags, list[0], lists_n);
+      KCHECK(); count_launch(c, CRF_STAGE_RESIZE, 2);
       for (size_t g = 1; g < bounds.size(); g++) {
         const int in = (int)((g - 1) & 1), out = (int)(g & 1);
         if (g >= 2) CU(cudaMemsetAsync(lists_n + out, 0, sizeof(unsigned), s));
-        k_haar_eval_list<<<c->sm_count * 8, 128, 0, s>>>(d_inst, keys, ninst, S, dev, bounds[g - 1], bounds[g], list[in], lists_n + in, flags, list[out], lists_n + out);
+        eval_list<<<c->sm_count * 8, 128, 0, s>>>(d_inst, keys, ninst, S, T, dev, bounds[g - 1], bounds[g], list[in], lists_n + in, flags, list[out], lists_n + out);
         KCHECK(); count_launch(c, CRF_STAGE_RESIZE);
       }
       int* d_rows = c->d_haar_rows.as<int>();
@@ -1149,7 +1176,7 @@ int crf_cascade_info(const crf_cascade* c, int* win_w, int* win_h, int* nstages,
   if (win_w) *win_w = c->c.win_w;
   if (win_h) *win_h = c->c.win_h;
   if (nstages) *nstages = (int)c->c.stages.size();
-  if (nweak) *nweak = (int)c->c.weak.size();
+  if (nweak) *nweak = c->c.nweak();
   return CRF_OK;
 }
 
@@ -1471,7 +1498,7 @@ void crf_ctx_destroy(crf_ctx* c) {
   if (c->tex_mp_wide) cudaDestroyTextureObject(c->tex_mp_wide);
   Buf* all[] = {&c->d_hp_slotsn, &c->d_mp_slotsn, &c->d_hp_nroot, &c->d_mp_nroot, &c->d_hp_slotsw, &c->d_mp_slotsw, &c->d_hp_slots16, &c->d_mp_slots16, &c->d_hp_slots, &c->d_hp_roots, &c->d_hp_m, &c->d_mp_slots, &c->d_mp_roots, &c->d_mp_mask, &c->d_mp_leaf, &c->d_xs, &c->d_coef[0], &c->d_coef[1],
                 &c->d_coef[2], &c->d_coef[3], &c->d_coef[4], &c->d_coef_sep[1], &c->d_coef_sep[2], &c->d_coef_sep[3], &c->d_coef_sep[4], &c->d_imgs[0], &c->d_imgs[1], &c->d_fd, &c->d_faces, &c->d_counters, &c->d_misc,
-                &c->d_haar_stages, &c->d_haar_weak, &c->d_haar_feats, &c->d_haar_frames, &c->d_haar_S, &c->d_haar_Q, &c->d_haar_flags, &c->d_haar_list[0],
+                &c->d_haar_stages, &c->d_haar_weak, &c->d_haar_feats, &c->d_haar_nodes, &c->d_haar_leaves, &c->d_haar_tilt, &c->d_haar_T, &c->d_haar_frames, &c->d_haar_S, &c->d_haar_Q, &c->d_haar_flags, &c->d_haar_list[0],
                 &c->d_haar_list[1], &c->d_haar_rows, &c->d_haar_levels, &c->d_haar_counts, &c->d_haar_cand};
   for (Buf* b : all) b->release();
   for (auto& w : c->ws) {

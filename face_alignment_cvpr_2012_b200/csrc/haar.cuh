@@ -1,6 +1,7 @@
 // Face-box source of FaceForest::detectFace (reference src/FaceForest.cpp:136-159, SURVEY 8 f2):
 // cv::CascadeClassifier::detectMultiScale for the stump-based HAAR cascade the reference ships
-// (data/haarcascade_frontalface_alt.xml, new-format XML), evaluated on the GPU.
+// (data/haarcascade_frontalface_alt.xml, new-format XML), evaluated on the GPU; and for every other HAAR cascade cv::CascadeClassifier
+// loads: tree weak classifiers, 45-degree tilted features (from a tilted integral built only for such cascades), the old XML format.
 //
 // The algorithm is OpenCV's (objdetect/cascadedetect.cpp; not under /root/reference): per scale factor = 1.3^k a bilinear
 // pyramid level of the gray frame, integral images of values and squares, then every window position of the level's
@@ -20,17 +21,32 @@ struct HaarStage { int first, count; float threshold; };
 struct HaarWeak { int feature; float threshold, left, right; };
 struct HaarRect { int x, y, w, h; float weight; };
 struct HaarFeature { HaarRect r[3]; };
+// Tree weak classifiers (OpenCV's predictOrdered): a tree's nodes are nodes[node, node + n), its n + 1 leaves leaves[leaf, leaf + n + 1).
+// A child > 0 is a node of the same tree, a child <= 0 the leaf -child.  The walk starts at node 0 and goes left when value * inv <
+// threshold.  The loader checks that every child index is greater than its parent's, so a walk ends within n steps.
+struct HaarNode { int feature; float threshold; int left, right; };
+struct HaarTree { int node, leaf; };
+constexpr int kHaarMaxTreeNodes = 16;   // nodes per tree accepted by the loader; OpenCV's shipped cascades use at most 3
 
+// A stump cascade (every weak classifier a single node) keeps its weak classifiers in `weak`; a tree cascade keeps them in `trees`,
+// `nodes` and `leaves`, with single-node trees among them.  Stages index whichever is used.
 struct Cascade {
   int win_w = 0, win_h = 0;
   std::vector<HaarStage> stages;
   std::vector<HaarWeak> weak;
+  std::vector<HaarTree> trees;
+  std::vector<HaarNode> nodes;
+  std::vector<float> leaves;
   std::vector<HaarFeature> features;
+  std::vector<uint8_t> tilted;   // per feature: 1 = 45-degree feature, its rects summed from the tilted integral
+  bool has_tilted = false;
+  bool is_tree() const { return !trees.empty(); }
+  int nweak() const { return (int)(is_tree() ? trees.size() : weak.size()); }
 };
 
-// ---- minimal XML reader for OpenCV's FileStorage cascade files: elements with text, no attributes needed ----------------
+// ---- minimal XML reader for OpenCV's FileStorage cascade files: elements with text, the attributes kept as written -------------
 struct XmlNode {
-  std::string name, text;
+  std::string name, attrs, text;
   std::vector<XmlNode> kids;
   const XmlNode* child(const char* n) const { for (auto& k : kids) if (k.name == n) return &k; return nullptr; }
 };
@@ -41,7 +57,9 @@ static bool xml_parse(const std::string& s, size_t& i, XmlNode& out) {
   std::string tag = s.substr(i + 1, e - i - 1);
   const bool self_closing = !tag.empty() && tag.back() == '/';
   if (self_closing) tag.pop_back();
-  out.name = tag.substr(0, tag.find_first_of(" \t\r\n"));
+  const size_t sp = tag.find_first_of(" \t\r\n");
+  out.name = tag.substr(0, sp);
+  if (sp != std::string::npos) out.attrs = tag.substr(sp);
   i = e + 1;
   if (self_closing) return true;
   for (;;) {
@@ -56,6 +74,164 @@ static bool xml_parse(const std::string& s, size_t& i, XmlNode& out) {
   }
 }
 
+// A feature element of either format (<rects> of 2 or 3 "x y w h weight", optional <tilted>) appended to c.features / c.tilted.
+// An upright rect lies in the window; a tilted one (corners (x, y), (x + w, y + w), (x - h, y + h), (x + w - h, y + w + h)) too.
+static int parse_feature(const XmlNode& ft, Cascade& c, std::string& err) {
+  HaarFeature hf{};
+  const bool tilt = ft.child("tilted") && std::atoi(ft.child("tilted")->text.c_str()) != 0;
+  const XmlNode* rects = ft.child("rects");
+  if (!rects || rects->kids.empty() || rects->kids.size() > 3) { err = "feature with an unsupported rectangle count"; return CRF_ERR_FORMAT; }
+  for (size_t k = 0; k < rects->kids.size(); k++) {
+    double v[5] = {0, 0, 0, 0, 0};
+    if (std::sscanf(rects->kids[k].text.c_str(), "%lf %lf %lf %lf %lf", &v[0], &v[1], &v[2], &v[3], &v[4]) != 5) { err = "bad feature rectangle"; return CRF_ERR_FORMAT; }
+    const HaarRect r{(int)v[0], (int)v[1], (int)v[2], (int)v[3], (float)v[4]};
+    const bool inside = tilt ? r.x - r.h >= 0 && r.y >= 0 && r.w >= 1 && r.h >= 1 && r.x + r.w <= c.win_w && r.y + r.w + r.h <= c.win_h
+                             : r.x >= 0 && r.y >= 0 && r.w >= 1 && r.h >= 1 && r.x + r.w <= c.win_w && r.y + r.h <= c.win_h;
+    if (!inside) { err = "feature rectangle outside the window"; return CRF_ERR_FORMAT; }
+    hf.r[k] = r;
+  }
+  c.features.push_back(hf);
+  c.tilted.push_back(tilt ? 1 : 0);
+  c.has_tilted |= tilt;
+  return CRF_OK;
+}
+
+// One weak classifier as read, before it is stored as a stump or a tree.
+struct HaarWeakIn { std::vector<HaarNode> nodes; std::vector<float> leaves; };
+
+// Checks every tree (so that no malformed tree reaches a kernel: the device walk trusts these rules) and stores the cascade: as stumps
+// when every weak classifier has one node, else as trees.
+static int finish_cascade(Cascade& c, const std::vector<float>& stage_thr, const std::vector<std::vector<HaarWeakIn>>& stage_weak, std::string& err) {
+  bool stumps = true;
+  for (const auto& ws : stage_weak)
+    for (const HaarWeakIn& w : ws) {
+      const int n = (int)w.nodes.size();
+      if (n < 1 || n > kHaarMaxTreeNodes) { err = "tree with an unsupported node count (1 to " + std::to_string(kHaarMaxTreeNodes) + ")"; return CRF_ERR_FORMAT; }
+      if ((int)w.leaves.size() != n + 1) { err = "tree without nodes + 1 leaves"; return CRF_ERR_FORMAT; }
+      std::vector<uint8_t> reached((size_t)n, 0);
+      reached[0] = 1;
+      for (int k = 0; k < n; k++) {
+        const HaarNode& nd = w.nodes[(size_t)k];
+        if (nd.feature < 0 || nd.feature >= (int)c.features.size()) { err = "weak classifier names a missing feature"; return CRF_ERR_FORMAT; }
+        for (const int ch : {nd.left, nd.right}) {
+          if (ch > 0) {
+            if (ch <= k || ch >= n) { err = "tree node whose child does not follow it"; return CRF_ERR_FORMAT; }
+            reached[(size_t)ch] = 1;
+          } else if (-ch > n) { err = "tree leaf index out of range"; return CRF_ERR_FORMAT; }
+        }
+      }
+      for (int k = 1; k < n; k++)
+        if (!reached[(size_t)k]) { err = "tree with an unreachable node"; return CRF_ERR_FORMAT; }
+      stumps &= n == 1;
+    }
+  for (size_t si = 0; si < stage_weak.size(); si++) {
+    HaarStage hs{stumps ? (int)c.weak.size() : (int)c.trees.size(), (int)stage_weak[si].size(), stage_thr[si]};
+    for (const HaarWeakIn& w : stage_weak[si]) {
+      if (stumps) {
+        const HaarNode& nd = w.nodes[0];
+        c.weak.push_back(HaarWeak{nd.feature, nd.threshold, w.leaves[(size_t)-nd.left], w.leaves[(size_t)-nd.right]});
+      } else {
+        c.trees.push_back(HaarTree{(int)c.nodes.size(), (int)c.leaves.size()});
+        c.nodes.insert(c.nodes.end(), w.nodes.begin(), w.nodes.end());
+        c.leaves.insert(c.leaves.end(), w.leaves.begin(), w.leaves.end());
+      }
+    }
+    c.stages.push_back(hs);
+  }
+  if (c.stages.empty() || c.win_w < 3 || c.win_h < 3) { err = "empty cascade"; return CRF_ERR_FORMAT; }
+  return CRF_OK;
+}
+
+// New format (<cascade type_id="opencv-cascade-classifier">): features in one list, weak classifiers as <internalNodes> (left right
+// featureIdx threshold per node) and <leafValues>.
+static int load_new_format(const XmlNode& cas, Cascade& c, std::string& err) {
+  if (cas.child("featureType") && cas.child("featureType")->text.find("HAAR") == std::string::npos) { err = "only HAAR cascades are supported"; return CRF_ERR_UNSUPPORTED; }
+  const XmlNode* fp = cas.child("featureParams");
+  if (fp && fp->child("maxCatCount") && std::atoi(fp->child("maxCatCount")->text.c_str()) > 0) { err = "categorical (maxCatCount > 0) cascades are not supported"; return CRF_ERR_UNSUPPORTED; }
+  c.win_w = std::atoi(cas.child("width")->text.c_str());
+  c.win_h = std::atoi(cas.child("height")->text.c_str());
+  int rc;
+  for (const XmlNode& ft : cas.child("features")->kids)
+    if ((rc = parse_feature(ft, c, err))) return rc;
+  std::vector<float> thr;
+  std::vector<std::vector<HaarWeakIn>> weak;
+  for (const XmlNode& st : cas.child("stages")->kids) {
+    const XmlNode* t = st.child("stageThreshold");
+    const XmlNode* wcs = st.child("weakClassifiers");
+    if (!t || !wcs) { err = "stage without threshold / classifiers"; return CRF_ERR_FORMAT; }
+    thr.push_back((float)std::atof(t->text.c_str()));
+    weak.emplace_back();
+    for (const XmlNode& wc : wcs->kids) {
+      const XmlNode* in = wc.child("internalNodes");
+      const XmlNode* lv = wc.child("leafValues");
+      if (!in || !lv) { err = "bad weak classifier"; return CRF_ERR_FORMAT; }
+      HaarWeakIn w;
+      std::istringstream ns(in->text), ls(lv->text);
+      std::vector<double> v;
+      for (double x; ns >> x;) v.push_back(x);
+      if (!ns.eof() || v.empty() || v.size() % 4) { err = "bad weak classifier"; return CRF_ERR_FORMAT; }
+      for (size_t k = 0; k < v.size(); k += 4) {
+        if (v[k] != std::floor(v[k]) || v[k + 1] != std::floor(v[k + 1]) || v[k + 2] != std::floor(v[k + 2]) || std::fabs(v[k]) > 1e6 || std::fabs(v[k + 1]) > 1e6 ||
+            std::fabs(v[k + 2]) > 1e9) { err = "bad weak classifier"; return CRF_ERR_FORMAT; }
+        w.nodes.push_back(HaarNode{(int)v[k + 2], (float)v[k + 3], (int)v[k], (int)v[k + 1]});
+      }
+      for (double x; ls >> x;) w.leaves.push_back((float)x);
+      if (!ls.eof()) { err = "bad weak classifier"; return CRF_ERR_FORMAT; }
+      weak.back().push_back(std::move(w));
+    }
+  }
+  return finish_cascade(c, thr, weak, err);
+}
+
+// Old format (<name type_id="opencv-haar-classifier">): <size>, stages of <trees> (nodes with an inline <feature>, <threshold> and
+// left_val | left_node, right_val | right_node), <stage_threshold>, <parent>, <next>.  Converted the way OpenCV converts it: one feature
+// per node, a tree's leaves numbered in node order, left before right.  Only a chain of stages (parent = previous, no next) is accepted.
+static int load_old_format(const XmlNode& cas, Cascade& c, std::string& err) {
+  const XmlNode* size = cas.child("size");
+  const XmlNode* stages = cas.child("stages");
+  if (!size || !stages || std::sscanf(size->text.c_str(), "%d %d", &c.win_w, &c.win_h) != 2) { err = "old-format cascade without <size> / <stages>"; return CRF_ERR_FORMAT; }
+  std::vector<float> thr;
+  std::vector<std::vector<HaarWeakIn>> weak;
+  int rc;
+  for (const XmlNode& st : stages->kids) {
+    const int si = (int)thr.size();
+    const XmlNode* trees = st.child("trees");
+    const XmlNode* t = st.child("stage_threshold");
+    if (!trees || !t) { err = "stage without threshold / trees"; return CRF_ERR_FORMAT; }
+    const XmlNode* parent = st.child("parent");
+    const XmlNode* next = st.child("next");
+    if ((parent && std::atoi(parent->text.c_str()) != si - 1) || (next && std::atoi(next->text.c_str()) != -1)) {
+      err = "old-format cascade whose stages do not form a chain"; return CRF_ERR_UNSUPPORTED;
+    }
+    thr.push_back((float)std::atof(t->text.c_str()));
+    weak.emplace_back();
+    for (const XmlNode& tree : trees->kids) {
+      HaarWeakIn w;
+      for (const XmlNode& node : tree.kids) {
+        const XmlNode* ft = node.child("feature");
+        const XmlNode* th = node.child("threshold");
+        if (!ft || !th) { err = "tree node without feature / threshold"; return CRF_ERR_FORMAT; }
+        if ((rc = parse_feature(*ft, c, err))) return rc;
+        HaarNode nd{(int)c.features.size() - 1, (float)std::atof(th->text.c_str()), 0, 0};
+        for (int side = 0; side < 2; side++) {
+          const XmlNode* val = node.child(side ? "right_val" : "left_val");
+          const XmlNode* idx = node.child(side ? "right_node" : "left_node");
+          int ch;
+          if (val) { ch = -(int)w.leaves.size(); w.leaves.push_back((float)std::atof(val->text.c_str())); }
+          else if (idx) ch = std::atoi(idx->text.c_str());
+          else { err = "tree node without a left / right child"; return CRF_ERR_FORMAT; }
+          (side ? nd.right : nd.left) = ch;
+        }
+        w.nodes.push_back(nd);
+      }
+      weak.back().push_back(std::move(w));
+    }
+  }
+  return finish_cascade(c, thr, weak, err);
+}
+
+// OpenCV's HAAR cascades as cv::CascadeClassifier::load reads them: the new format with stump or tree weak classifiers, upright and
+// tilted features, and the old opencv-haar-classifier format.  LBP / HOG features, categorical splits and stage trees are rejected.
 static int load_cascade(const std::string& path, Cascade& c, std::string& err) {
   FILE* f = std::fopen(path.c_str(), "rb");
   if (!f) { err = "File not found: " + path; return CRF_ERR_IO; }
@@ -68,44 +244,11 @@ static int load_cascade(const std::string& path, Cascade& c, std::string& err) {
   XmlNode root;
   if (i == std::string::npos || !xml_parse(s, i, root)) { err = "not an OpenCV cascade file: " + path; return CRF_ERR_FORMAT; }
   const XmlNode* cas = root.child("cascade");
-  if (!cas || !cas->child("stages") || !cas->child("features") || !cas->child("width") || !cas->child("height")) {
-    err = "unsupported cascade layout (expected the new-format opencv-cascade-classifier): " + path; return CRF_ERR_FORMAT;
-  }
-  if (cas->child("featureType") && cas->child("featureType")->text.find("HAAR") == std::string::npos) { err = "only HAAR cascades are supported"; return CRF_ERR_UNSUPPORTED; }
-  c.win_w = std::atoi(cas->child("width")->text.c_str());
-  c.win_h = std::atoi(cas->child("height")->text.c_str());
-  for (const XmlNode& ft : cas->child("features")->kids) {
-    HaarFeature hf{};
-    if (ft.child("tilted") && std::atoi(ft.child("tilted")->text.c_str()) != 0) { err = "tilted features are not supported"; return CRF_ERR_UNSUPPORTED; }
-    const XmlNode* rects = ft.child("rects");
-    if (!rects || rects->kids.empty() || rects->kids.size() > 3) { err = "feature with an unsupported rectangle count"; return CRF_ERR_FORMAT; }
-    for (size_t k = 0; k < rects->kids.size(); k++) {
-      double v[5] = {0, 0, 0, 0, 0};
-      if (std::sscanf(rects->kids[k].text.c_str(), "%lf %lf %lf %lf %lf", &v[0], &v[1], &v[2], &v[3], &v[4]) != 5) { err = "bad feature rectangle"; return CRF_ERR_FORMAT; }
-      hf.r[k] = HaarRect{(int)v[0], (int)v[1], (int)v[2], (int)v[3], (float)v[4]};
-      if (hf.r[k].x < 0 || hf.r[k].y < 0 || hf.r[k].w < 1 || hf.r[k].h < 1 || hf.r[k].x + hf.r[k].w > c.win_w || hf.r[k].y + hf.r[k].h > c.win_h) { err = "feature rectangle outside the window"; return CRF_ERR_FORMAT; }
-    }
-    c.features.push_back(hf);
-  }
-  for (const XmlNode& st : cas->child("stages")->kids) {
-    const XmlNode* thr = st.child("stageThreshold");
-    const XmlNode* wcs = st.child("weakClassifiers");
-    if (!thr || !wcs) { err = "stage without threshold / classifiers"; return CRF_ERR_FORMAT; }
-    HaarStage hs{(int)c.weak.size(), 0, (float)std::atof(thr->text.c_str())};
-    for (const XmlNode& wc : wcs->kids) {
-      const XmlNode* in = wc.child("internalNodes");
-      const XmlNode* lv = wc.child("leafValues");
-      int a = 0, b = 0, fi = 0; double t = 0, l = 0, r = 0;
-      if (!in || !lv || std::sscanf(in->text.c_str(), "%d %d %d %lf", &a, &b, &fi, &t) != 4 || std::sscanf(lv->text.c_str(), "%lf %lf", &l, &r) != 2) { err = "bad weak classifier"; return CRF_ERR_FORMAT; }
-      if (a != 0 || b != -1) { err = "only stump-based cascades are supported"; return CRF_ERR_UNSUPPORTED; }
-      if (fi < 0 || fi >= (int)c.features.size()) { err = "weak classifier names a missing feature"; return CRF_ERR_FORMAT; }
-      c.weak.push_back(HaarWeak{fi, (float)t, (float)l, (float)r});
-      hs.count++;
-    }
-    c.stages.push_back(hs);
-  }
-  if (c.stages.empty() || c.win_w < 3 || c.win_h < 3) { err = "empty cascade"; return CRF_ERR_FORMAT; }
-  return CRF_OK;
+  if (cas && cas->child("stages") && cas->child("features") && cas->child("width") && cas->child("height")) return load_new_format(*cas, c, err);
+  for (const XmlNode& k : root.kids)
+    if (k.attrs.find("opencv-haar-classifier") != std::string::npos) return load_old_format(k, c, err);
+  err = "unsupported cascade layout (expected opencv-cascade-classifier or opencv-haar-classifier): " + path;
+  return CRF_ERR_FORMAT;
 }
 
 // ---- kernels ---------------------------------------------------------------------------------------------------------------
@@ -115,9 +258,11 @@ static int load_cascade(const std::string& path, Cascade& c, std::string& err) {
 //   S, Q   [instance][(sh + 1) x (sw + 1)] u32 integrals of values and squares (pitch sw + 1)
 //   flags  [instance][ny][nx] u8 per window of the level's ystep grid: bit 0 = passed every stage, bit 1 = rejected by stage 0
 //   rows   [instance][iy] candidates per window row, then their offsets within the frame (a frame's rows are contiguous)
+//   T      [instance][(sh + 1) x (sw + 1)] u32 tilted integral, same layout as S (cascades with tilted features only)
 // Each pyramid pass is one launch over every instance of the group; a block finds its instance by binary search on the instance's first
-// block of that launch.  Launches per group: 3 for the pyramid passes, 1 per later stage group, 3 for the scan rule and the candidate
-// compaction, whatever the number, sizes and levels of the frames.
+// block of that launch.  Launches per group: 3 for the pyramid passes (4 with tilted features: k_haar_tilted), 1 per later stage group, 3
+// for the scan rule and the candidate compaction, whatever the number, sizes and levels of the frames.  Tree weak classifiers add none:
+// the evaluation kernels are instantiated for stumps or trees and upright-only or tilted features, picked from the cascade.
 struct HaarInst {
   double factor, scale_x, scale_y;
   int sw, sh, nx, ny, ystep, win_w, win_h;
@@ -130,7 +275,11 @@ struct HaarInst {
   int blk_rows, blk_cols, blk_eval;   // first block of the instance in k_haar_rows / k_haar_cols / k_haar_eval_first
 };
 
-struct HaarDev { const HaarStage* stages; const HaarWeak* weak; const HaarFeature* feats; int nstages, win_w, win_h; };
+// weak: the stumps of a stump cascade; trees / nodes / leaves: those of a tree cascade; tilt: per feature, for a cascade with tilted features
+struct HaarDev {
+  const HaarStage* stages; const HaarWeak* weak; const HaarFeature* feats; int nstages, win_w, win_h;
+  const HaarTree* trees; const HaarNode* nodes; const float* leaves; const uint8_t* tilt;
+};
 
 // The search keys of the instance table, one compact array per key (a few KB, so the searches stay in L1): key[i] is the instance's
 // blk_rows / blk_cols / blk_eval / row_off / flag_off.  Each array is sorted, as the table is ordered by every offset.
@@ -169,10 +318,11 @@ __device__ __forceinline__ int haar_level_px(const uint8_t* __restrict__ bgr, co
   return min(max(v, 0), 255);
 }
 
-// Pyramid level fused with the row pass of its integrals: one warp per level row builds the row's pixels and scans them along x.
-// ceil(sh / 8) blocks per instance, 256 threads.
+// Pyramid level fused with the row pass of its integrals: one warp per level row builds the row's pixels and scans them along x.  TILT:
+// also zeroes the level's tilted integral T, which k_haar_tilted accumulates into.  ceil(sh / 8) blocks per instance, 256 threads.
+template <bool TILT>
 __global__ void __launch_bounds__(256) k_haar_rows(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, const uint8_t* __restrict__ frames,
-                                                   uint32_t* __restrict__ S, uint32_t* __restrict__ Q) {
+                                                   uint32_t* __restrict__ S, uint32_t* __restrict__ Q, uint32_t* __restrict__ T) {
   const int b = (int)blockIdx.x;
   const HaarInst L = inst[haar_inst_of(keys.blk_rows, ninst, b)];
   const int y = (b - L.blk_rows) * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -183,6 +333,11 @@ __global__ void __launch_bounds__(256) k_haar_rows(const HaarInst* __restrict__ 
   uint32_t* __restrict__ q = Q + L.int_off;
   if (y == 0) for (size_t x = lane; x < P; x += 32) { s[x] = 0; q[x] = 0; }
   if (lane == 0) { s[(size_t)(y + 1) * P] = 0; q[(size_t)(y + 1) * P] = 0; }
+  if constexpr (TILT) {
+    uint32_t* __restrict__ t = T + L.int_off;
+    if (y == 0) for (size_t x = lane; x < P; x += 32) t[x] = 0;
+    for (size_t x = lane; x < P; x += 32) t[(size_t)(y + 1) * P + x] = 0;
+  }
   uint32_t cs = 0, cq = 0;
   for (int x0 = 0; x0 < L.sw; x0 += 32) {
     const int x = x0 + lane;
@@ -227,27 +382,102 @@ __global__ void __launch_bounds__(1024) k_haar_cols(const HaarInst* __restrict__
     }
 }
 
+// Tilted integral (cv::integral's third output, OpenCV's CV_TILTED_OFS table) of every instance, between k_haar_rows and k_haar_cols,
+// while S still holds the row prefixes R(y, x) = sum_{x' < x} I(y, x') (x in [0, sw]).  With R clamped in x,
+//   T(Y, X) = sum_{y < Y} R(y, clamp(X + Y - 1 - y)) - R(y, clamp(X - Y + y)),
+// a prefix sum down each anti-diagonal d = X + Y - 1 minus one down each diagonal e = X - Y.  A CTA owns 32 (anti-)diagonals, its 32
+// warps 32 chunks of rows; a warp reads adjacent x of one row.  As in k_haar_cols the chunk totals are scanned in shared memory and each
+// chunk walked again with its carry; the two families meet in T (zeroed by k_haar_rows) through u32 atomic adds, which are exact
+// modulo 2^32 in any order, so T has the bits of a serial evaluation.  2 x ceil((sw + sh) / 32) blocks per instance from blk_tilt[],
+// the first half anti-diagonals, block (32, 32).
+__global__ void __launch_bounds__(1024) k_haar_tilted(const HaarInst* __restrict__ inst, const int* __restrict__ blk_tilt, int ninst, const uint32_t* __restrict__ S,
+                                                      uint32_t* __restrict__ T) {
+  __shared__ uint32_t ts[32][32];
+  const int b = (int)blockIdx.x;
+  const int li = haar_inst_of(blk_tilt, ninst, b);
+  const HaarInst& L = inst[li];
+  const int W = L.sw, H = L.sh, nb = (W + H + 31) / 32, lb = b - blk_tilt[li];
+  const bool anti = lb < nb;
+  const int tx = threadIdx.x, ty = threadIdx.y, t = (anti ? lb : lb - nb) * 32 + tx;
+  const bool on = t < W + H;
+  const int c0 = anti ? t : t - H;          // d, or e
+  const size_t P = (size_t)W + 1;
+  const uint32_t* __restrict__ r = S + L.int_off + P;   // R(y, x) = r[y * P + x]
+  uint32_t* __restrict__ out = T + L.int_off + P;       // T(y + 1, X) = out[y * P + X]
+  const int R = (H + 31) / 32, y0 = ty * R, y1 = min(H, y0 + R);
+  uint32_t a = 0;
+  if (on)
+    for (int y = y0; y < y1; y++) a += r[(size_t)y * P + min(max(anti ? c0 - y : c0 + y, 0), W)];
+  ts[ty][tx] = a;
+  __syncthreads();
+  uint32_t acc = 0;
+  for (int k = 0; k < ty; k++) acc += ts[k][tx];
+  if (on)
+    for (int y = y0; y < y1; y++) {
+      acc += r[(size_t)y * P + min(max(anti ? c0 - y : c0 + y, 0), W)];
+      const int X = anti ? c0 - y : c0 + y + 1;
+      if (X >= 0 && X <= W) atomicAdd(out + (size_t)y * P + X, anti ? acc : 0u - acc);
+    }
+}
+
 __device__ __forceinline__ uint32_t haar_rectsum(const uint32_t* __restrict__ p, size_t P, int rx, int ry, int rw, int rh) {
   return p[(size_t)(ry + rh) * P + rx + rw] - p[(size_t)ry * P + rx + rw] - p[(size_t)(ry + rh) * P + rx] + p[(size_t)ry * P + rx];
 }
 
-// Stages [s_begin, s_end) of the window at s0, one thread per window, in the cascade's order: v = v + weight * rectsum over the feature's
-// rects, sum = sum + leaf over the stumps (f32, unfused under -fmad=false).  A window's sums are never split across lanes: a reordered
-// f32 sum could flip a stump or a stage near its threshold.  Returns the first stage whose sum falls below its threshold, or -1.
-__device__ __forceinline__ int haar_stages(const uint32_t* __restrict__ s0, size_t P, float inv, const HaarDev& K, int s_begin, int s_end) {
+// CV_TILTED_OFS: the 45-degree rect with corners (x, y), (x + w, y + w), (x - h, y + h), (x + w - h, y + w + h) from the tilted integral
+__device__ __forceinline__ uint32_t haar_tiltsum(const uint32_t* __restrict__ t, size_t P, int rx, int ry, int rw, int rh) {
+  return t[(size_t)ry * P + rx] - t[(size_t)(ry + rh) * P + rx - rh] - t[(size_t)(ry + rw) * P + rx + rw] + t[(size_t)(ry + rw + rh) * P + rx + rw - rh];
+}
+
+// feature value: v = v + weight * rectsum over the feature's rects; TILT: a tilted feature's rects come from t0
+template <bool TILT>
+__device__ __forceinline__ float haar_feature(const uint32_t* __restrict__ s0, const uint32_t* __restrict__ t0, size_t P, const HaarDev& K, int fi) {
+  const HaarFeature& f = K.feats[fi];
+  float v = 0.f;
+  if constexpr (TILT) {
+    if (K.tilt[fi]) {
+#pragma unroll
+      for (int r = 0; r < 3; r++) {
+        const HaarRect hr = f.r[r];
+        if (hr.weight != 0.f) v = v + hr.weight * (float)haar_tiltsum(t0, P, hr.x, hr.y, hr.w, hr.h);
+      }
+      return v;
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < 3; r++) {
+    const HaarRect hr = f.r[r];
+    if (hr.weight != 0.f) v = v + hr.weight * (float)haar_rectsum(s0, P, hr.x, hr.y, hr.w, hr.h);
+  }
+  return v;
+}
+
+// Stages [s_begin, s_end) of the window at s0 (t0 in the tilted integral), one thread per window, in the cascade's order: the feature
+// values, sum = sum + leaf over the weak classifiers (f32, unfused under -fmad=false).  A stump picks its leaf by value * inv <
+// threshold; TREE walks the tree (OpenCV's predictOrdered) with the same comparison at every node, of which a stump is the one-node
+// case.  A window's sums are never split across lanes: a reordered f32 sum could flip a stump or a stage near its threshold.  Returns
+// the first stage whose sum falls below its threshold, or -1.
+template <bool TREE, bool TILT>
+__device__ __forceinline__ int haar_stages(const uint32_t* __restrict__ s0, const uint32_t* __restrict__ t0, size_t P, float inv, const HaarDev& K,
+                                           int s_begin, int s_end) {
   for (int si = s_begin; si < s_end; si++) {
     const HaarStage st = K.stages[si];
     float sum = 0.f;
     for (int k = st.first; k < st.first + st.count; k++) {
-      const HaarWeak wk = K.weak[k];
-      const HaarFeature& f = K.feats[wk.feature];
-      float v = 0.f;
-#pragma unroll
-      for (int r = 0; r < 3; r++) {
-        const HaarRect hr = f.r[r];
-        if (hr.weight != 0.f) v = v + hr.weight * (float)haar_rectsum(s0, P, hr.x, hr.y, hr.w, hr.h);
+      if constexpr (TREE) {
+        const HaarTree tr = K.trees[k];
+        int idx = 0;
+        do {   // child indices grow along a walk (checked at load), so this ends within the tree's node count
+          const HaarNode nd = K.nodes[tr.node + idx];
+          const float v = haar_feature<TILT>(s0, t0, P, K, nd.feature);
+          idx = (v * inv < nd.threshold) ? nd.left : nd.right;
+        } while (idx > 0);
+        sum = sum + K.leaves[tr.leaf - idx];
+      } else {
+        const HaarWeak wk = K.weak[k];
+        const float v = haar_feature<TILT>(s0, t0, P, K, wk.feature);
+        sum = sum + ((v * inv < wk.threshold) ? wk.left : wk.right);
       }
-      sum = sum + ((v * inv < wk.threshold) ? wk.left : wk.right);
     }
     if (!(sum >= st.threshold)) return si;
   }
@@ -267,9 +497,10 @@ __device__ __forceinline__ void haar_append(bool keep, uint2 item, uint2* __rest
 
 // First stage group, every window of every instance of the group: HaarEvaluator::setWindow's variance normalisation over the inner
 // (w - 2) x (h - 2) rect, stages [0, s_end); writes the window's flag byte and appends the survivors (flag index, 1 / nf) to the work list
-// of the next stage group.  ceil(nx / 128) x ny blocks per instance, 128 threads.
+// of the next stage group.  T: the tilted integrals (TILT only).  ceil(nx / 128) x ny blocks per instance, 128 threads.
+template <bool TREE, bool TILT>
 __global__ void __launch_bounds__(128) k_haar_eval_first(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, const uint32_t* __restrict__ S, const uint32_t* __restrict__ Q,
-                                                         HaarDev K, int s_end, uint8_t* __restrict__ flags, uint2* __restrict__ list, unsigned* __restrict__ count) {
+                                                         const uint32_t* __restrict__ T, HaarDev K, int s_end, uint8_t* __restrict__ flags, uint2* __restrict__ list, unsigned* __restrict__ count) {
   const int b = (int)blockIdx.x;
   const HaarInst& L = inst[haar_inst_of(keys.blk_eval, ninst, b)];
   const int nx = L.nx, ystep = L.ystep, bx = (nx + 127) / 128, lb = b - L.blk_eval, iy = lb / bx;
@@ -289,7 +520,7 @@ __global__ void __launch_bounds__(128) k_haar_eval_first(const HaarInst* __restr
     if (nf > 0.) {
       inv = (float)(1.0 / sqrt(nf));
       if ((float)area * inv < 0.1f) {
-        const int r = haar_stages(s0, P, inv, K, 0, s_end);
+        const int r = haar_stages<TREE, TILT>(s0, TILT ? T + o : nullptr, P, inv, K, 0, s_end);
         if (r < 0) { if (s_end >= K.nstages) out = 1; else keep = true; }
         else if (r == 0) out = 2;
       }
@@ -304,7 +535,9 @@ __global__ void __launch_bounds__(128) k_haar_eval_first(const HaarInst* __restr
 // A later stage group [s_begin, s_end) on the previous group's survivors, grid-stride over the list (its length is on the device, so the
 // launch does not wait for the host).  Compaction changes which thread handles a window, never the order of its arithmetic.  Survivors of
 // the last group get bit 0 of their flag; the others are appended to the next list.
-__global__ void __launch_bounds__(128) k_haar_eval_list(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, const uint32_t* __restrict__ S, HaarDev K,
+template <bool TREE, bool TILT>
+__global__ void __launch_bounds__(128) k_haar_eval_list(const HaarInst* __restrict__ inst, HaarKeys keys, int ninst, const uint32_t* __restrict__ S,
+                                                        const uint32_t* __restrict__ T, HaarDev K,
                                                         int s_begin, int s_end, const uint2* __restrict__ list_in, const unsigned* __restrict__ count_in,
                                                         uint8_t* __restrict__ flags, uint2* __restrict__ list_out, unsigned* __restrict__ count_out) {
   const unsigned n = *count_in;
@@ -319,8 +552,8 @@ __global__ void __launch_bounds__(128) k_haar_eval_list(const HaarInst* __restri
       const size_t w = it.x - L.flag_off;
       const int iy = (int)(w / L.nx), ix = (int)(w - (size_t)iy * L.nx);
       const size_t P = (size_t)L.sw + 1;
-      const uint32_t* __restrict__ s0 = S + L.int_off + (size_t)(iy * L.ystep) * P + (size_t)ix * L.ystep;
-      if (haar_stages(s0, P, __uint_as_float(it.y), K, s_begin, s_end) < 0) {
+      const size_t o = L.int_off + (size_t)(iy * L.ystep) * P + (size_t)ix * L.ystep;
+      if (haar_stages<TREE, TILT>(S + o, TILT ? T + o : nullptr, P, __uint_as_float(it.y), K, s_begin, s_end) < 0) {
         if (last) flags[it.x] = 1; else keep = true;
       }
     }

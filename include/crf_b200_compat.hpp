@@ -18,8 +18,8 @@
 //   * FaceForest's constructor loads the face cascade only if fd_option.path_face_cascade is set (the reference requires it,
 //     src/FaceForest.cpp:23-28); without it analyzeImage(img, bboxes, faces) takes the boxes from the caller.  Either way all
 //     faces of a frame are analysed in one launch.
-//   * crf_b200::CascadeClassifier stands for cv::CascadeClassifier (load + detectMultiScale, evaluated on the GPU); it reads the
-//     new-format stump-based HAAR cascades, which is what the reference ships.
+//   * crf_b200::CascadeClassifier stands for cv::CascadeClassifier (load + detectMultiScale, evaluated on the GPU); it reads every
+//     HAAR cascade cv::CascadeClassifier reads (stumps or trees, tilted features, old or new XML format), not LBP / HOG ones.
 //   * FaceForestOptions carries three extra members at its end (device, ms_mode, mean_shift_option).
 #ifndef CRF_B200_COMPAT_HPP
 #define CRF_B200_COMPAT_HPP

@@ -12,7 +12,12 @@ crf_analyze_batch_mixed call.  Every call ends in a device synchronise, so host 
 With --lib pointing at the library of an earlier build, entry points that build lacks are skipped, to give the "before" numbers on the
 same frames.
 
-  python tools/detect_bench.py [--lib path/to/libcrf_b200.so] [--reps 3] [--out detect_bench.json]
+--cascade names another cascade file (default: the face cascade); --sets C3,R64 limits the run to those frame sets (the extras: boxes
+given, single-frame latency, split sweep, only run with the default sets).  --cv2 also times cv2.CascadeClassifier.detectMultiScale with
+the same cascade and parameters on the first 16 frames of each set, one host call per frame on the host's cores, for scale.  With a library that has
+the counters, `launches_per_group` is the kernel launches of crf_detect_faces_batch on one group (one C3 frame).
+
+  python tools/detect_bench.py [--lib path/to/libcrf_b200.so] [--reps 3] [--cascade file.xml] [--sets C3,R64] [--cv2] [--out detect_bench.json]
 """
 from __future__ import annotations
 
@@ -186,6 +191,9 @@ def main():
     ap.add_argument("--frames", type=int, default=64)
     ap.add_argument("--splits", default="0;1;1,3;2,5;3,8;1,2,4,8", help="CRF_HAAR_SPLIT values for the split sweep of (b) ('0' = one stage group)")
     ap.add_argument("--out", default="detect_bench.json", help="where the JSON result goes")
+    ap.add_argument("--cascade", default=None, help="cascade XML (default: the face cascade, staged or cv2's haarcascade_frontalface_alt.xml)")
+    ap.add_argument("--sets", default="C3,C5,R64", help="frame sets to run, of C3, C5, R64; the extras run only with all three")
+    ap.add_argument("--cv2", action="store_true", help="also time cv2's detectMultiScale on the same frames (host cores)")
     a = ap.parse_args()
     import cv2
     from face_alignment_cvpr_2012_b200 import synthetic_model as sm
@@ -207,6 +215,9 @@ def main():
     xml = wl.STAGED / "haarcascade_frontalface_alt.xml"
     if not xml.exists():
         xml = Path(cv2.data.haarcascades) / "haarcascade_frontalface_alt.xml"
+    if a.cascade:
+        xml = Path(a.cascade)
+    sets = set(a.sets.split(","))
     cas = vp()
     check(L, L.crf_cascade_load(str(xml).encode(), C.byref(cas)))
 
@@ -248,12 +259,39 @@ def main():
             row["d_detect_mixed_one_call"] = {"faces_found": n, "frames_per_s": nfr / t, "detect_ms_per_frame": 1e3 * t / nfr}
             n, t = med(lambda: mixed_analyze(L, ctx, cas, frames), a.reps)
             row["d_analyze_images_mixed_one_call"] = {"faces_found": n, "frames_per_s": nfr / t, "ms_per_frame": 1e3 * t / nfr}
+        if a.cv2:
+            cc = cv2.CascadeClassifier(str(xml))
+            frames = [cv2.cvtColor(f, cv2.COLOR_BGR2GRAY) for g in groups for f in g][:16]   # the first 16 frames, once: it is slow
+            cc.detectMultiScale(frames[0], SF, MN, minSize=(MS, MS))
+            t0 = time.perf_counter()
+            n = sum(len(cc.detectMultiScale(f, SF, MN, minSize=(MS, MS))) for f in frames)
+            t = time.perf_counter() - t0
+            row["cv2_detect_host"] = {"frames": len(frames), "faces_found": n, "threads": cv2.getNumThreads(), "cpus": os.cpu_count(),
+                                      "detect_ms_per_frame": 1e3 * t / len(frames)}
         res["sets"][name] = row
         print(name, json.dumps(row), flush=True)
 
-    run_set(f"C3_{a.frames}x1080p", [c3])
-    run_set("C5_mixed_64", list(by_res.values()))
-    run_set("R64_ragged_64", [[f] for f, _ in r64])
+    if hasattr(L, "crf_ctx_counters") and batched:
+        from face_alignment_cvpr_2012_b200 import capi
+        cnt = capi.Counters()
+        L.crf_ctx_counters.argtypes = [vp, C.c_void_p]
+        L.crf_ctx_reset_counters.argtypes = [vp]
+        L.crf_ctx_reset_counters(ctx)
+        batch_detect(L, ctx, cas, c3[:1])   # one frame: one group
+        L.crf_ctx_counters(ctx, C.byref(cnt))
+        res["launches_per_group"] = int(cnt.kernel_launches)
+    if "C3" in sets:
+        run_set(f"C3_{a.frames}x1080p", [c3])
+    if "C5" in sets:
+        run_set("C5_mixed_64", list(by_res.values()))
+    if "R64" in sets:
+        run_set("R64_ragged_64", [[f] for f, _ in r64])
+    if sets != {"C3", "C5", "R64"}:
+        L.crf_ctx_destroy(ctx)
+        Path(a.out).parent.mkdir(parents=True, exist_ok=True)
+        Path(a.out).write_text(json.dumps(res, indent=1))
+        print(json.dumps(res))
+        return
     given = {}
     n, t = med(lambda: boxes_per_image(L, ctx, mixed), a.reps)
     given["per_image_analyze_faces"] = {"faces": n, "faces_per_s": n / t, "ms_per_call_set": 1e3 * t}
