@@ -43,6 +43,11 @@ def images(frames) -> "C.Array":
     return (Image * max(len(frames), 1))(*[Image(f.ctypes.data, f.shape[0], f.shape[1], f.strides[0]) for f in frames])
 
 
+class HaarLevel(C.Structure):
+    """crf_haar_level_t: one (frame, pyramid level) instance of the detector."""
+    _fields_ = [("factor", C.c_double)] + [(n, C.c_int) for n in ("frame", "sw", "sh", "ystep", "nx", "ny", "win_w", "win_h", "tilted")]
+
+
 class Options(C.Structure):
     _fields_ = [("hp_stride", C.c_int), ("hp_min_foreground", C.c_float), ("ffd_stride", C.c_int), ("ffd_min_samples", C.c_int),
                 ("ffd_min_foreground", C.c_float), ("ffd_min_pf", C.c_float), ("ffd_max_variance", C.c_float),
@@ -80,6 +85,7 @@ EXPORTS = [
     "crf_cascade_load", "crf_cascade_free", "crf_cascade_info", "crf_detect_faces", "crf_detect_faces_batch", "crf_analyze_images",
     "crf_multi_create", "crf_multi_destroy", "crf_multi_device_count", "crf_multi_ctx", "crf_multi_analyze_batch", "crf_multi_analyze_crops",
     "crf_analyze_batch_mixed", "crf_detect_faces_batch_mixed", "crf_analyze_images_mixed", "crf_multi_analyze_batch_mixed",
+    "crf_stage_haar_levels",
 ]
 
 _lib = None
@@ -167,6 +173,8 @@ def lib() -> C.CDLL:
                                      C.POINTER(Rect), i32p, vp, C.c_int]
     L.crf_detect_faces_batch_mixed.argtypes = [vp, vp, C.POINTER(Image), C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(Rect), i32p, C.c_int]
     L.crf_analyze_images_mixed.argtypes = [vp, vp, C.POINTER(Image), C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(Rect), i32p, vp, C.c_int]
+    L.crf_stage_haar_levels.argtypes = [vp, vp, C.POINTER(Image), C.c_int, C.c_double, C.c_int, C.POINTER(HaarLevel), C.c_int, C.POINTER(C.c_uint32),
+                                        C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), u8p]
     L.crf_multi_create.argtypes = [vp, i32p, C.c_int, C.POINTER(Options), C.POINTER(vp)]
     L.crf_multi_destroy.argtypes = [vp]
     L.crf_multi_destroy.restype = None

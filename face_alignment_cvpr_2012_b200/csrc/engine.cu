@@ -965,12 +965,23 @@ static int upload_frames(crf_ctx* c, const crf_image_t* images, int f0, int nf, 
   return CRF_OK;
 }
 
+// A group's device results after its last stage group, before the scan, in instance order: the integrals S, Q and T (T for a tilted
+// cascade only, else null), the window flags, their sizes (integral elements, windows) and the group's stream.
+struct HaarPasses {
+  const uint32_t *S, *Q, *T;
+  const uint8_t* flags;
+  size_t nint, nwin;
+  cudaStream_t s;
+};
+struct NoPasses { int operator()(const HaarPasses&) const { return CRF_OK; } };
+
 // detectMultiScale on n_images frames of any sizes, a group of consecutive frames at a time.  After a group's boxes are grouped,
 // per_group(f0, nf, off, boxes) runs while the group's frames are still in d_haar_frames (frame f0 + k at off[k]); boxes[k] are frame
-// f0 + k's.
-template <class F>
+// f0 + k's.  passes(HaarPasses) runs on every group with instances once its stage groups are enqueued (crf_stage_haar_levels copies them
+// back there); the detection calls leave it at NoPasses.
+template <class F, class P = NoPasses>
 static int detect_frames(crf_ctx* c, const crf_cascade* cas, const crf_image_t* images, int n_images, double scale_factor, int min_neighbors,
-                         int min_size, F&& per_group) {
+                         int min_size, F&& per_group, P&& passes = P{}) {
   const Cascade& K = cas->c;
   std::vector<FramePlan> plans((size_t)n_images);
   for (int i = 0; i < n_images; i++) {
@@ -1086,6 +1097,7 @@ static int detect_frames(crf_ctx* c, const crf_cascade* cas, const crf_image_t* 
         eval_list<<<c->sm_count * 8, 128, 0, s>>>(d_inst, keys, ninst, S, T, dev, bounds[g - 1], bounds[g], list[in], lists_n + in, flags, list[out], lists_n + out);
         KCHECK(); count_launch(c, CRF_STAGE_RESIZE);
       }
+      if ((rc = passes(HaarPasses{S, Q, T, flags, io, fo, s}))) return rc;
       int* d_rows = c->d_haar_rows.as<int>();
       k_haar_scan<true><<<(nrows + 7) / 8, 256, 0, s>>>(d_inst, keys, ninst, nrows, flags, d_rows, nullptr, nullptr);
       k_haar_row_offsets<<<nf, 1024, 0, s>>>(d_frame_rows, d_rows, fcount);
@@ -1178,6 +1190,33 @@ int crf_cascade_info(const crf_cascade* c, int* win_w, int* win_h, int* nstages,
   if (nstages) *nstages = (int)c->c.stages.size();
   if (nweak) *nweak = c->c.nweak();
   return CRF_OK;
+}
+
+int crf_stage_haar_levels(crf_ctx* c, const crf_cascade* cas, const crf_image_t* images, int n_images, double scale_factor, int min_size,
+                          crf_haar_level_t* levels, int cap, uint32_t* S, uint32_t* Q, uint32_t* T, uint8_t* flags) {
+  if (int rc = detect_args(c, cas, images, n_images, scale_factor, cap, levels)) return rc;
+  const int tilted = cas->c.has_tilted ? 1 : 0;
+  int total = 0;
+  for (int i = 0; i < n_images; i++)
+    for (const HaarInst& L : detect_plan(cas->c, images[i], scale_factor, min_size).levels) {
+      if (total < cap) levels[total] = crf_haar_level_t{L.factor, i, L.sw, L.sh, L.ystep, L.nx, L.ny, L.win_w, L.win_h, tilted};
+      total++;
+    }
+  if (total > cap || !(S || Q || T || flags)) return total;
+  size_t io = 0, fo = 0;   // the group's first integral element and window among all the frames'
+  const int rc = detect_frames(c, cas, images, n_images, scale_factor, 0, min_size,
+                               [](int, int, const std::vector<size_t>&, std::vector<std::vector<crf_rect_t>>&) { return CRF_OK; },
+                               [&](const HaarPasses& g) -> int {
+    const size_t ib = g.nint * sizeof(uint32_t);
+    if (S) CU(cudaMemcpyAsync(S + io, g.S, ib, cudaMemcpyDeviceToHost, g.s));
+    if (Q) CU(cudaMemcpyAsync(Q + io, g.Q, ib, cudaMemcpyDeviceToHost, g.s));
+    if (T && g.T) CU(cudaMemcpyAsync(T + io, g.T, ib, cudaMemcpyDeviceToHost, g.s));
+    if (flags) CU(cudaMemcpyAsync(flags + fo, g.flags, g.nwin, cudaMemcpyDeviceToHost, g.s));
+    c->cnt.d2h_bytes += (S ? ib : 0) + (Q ? ib : 0) + (T && g.T ? ib : 0) + (flags ? g.nwin : 0);
+    io += g.nint; fo += g.nwin;
+    return CRF_OK;
+  });
+  return rc ? rc : total;
 }
 
 int crf_detect_faces_batch_mixed(crf_ctx* c, const crf_cascade* cas, const crf_image_t* images, int n_images, double scale_factor, int min_neighbors,

@@ -431,6 +431,45 @@ class Context:
         capi.check(capi.lib().crf_stage_meanshift(self.h, capi.ptr(v, C.c_float), len(v), capi.ptr(mean, C.c_float), capi.ptr(rnd, C.c_int32), C.byref(it)))
         return mean, rnd, it.value
 
+    def stage_haar_levels(self, cascade: "CascadeClassifier", frames, scale_factor: float = 1.3, min_size: int = 0, integrals: bool = True) -> list:
+        """The detector's device passes on BGR frames of any sizes (crf_stage_haar_levels): one dict per (frame, pyramid level) instance,
+        frame-major then level, with the plan (frame, factor, sw, sh, ystep, nx, ny, win_w, win_h), the window flags [ny, nx] u8 and,
+        with integrals, S and Q [sh + 1, sw + 1] u32 and T (the tilted integral, None for an upright cascade)."""
+        frames = _frame_list(frames)
+        L = capi.lib()
+        args = (self.h, cascade.h, capi.images(frames), len(frames), float(scale_factor), int(min_size))
+
+        def call(lv, cap, *bufs):
+            rc = L.crf_stage_haar_levels(*args, lv, cap, *bufs)
+            if rc < 0:
+                capi.check(rc)
+            return rc
+
+        n = call(None, 0, None, None, None, None)
+        if n == 0:
+            return []
+        lv = (capi.HaarLevel * n)()
+        call(lv, n, None, None, None, None)   # the plan only
+        nint = [(v.sh + 1) * (v.sw + 1) for v in lv]
+        nwin = [v.nx * v.ny for v in lv]
+        tilted = integrals and lv[0].tilted
+        S, Q, T = (np.zeros(sum(nint) if k else 1, np.uint32) for k in (integrals, integrals, tilted))
+        flags = np.zeros(sum(nwin), np.uint8)
+        u32 = C.c_uint32
+        call(lv, n, capi.ptr(S, u32) if integrals else None, capi.ptr(Q, u32) if integrals else None, capi.ptr(T, u32) if tilted else None,
+             capi.ptr(flags, C.c_uint8))
+        out, io, fo = [], 0, 0
+        for v, ni, nw in zip(lv, nint, nwin):
+            d = {k: getattr(v, k) for k, _ in v._fields_ if k != "tilted"}
+            shape = (v.sh + 1, v.sw + 1)
+            d["flags"] = flags[fo:fo + nw].reshape(v.ny, v.nx)
+            if integrals:
+                d["S"], d["Q"] = S[io:io + ni].reshape(shape), Q[io:io + ni].reshape(shape)
+                d["T"] = T[io:io + ni].reshape(shape) if tilted else None
+            out.append(d)
+            io += ni; fo += nw
+        return out
+
 
 class CascadeClassifier:
     """cv::CascadeClassifier (src/FaceForest.cpp:23) for OpenCV's HAAR cascades: the reference's face cascade or any other that

@@ -314,6 +314,20 @@ int crf_stage_meanshift_opt(crf_ctx* ctx, const float* votes_xyw, int n, int ker
 /* areaUnderCurve(x1, x2, mean, std) (src/face_utils.cpp:304-323; include/face_utils.hpp:103-108). */
 int crf_stage_area_under_curve(crf_ctx* ctx, float x1, float x2, double mean, double std_, float* area);
 
+/* One (frame, pyramid level) instance of the detector: the scale, the level's size sw x sh, its window grid (nx x ny windows, ystep
+ * level pixels apart), the window in frame pixels, and tilted = 1 when the cascade has tilted features (T is built). */
+typedef struct { double factor; int frame, sw, sh, ystep, nx, ny, win_w, win_h, tilted; } crf_haar_level_t;
+/* The device passes of crf_detect_faces_batch_mixed(ctx, c, images, n_images, scale_factor, ., min_size, ...), copied back after the
+ * last cascade stage group (the same launches, groups of frames and CRF_HAAR_SPLIT stage groups as detection).  Returns the instance
+ * count (frame-major, then level); levels[0 .. cap) get the instances.  With cap at least the count and any of S / Q / T / flags
+ * non-null, the passes run and each given buffer receives every instance's data back to back in instance order:
+ *   S, Q   (sh + 1) x (sw + 1) u32 integrals of the level's pixels and of their squares, modulo 2^32 (cv::integral's layout)
+ *   T      the same layout for the tilted integral (cv::integral's third output); written only when the cascade has tilted features
+ *   flags  ny x nx bytes, one per window: 1 passed every stage, 2 rejected by stage 0, 0 otherwise (rejected by a later stage, or
+ *          skipped by the variance test: area * sqsum - sum^2 <= 0, or area / sqrt(that) >= 0.1) */
+int crf_stage_haar_levels(crf_ctx* ctx, const crf_cascade* c, const crf_image_t* images, int n_images, double scale_factor, int min_size,
+                          crf_haar_level_t* levels, int cap, uint32_t* S, uint32_t* Q, uint32_t* T, uint8_t* flags);
+
 #ifdef __cplusplus
 }
 #endif

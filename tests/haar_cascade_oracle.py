@@ -10,7 +10,9 @@ It extends oracle/haar.py (stump cascades, upright features, new format), whose 
            one feature per node, a tree's leaves numbered in node order, left before right
 The arithmetic per window is the GPU's: f32 feature values and stage sums in the cascade's order.
 
-Also here: write_cascade, a seeded writer of synthetic cascades (trees of 1 to 3 nodes, tilted and upright features) in either format.
+Also here: the detector's device passes level by level (level_plan, level_image, level_integrals, window_flags), the reference of
+crf_stage_haar_levels; and write_cascade, a seeded writer of synthetic cascades (trees of 1 to 3 nodes, tilted and upright features) in
+either format.
 """
 from __future__ import annotations
 
@@ -113,7 +115,7 @@ def stage_sums(c: Cascade, gray: np.ndarray, factor: float = 1.0, cv2_arith: boo
     img = H._resize(gray, sh, sw).astype(np.int64) if factor != 1.0 else gray.astype(np.int64)
     S = np.zeros((sh + 1, sw + 1), np.int64); S[1:, 1:] = img.cumsum(0).cumsum(1)
     Q = np.zeros((sh + 1, sw + 1), np.int64); Q[1:, 1:] = (img * img).cumsum(0).cumsum(1)
-    T = tilted_integral(img.astype(np.uint8)).astype(np.int64) if c.tilted.any() else None
+    T = cv2_tilted_integral(img.astype(np.uint8)).astype(np.int64) if c.tilted.any() else None
     ystep = 1 if factor > 2.0 else 2
     ys, xs = np.arange(0, sh - c.h + 1, ystep), np.arange(0, sw - c.w + 1, ystep)
     yy, xx = np.meshgrid(ys, xs, indexing="ij")
@@ -171,31 +173,87 @@ def stage_sums(c: Cascade, gray: np.ndarray, factor: float = 1.0, cv2_arith: boo
     return sums, ok, ys, xs
 
 
+def window_flags(c: Cascade, sums, ok) -> np.ndarray:
+    """The detector's flag byte of each window of a level from stage_sums' (sums, ok): 1 passed every stage, 2 rejected by stage 0, 0
+    otherwise (rejected by a later stage, or skipped by the variance test: nf <= 0 or area / nf >= 0.1)."""
+    passed = np.stack([sums[si] >= thr for si, (thr, _) in enumerate(c.stages)])
+    return np.where(ok & passed.all(0), 1, np.where(ok & ~passed[0], 2, 0)).astype(np.uint8)
+
+
+def scan_candidates(flags, ys, xs, factor, win):
+    """OpenCV's scan of one level: windows in (iy, ix) order, one extra step after a stage-0 reject; the visited windows that passed every
+    stage, as frame rectangles."""
+    rej0 = (flags & 2) != 0
+    pos = np.arange(flags.shape[1])
+    # a window is visited when an even number of stage-0 rejects precede it in its row (each visited reject skips the next window)
+    last = np.maximum.accumulate(np.where(rej0, -1, pos), axis=1)   # last position at or before ix that stage 0 did not reject
+    run = np.zeros(flags.shape, np.int64)
+    run[:, 1:] = pos[:-1] - last[:, :-1]
+    iy, ix = np.nonzero(((flags & 1) != 0) & (run % 2 == 0))
+    x, y = np.rint(xs[ix] * factor).astype(np.int64), np.rint(ys[iy] * factor).astype(np.int64)
+    return [(int(a), int(b), win[0], win[1]) for a, b in zip(x, y)]
+
+
+def detect_levels(c: Cascade, gray: np.ndarray, scale_factor: float = 1.3, min_size: int = 30):
+    """Per level of level_plan: (level, window flags [ny][nx], ys, xs)."""
+    for L in level_plan(c.w, c.h, *gray.shape, scale_factor, min_size):
+        sums, ok, ys, xs = stage_sums(c, gray, L["factor"])
+        yield L, window_flags(c, sums, ok), ys, xs
+
+
+def level_candidates(levels):
+    """The raw candidates of detect_levels' levels, in (level, iy, ix) order."""
+    return [r for L, flags, ys, xs in levels for r in scan_candidates(flags, ys, xs, L["factor"], (L["win_w"], L["win_h"]))]
+
+
 def detect_candidates(c: Cascade, gray: np.ndarray, scale_factor: float = 1.3, min_size: int = 30):
     """oracle.haar.detect_candidates for any cascade: raw candidates in (level, iy, ix) order."""
-    Hh, W = gray.shape
+    return level_candidates(detect_levels(c, gray, scale_factor, min_size))
+
+
+# ---- the detector's device passes, level by level ----------------------------------------------------------------------------------
+def level_plan(win_w: int, win_h: int, rows: int, cols: int, scale_factor: float, min_size: int = 0) -> list:
+    """The pyramid levels of one rows x cols frame, as detect_plan (csrc/engine.cu) and oracle.haar's scale loop build them: factor = 1,
+    scale_factor, scale_factor^2, ...; the level is round(cols / factor) x round(rows / factor) and the window round(win * factor); the
+    loop stops when the window exceeds the frame or the level is smaller than the cascade's window, and skips levels whose window is
+    below min_size.  Windows lie ystep level pixels apart (2 while factor <= 2, then 1).  One dict per level with the fields of
+    crf_haar_level_t."""
     out = []
     factor = 1.0
     while True:
-        win = (int(round(c.w * factor)), int(round(c.h * factor)))
-        sw, sh = int(round(W / factor)), int(round(Hh / factor))
-        if win[0] > W or win[1] > Hh or sw < c.w or sh < c.h:
-            break
-        if win[0] >= min_size and win[1] >= min_size:
-            sums, ok, ys, xs = stage_sums(c, gray, factor)
-            passed = np.stack([sums[si] >= thr for si, (thr, _) in enumerate(c.stages)])
-            alive = ok & passed.all(0)
-            first_fail = ok & ~passed[0]
-            for iy in range(len(ys)):
-                ix = 0
-                while ix < len(xs):
-                    if alive[iy, ix]:
-                        out.append((int(round(xs[ix] * factor)), int(round(ys[iy] * factor)), win[0], win[1]))
-                    if first_fail[iy, ix]:
-                        ix += 1
-                    ix += 1
+        ww, wh = int(round(win_w * factor)), int(round(win_h * factor))
+        sw, sh = int(round(cols / factor)), int(round(rows / factor))
+        if ww > cols or wh > rows or sw < win_w or sh < win_h:
+            return out
+        if ww >= min_size and wh >= min_size:
+            ystep = 1 if factor > 2.0 else 2
+            out.append(dict(factor=factor, sw=sw, sh=sh, ystep=ystep, nx=(sw - win_w + ystep) // ystep, ny=(sh - win_h + ystep) // ystep,
+                            win_w=ww, win_h=wh))
         factor *= scale_factor
-    return out
+
+
+def level_image(gray: np.ndarray, level: dict) -> np.ndarray:
+    """The level's u8 pixels: oracle.haar's bilinear resize of the gray frame (the frame itself at factor 1)."""
+    return H._resize(gray, level["sh"], level["sw"]) if level["factor"] != 1.0 else gray
+
+
+def cv2_tilted_integral(img: np.ndarray) -> np.ndarray:
+    """cv2.integral3(img)[2] as u32: the tilted integral tilted_integral restates (test_tilted_integral_equals_cv2), at cv2's speed."""
+    import cv2
+    return cv2.integral3(np.ascontiguousarray(img, np.uint8), sdepth=cv2.CV_32S)[2].view(np.uint32)
+
+
+def level_integrals(img: np.ndarray, tilted: bool = True):
+    """(S, Q, T) of a u8 level image, each [(h + 1) x (w + 1)] u32: the integrals of the values and of their squares (np.cumsum in u64,
+    reduced modulo 2^32 as the detector's u32 sums are) and the tilted integral (None unless tilted)."""
+    h, w = img.shape
+    v = img.astype(np.uint64)
+    S = np.zeros((h + 1, w + 1), np.uint64)
+    Q = np.zeros((h + 1, w + 1), np.uint64)
+    S[1:, 1:] = np.cumsum(np.cumsum(v, 0), 1)
+    Q[1:, 1:] = np.cumsum(np.cumsum(v * v, 0), 1)
+    m = np.uint64(0xffffffff)
+    return (S & m).astype(np.uint32), (Q & m).astype(np.uint32), cv2_tilted_integral(img) if tilted else None
 
 
 def detect_multi_scale(c: Cascade, bgr_or_gray: np.ndarray, scale_factor: float = 1.3, min_neighbors: int = 1, min_size: int = 30):

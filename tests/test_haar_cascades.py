@@ -246,3 +246,87 @@ def test_malformed_cascades_fail_cleanly(crf, synth, tmp_path):
     p = tmp_path / "other.xml"
     p.write_text('<?xml version="1.0"?>\n<opencv_storage>\n<thing type_id="opencv-matrix"><rows>1</rows></thing>\n</opencv_storage>\n')
     assert load(crf, p)[0] == ERR_FORMAT
+
+
+# ---- the level reference of the detector's device passes (crf_stage_haar_levels) -------------------------------------------------------
+def test_level_integrals_equal_cv2():
+    """S equals cv2.integral, Q cv2.integral2's square sums modulo 2^32 and T the closed-form tilted integral, on levels whose square sums
+    pass 2^32 (so Q wraps): a bright textured frame, an all-255 frame and a 0/255 checkerboard."""
+    from oracle import oracle as O
+    rng = np.random.default_rng(3)
+    bright = cv2.GaussianBlur(rng.integers(128, 256, (330, 420, 3), dtype=np.uint8), (0, 0), 1.0)
+    white = np.full((300, 330, 3), 255, np.uint8)
+    check = np.repeat(((np.indices((320, 420)).sum(0) % 2) * 255).astype(np.uint8)[..., None], 3, 2)
+    for frame in (bright, white, check):
+        gray = O.bgr2gray(frame)
+        plan = G.level_plan(20, 20, *gray.shape, 1.3)
+        assert len(plan) >= 3
+        wrapped = False
+        for L in plan[:3]:
+            img = G.level_image(gray, L)
+            assert img.shape == (L["sh"], L["sw"])
+            S, Q, T = G.level_integrals(img)
+            assert np.array_equal(S, cv2.integral(img, sdepth=cv2.CV_32S).view(np.uint32))
+            q = cv2.integral2(img, sdepth=cv2.CV_32S, sqdepth=cv2.CV_64F)[1]
+            assert np.array_equal(Q, (q.astype(np.uint64) & np.uint64(0xffffffff)).astype(np.uint32))
+            assert np.array_equal(T, G.tilted_integral(img).view(np.uint32))
+            wrapped |= q[-1, -1] >= 2.0 ** 32
+        assert wrapped
+
+
+def test_level_plan_equals_oracle_scale_loop(monkeypatch):
+    """level_plan gives the levels of oracle.haar.detect_candidates' scale loop: the level sizes it resizes to, its window grids (count
+    and ystep) and the levels it skips below min_size or stops at, for scale factors 1.05 to 2.5 and frames from 1 x 1 to 1080p."""
+    from oracle import haar as H
+    c = H.Cascade(CV2_DIR / "haarcascade_frontalface_alt.xml")
+    seen = []
+    real_meshgrid = np.meshgrid
+    # the oracle's scale loop on zero frames: every window fails the variance test, so only the loop itself runs
+    monkeypatch.setattr(H, "_resize", lambda gray, dh, dw: (seen.append(("resize", dh, dw)), np.zeros((dh, dw), np.uint8))[1])
+
+    class RecordingNumpy:
+        def __getattr__(self, name):
+            return getattr(np, name)
+
+        @staticmethod
+        def meshgrid(ys, xs, **kw):
+            seen.append(("grid", len(ys), len(xs), int(xs[1] - xs[0]) if len(xs) > 1 else None))
+            return real_meshgrid(ys, xs, **kw)
+
+    monkeypatch.setattr(H, "np", RecordingNumpy())
+    ystep1 = ystep2 = skipped = 0
+    for rows, cols in [(250, 250), (480, 640), (97, 131), (20, 20), (21, 21), (19, 19), (1, 1), (48, 4000), (4000, 48), (1080, 1920)]:
+        for sf in (1.05, 1.1, 1.3, 2.5):
+            for ms in (0, 30, 50, 100):
+                seen.clear()
+                assert H.detect_candidates(c, np.zeros((rows, cols), np.uint8), sf, ms) == []
+                plan = G.level_plan(c.w, c.h, rows, cols, sf, ms)
+                want = []
+                for L in plan:
+                    if L["factor"] != 1.0:
+                        want.append(("resize", L["sh"], L["sw"]))
+                    want.append(("grid", L["ny"], L["nx"], L["ystep"] if L["nx"] > 1 else None))
+                    assert (L["win_w"], L["win_h"]) == (int(round(20 * L["factor"])), int(round(20 * L["factor"]))) and min(L["win_w"], L["win_h"]) >= ms
+                    ystep1 += L["ystep"] == 1
+                    ystep2 += L["ystep"] == 2
+                assert seen == want, (rows, cols, sf, ms)
+                skipped += len(plan) < len(G.level_plan(c.w, c.h, rows, cols, sf, 0))
+    assert ystep1 and ystep2 and skipped
+
+
+def test_level_candidates_equal_oracle(tmp_path):
+    """detect_candidates through level_plan, window_flags and the scan of scan_candidates gives oracle.haar.detect_candidates' raw
+    candidates for a stump cascade (the face cascade's first stages and a synthetic one)."""
+    from oracle import haar as H
+    from oracle import oracle as O
+    from test_gpu_detect_batch import write_stump_cascade
+    paths = [G.truncate_cascade(CV2_DIR / "haarcascade_frontalface_alt.xml", tmp_path / "face3.xml", 3), write_stump_cascade(tmp_path / "stumps.xml")]
+    found = 0
+    for path in paths:
+        for k, (rows, cols) in enumerate([(161, 203), (240, 320)]):
+            gray = O.bgr2gray(cv2.cvtColor(_textured(rows, cols, 40 + k), cv2.COLOR_GRAY2BGR))
+            for sf, ms in ((1.1, 0), (1.3, 30), (2.5, 0)):
+                want = H.detect_candidates(H.Cascade(path), gray, sf, ms)
+                assert G.detect_candidates(G.Cascade(path), gray, sf, ms) == want, (path, rows, sf, ms)
+                found += len(want)
+    assert found > 0
